@@ -2,7 +2,7 @@
 """bench.py -- headline benchmark of the hot path (BASELINE.json): decoded frames/s and info-bits/s,
 BCH(63,36) normalised min-sum (alpha = 0.8, <= 50 iterations, early exit), 1/2/4/8 B200 vs host CPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--ebno 4.0]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--ebno 4.0] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step is one pass of the hot path over one batch of synthetic AWGN frames (all-zero codeword, like
@@ -15,7 +15,9 @@ the reference's simulation).  Three measurements per run:
           only 64 bytes leave the GPU), followed by the one NCCL all-reduce of the counters.
 The CPU baseline is the reference's own decoder (oracle/_ref/libccref.so = the reference compiled by
 oracle/build_ref.sh) running simulation.c++'s inner loop on all host cores; if that library is absent,
-the C restatement in oracle/ (kind "port").
+the C restatement in oracle/ (kind "port").  The same holds for the CPU baselines of the other configurations.
+--dump-outputs DIR writes what the last timed step of `value` returned (see dump_outputs) for output-for-output
+comparisons of two builds.
 """
 import argparse
 import json
@@ -65,6 +67,24 @@ def ncu_capture(label):
         return None, False
 
 
+DUMP_FRAMES = 1 << 17  # 131072 frames x 63 decisions as float32 = 33 MB: a dump stays a few tens of MB at any --frames
+
+
+def dump_outputs(path, out, np, torch):
+    """what the timed decode returned to its caller in its last step -- decided bits (frames, n), iteration index and
+    failure flag per frame -- for a fixed, seeded sample of the batch's frames, as float32 .npy files under `path`
+    (frame_index.npy, float64, names the sampled frames).  The LLR batch is seeded too, so two builds run with the same
+    arguments can be compared output for output."""
+    bits, _, it, failed = out
+    B = bits.shape[0]
+    idx = np.sort(np.random.default_rng(0).choice(B, min(B, DUMP_FRAMES), replace=False))
+    sel = torch.from_numpy(idx).to(bits.device)
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "frame_index.npy"), idx.astype(np.float64))
+    for name, t in (("bits", bits), ("iterations", it), ("failed", failed)):
+        np.save(os.path.join(path, name + ".npy"), t[sel].cpu().numpy().astype(np.float32))
+
+
 def measured_peaks():
     try:
         with open(os.path.join(ROOT, "MEASURED_PEAKS.json")) as f:
@@ -112,6 +132,38 @@ class ClockSampler:
                 "reasons": reasons, "samples": len(sm)}
 
 
+def cpu_port_point(q, errors, variant_id, ebno, seconds, frames_per_thread=0, threads=None):
+    """the C restatement in oracle/ standing in for the reference's soft decoder `variant_id` (ids of oracle/ccref.py) of
+    BCH(2^q - 1, t = errors) where the reference library is not built: one python thread per core (ctypes releases the
+    GIL) -> (frames, word_errors, seconds)"""
+    import numpy as np
+    import oracle
+    from ccref import VARIANT_PARAMS
+    from concurrent.futures import ThreadPoolExecutor
+    variant, alpha, beta, max_iter = VARIANT_PARAMS[variant_id]
+    threads = threads or (os.cpu_count() or 1)
+    code = oracle.Code(0, q, errors)
+    H = code.H()
+    sig = oracle.sigma(code.rate, ebno)
+    per = frames_per_thread or max(8, 12600 // code.n)  # 200 frames of BCH(63,36) between two looks at the clock
+
+    def work(t):
+        rng = np.random.default_rng(t)
+        done = err = 0
+        t0 = time.time()
+        while True:
+            y = (1 + sig * rng.standard_normal((per, code.n))).astype(np.float32)
+            bits, _, _, failed = oracle.min_sum(H, y, variant, alpha, beta, max_iter)
+            done += per
+            err += int(((failed == 1) | bits.any(axis=1)).sum())
+            if frames_per_thread or time.time() - t0 >= seconds:
+                return done, err
+    t0 = time.time()
+    with ThreadPoolExecutor(threads) as ex:
+        res = list(ex.map(work, range(threads)))
+    return sum(r[0] for r in res), sum(r[1] for r in res), time.time() - t0
+
+
 def cpu_reference(ebno, seconds, frames_per_thread=0, seed=0):
     """the reference's CPU decoder on all host cores -> (frames/s, cores, kind, word_errors, frames)"""
     cores = os.cpu_count() or 1
@@ -122,32 +174,8 @@ def cpu_reference(ebno, seconds, frames_per_thread=0, seed=0):
                                              seed=seed, seconds=seconds, threads=cores,
                                              max_frames_per_thread=frames_per_thread)
         return frames / el, cores, "reference", werr, frames
-    # port: the C restatement, one python thread per core (ctypes releases the GIL)
-    import numpy as np
-    import oracle
-    from concurrent.futures import ThreadPoolExecutor
-    code = oracle.Code(0, Q, T)
-    H = code.H()
-    sig = oracle.sigma(code.rate, ebno)
-    per = frames_per_thread or 200
-
-    def work(t):
-        rng = np.random.default_rng(t)
-        done = err = 0
-        t0 = time.time()
-        while True:
-            y = (1 + sig * rng.standard_normal((per, N))).astype(np.float32)
-            bits, _, _, failed = oracle.min_sum(H, y, "NMS", ALPHA, 0.0, MAX_ITER)
-            done += per
-            err += int(((failed == 1) | bits.any(axis=1)).sum())
-            if frames_per_thread or time.time() - t0 >= seconds:
-                return done, err
-    t0 = time.time()
-    with ThreadPoolExecutor(cores) as ex:
-        res = list(ex.map(work, range(cores)))
-    el = time.time() - t0
-    frames = sum(r[0] for r in res)
-    return frames / el, cores, "port", sum(r[1] for r in res), frames
+    frames, werr, el = cpu_port_point(Q, T, ccref.V_NMS, ebno, seconds, frames_per_thread, cores)
+    return frames / el, cores, "port", werr, frames
 
 
 def cpu_reference_point(q, errors, variant_id, ebno, seconds, threads=None):
@@ -170,6 +198,15 @@ def cpu_reference_rs(q, errors, words):
     ref = ccref.Ref()
     t0 = time.perf_counter()
     ref.hard_correct(ccref.FAM_RS, q, ccref.CAP_ERRORS, errors, ccref.ALG_EUKLID, words)
+    return len(words) / (time.perf_counter() - t0)
+
+
+def cpu_port_rs(q, errors, words):
+    """the C restatement's Euklid decoder (oracle/gf_oracle.c) where the reference library is not built -> words/s"""
+    import oracle
+    code = oracle.Code(oracle.FAM_RS, q, errors)
+    t0 = time.perf_counter()
+    code.hard_correct(words)
     return len(words) / (time.perf_counter() - t0)
 
 
@@ -216,11 +253,12 @@ def other_configs(ctx, torch, dist, np, world, rank, dev, timed, args):
         if note:
             rec["note"] = note
         if rank == 0 and cpu is not None and not args.no_cpu:
-            r = cpu_reference_point(*cpu, ebno, 3.0)
-            if r is not None:
-                f, w, el = r
-                rec["cpu_baseline"] = {"value": f / el, "unit": "frames/s", "cores": os.cpu_count(), "kind": "reference",
-                                       "sample": "3 s wall = %d frames, WER %.4f" % (f, w / max(1, f))}
+            r, kind = cpu_reference_point(*cpu, ebno, 3.0), "reference"
+            if r is None:
+                r, kind = cpu_port_point(*cpu, ebno, 3.0), "port"
+            f, w, el = r
+            rec["cpu_baseline"] = {"value": f / el, "unit": "frames/s", "cores": os.cpu_count(), "kind": kind,
+                                   "sample": "3 s wall = %d frames, WER %.4f" % (f, w / max(1, f))}
         out.append(rec)
 
     # ---- configs[0]: BCH(15,7) sum-product, Eb/N0 1..6 dB
@@ -314,11 +352,12 @@ def other_configs(ctx, torch, dist, np, world, rank, dev, timed, args):
     rec["e2e"] = {"value": world * nh * 3 / float(el.item()), "unit": "codewords/s", "h2d_bytes_per_step": nh * 255,
                   "d2h_bytes_per_step": nh * 257, "path": "ccgpu_gf_decode with pinned host buffers"}
     if rank == 0 and not args.no_cpu:
-        r = cpu_reference_rs(8, 16, bad[:2048])
-        if r is not None:
-            rec["cpu_baseline"] = {"value": r, "unit": "codewords/s", "cores": 1, "kind": "reference",
-                                   "sample": "2048 of the same words, euklid_tag, one thread (x %d cores = %.3g if every core ran one)"
-                                             % (os.cpu_count(), r * os.cpu_count())}
+        r, kind = cpu_reference_rs(8, 16, bad[:2048]), "reference"
+        if r is None:
+            r, kind = cpu_port_rs(8, 16, bad[:2048]), "port"
+        rec["cpu_baseline"] = {"value": r, "unit": "codewords/s", "cores": 1, "kind": kind,
+                               "sample": "2048 of the same words, euklid_tag, one thread (x %d cores = %.3g if every core ran one)"
+                                         % (os.cpu_count(), r * os.cpu_count())}
     out.append(rec)
     return out
 
@@ -366,6 +405,8 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=10.0)
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the table of the other BASELINE.json configurations")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (a fixed sample of frames) to DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -437,6 +478,8 @@ def main():
     launches = ctx.kernel_launches - launches0 - args.warmup
     clocks = sampler.stop() if rank == 0 else None
     value = world * B * args.steps / (ms_res * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out, np, torch)
 
     # iteration statistics of the batch (for the ALU model and the log)
     it = out[2].to(torch.int64)
