@@ -15,6 +15,7 @@
 
 #include "../../include/ccgpu.h"
 #include "channel.cuh"
+#include "chase.h"
 #include "codes.hpp"
 #include "gf_decode.h"
 #include "ms_csr.h"
@@ -1530,6 +1531,81 @@ int ccgpu_awgn_point_hard(ccgpu_ctx *ctx, const ccgpu_code *code, double ebno_db
     CU(cudaGetLastError());
     ctx->launches += 3;
   }
+  if (!dev) {
+    CU(cudaMemcpyAsync(ctx->h_counters, ctx->d_counters, sizeof(ccgpu_counters), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    *out = *ctx->h_counters;
+  }
+  return CCGPU_OK;
+}
+
+// ---- Chase-II (extension): K5 in chase.cu
+static int check_chase(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t p) {
+  if (code->ctx != ctx) return fail(ctx, CCGPU_ERR_INVALID, "code was not created on this context");
+  if (p > kChaseMaxP) return fail(ctx, CCGPU_ERR_INVALID, "Chase-II takes 0 <= p <= 8 test positions");
+  if (code->spec.family != 0) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "Chase-II decoding needs a binary BCH code");
+  if (p > code->spec.n) return fail(ctx, CCGPU_ERR_INVALID, "p > n");
+  return CCGPU_OK;
+}
+static int chase_rc(ccgpu_ctx *ctx, int rc) {
+  if (rc == -3) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "code not supported by the Chase kernel (t <= 31)");
+  if (rc != 0) return cuda_fail(ctx, cudaGetLastError(), "chase_launch");
+  ctx->launches++;
+  return CCGPU_OK;
+}
+
+int ccgpu_decode_llr_chase(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t p, const float *y, uint64_t frames,
+                           uint8_t *bits, uint8_t *failed, uint8_t *chosen) {
+  if (!ctx || !code || !y || !bits || !failed) return fail(ctx, CCGPU_ERR_INVALID, "null argument");
+  int rc = check_chase(ctx, code, p);
+  if (rc) return rc;
+  std::lock_guard<std::mutex> g(ctx->mu);
+  if (frames == 0) return CCGPU_OK;
+  CU(cudaSetDevice(ctx->device));
+  const size_t n = code->spec.n;
+  const bool dev = is_device_ptr(y);
+  if (is_device_ptr(bits) != dev || is_device_ptr(failed) != dev || (chosen && is_device_ptr(chosen) != dev))
+    return fail(ctx, CCGPU_ERR_INVALID, "y and the outputs must all be device pointers or all host pointers");
+  if (dev) return chase_rc(ctx, chase_launch(code->gf, p, y, frames, bits, failed, chosen, ctx->sm_count, ctx->stream));
+  // host buffers: chunks rotate over the staging slots so that copies and decoding overlap
+  const size_t per_frame = n * sizeof(float) + n + 2;
+  const uint64_t chunk = std::max<uint64_t>(1024, std::min<uint64_t>((frames + 15) / 16, (size_t(32) << 20) / per_frame));
+  rc = ensure_slots(ctx, chunk * per_frame + 256);
+  if (rc) return rc;
+  CU(cudaEventRecord(ctx->main_ready, ctx->stream));
+  for (int s = 0; s < kSlots; ++s) CU(cudaStreamWaitEvent(ctx->slot_stream[s], ctx->main_ready, 0));
+  int slot = 0;
+  for (uint64_t f0 = 0; f0 < frames; f0 += chunk, slot = (slot + 1) % kSlots) {
+    const uint64_t nf = std::min(chunk, frames - f0);
+    cudaStream_t st = ctx->slot_stream[slot];
+    float *d_y = static_cast<float *>(ctx->slot_buf[slot]);
+    uint8_t *d_bits = reinterpret_cast<uint8_t *>(d_y + chunk * n);
+    uint8_t *d_failed = d_bits + chunk * n;
+    uint8_t *d_chosen = d_failed + chunk;
+    CU(cudaMemcpyAsync(d_y, y + f0 * n, nf * n * sizeof(float), cudaMemcpyHostToDevice, st));
+    rc = chase_rc(ctx, chase_launch(code->gf, p, d_y, nf, d_bits, d_failed, chosen ? d_chosen : nullptr, ctx->sm_count, st));
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(bits + f0 * n, d_bits, nf * n, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(failed + f0, d_failed, nf, cudaMemcpyDeviceToHost, st));
+    if (chosen) CU(cudaMemcpyAsync(chosen + f0, d_chosen, nf, cudaMemcpyDeviceToHost, st));
+  }
+  for (int s = 0; s < kSlots; ++s) CU(cudaStreamSynchronize(ctx->slot_stream[s]));
+  return CCGPU_OK;
+}
+
+int ccgpu_awgn_point_chase(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t p, double ebno_db, uint64_t seed,
+                           uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out) {
+  if (!ctx || !code || !out) return fail(ctx, CCGPU_ERR_INVALID, "null argument");
+  int rc = check_chase(ctx, code, p);
+  if (rc) return rc;
+  std::lock_guard<std::mutex> g(ctx->mu);
+  CU(cudaSetDevice(ctx->device));
+  const bool dev = is_device_ptr(out);
+  unsigned long long *counters = dev ? reinterpret_cast<unsigned long long *>(out) : ctx->d_counters;
+  if (!dev) CU(cudaMemsetAsync(ctx->d_counters, 0, sizeof(ccgpu_counters), ctx->stream));
+  const float sigma = static_cast<float>(ccgpu_sigma(code->spec.rate, ebno_db));
+  rc = chase_rc(ctx, chase_awgn_launch(code->gf, p, sigma, seed, point, frame0, frames, counters, ctx->sm_count, ctx->stream));
+  if (rc) return rc;
   if (!dev) {
     CU(cudaMemcpyAsync(ctx->h_counters, ctx->d_counters, sizeof(ccgpu_counters), cudaMemcpyDeviceToHost, ctx->stream));
     CU(cudaStreamSynchronize(ctx->stream));

@@ -14,11 +14,7 @@
 // (its own BM has an out-of-bounds read, SURVEY.md fact 8), so results are compared against Euklid.
 //
 // Work split inside the warp
-//   syndromes   lane <-> syndrome index.  Multiplying by the constant alpha^(root_j) is ONE
-//               shared-memory lookup in a per-lane table T[x][lane] (32-bit entries: lane j always
-//               hits bank j, conflict free); the word is cut into four segments whose Horner chains
-//               run interleaved (4 independent dependency chains), symbols arrive as 32-bit
-//               broadcasts of four packed bytes.
+//   syndromes   lane <-> syndrome index (gf_device.cuh).
 //   BM          lane <-> locator coefficient, discrepancy by XOR butterfly.
 //   roots       lane <-> codeword position (log/antilog tables in shared memory).
 //   Forney      lane <-> error index.
@@ -30,6 +26,7 @@
 #include <vector>
 
 #include "gf_decode.h"
+#include "gf_device.cuh"
 
 namespace ccgpu {
 
@@ -37,7 +34,7 @@ namespace {
 
 constexpr int kGfThreads = 256;
 constexpr int kGfWarps = kGfThreads / 32;
-constexpr unsigned kAll = 0xffffffffu;
+constexpr unsigned kAll = kGfAll;
 constexpr int kWordBytes = 256;   // per-warp word buffer
 constexpr int kWarpBytes = 512;   // word + syndromes + locator + evaluator + positions
 
@@ -51,59 +48,12 @@ struct GfParams {
   uint8_t *corrected, *n_errors, *failed;
 };
 
-struct Gf {
-  const uint8_t *exp, *log;
-  __device__ __forceinline__ unsigned mul(unsigned a, unsigned b) const { return (a && b) ? exp[log[a] + log[b]] : 0u; }
-  __device__ __forceinline__ unsigned mul_alpha(unsigned a, unsigned e) const { return a ? exp[log[a] + e] : 0u; }  // e < n
-};
-
-__device__ __forceinline__ unsigned xor_reduce(unsigned v) {
-  return __reduce_xor_sync(kAll, v);  // REDUX.XOR: one instruction instead of a five-step shuffle butterfly
-}
-
-// syndromes of `word` (zero padded to a multiple of 4 bytes per segment) into synd[0..nroots)
-__device__ __forceinline__ bool syndromes(const GfParams &p, const Gf &F, const uint8_t *word, const uint32_t *mtab,
-                                          const uint8_t *rexp, uint8_t *synd, int lane) {
-  const int seg = ((p.n + 15) / 16) * 4;  // segment length in symbols, multiple of 4; 4 segments cover n
-  bool any = false;
-  for (int j0 = 0; j0 < p.nroots; j0 += 32) {
-    const int j = j0 + lane;
-    const uint32_t *T = mtab + (j0 / 32) * (32 << p.q) + lane;  // T[x * 32] = x * alpha^(root_j)
-    unsigned v0 = 0, v1 = 0, v2 = 0, v3 = 0;
-    for (int i = seg - 4; i >= 0; i -= 4) {
-      const uint32_t w0 = *reinterpret_cast<const uint32_t *>(word + i);
-      const uint32_t w1 = *reinterpret_cast<const uint32_t *>(word + seg + i);
-      const uint32_t w2 = *reinterpret_cast<const uint32_t *>(word + 2 * seg + i);
-      const uint32_t w3 = *reinterpret_cast<const uint32_t *>(word + 3 * seg + i);
-#pragma unroll
-      for (int b = 3; b >= 0; --b) {
-        v0 = T[v0 * 32] ^ ((w0 >> (8 * b)) & 0xffu);
-        v1 = T[v1 * 32] ^ ((w1 >> (8 * b)) & 0xffu);
-        v2 = T[v2 * 32] ^ ((w2 >> (8 * b)) & 0xffu);
-        v3 = T[v3 * 32] ^ ((w3 >> (8 * b)) & 0xffu);
-      }
-    }
-    unsigned s = 0;
-    if (j < p.nroots) {
-      // S = v0 + v1 X^seg + v2 X^(2 seg) + v3 X^(3 seg),  X = alpha^(root_j)
-      const unsigned e1 = (static_cast<unsigned>(rexp[j]) * seg) % p.n;
-      unsigned e2 = e1 + e1, e3;
-      if (e2 >= static_cast<unsigned>(p.n)) e2 -= p.n;
-      e3 = e2 + e1;
-      if (e3 >= static_cast<unsigned>(p.n)) e3 -= p.n;
-      s = v0 ^ F.mul_alpha(v1, e1) ^ F.mul_alpha(v2, e2) ^ F.mul_alpha(v3, e3);
-      synd[j] = static_cast<uint8_t>(s);
-    }
-    any |= __any_sync(kAll, s != 0);
-  }
-  __syncwarp();
-  return any;
-}
-
 __global__ void __launch_bounds__(kGfThreads) gf_decode_kernel(const GfParams p) {
   extern __shared__ __align__(16) uint8_t sm[];
   const int size = 1 << p.q, n = p.n;
   const int ntab = (p.nroots + 31) / 32;
+  // the table prologue of gf_fill_tables (gf_device.cuh), written out: routing it through that function changes this
+  // kernel's instruction schedule
   uint32_t *mtab = reinterpret_cast<uint32_t *>(sm);                    // [ntab][size][32]
   uint8_t *s_exp = sm + size_t(ntab) * size * 32 * sizeof(uint32_t);  // [2*size]
   uint8_t *s_log = s_exp + 2 * size;                                  // [size]
@@ -251,11 +201,7 @@ __global__ void __launch_bounds__(kGfThreads) gf_decode_kernel(const GfParams p)
   }
 }
 
-size_t gf_smem_bytes(const GfDevice &d) {
-  const size_t size = size_t(1) << d.q;
-  const size_t ntab = (d.nroots + 31) / 32;
-  return ntab * size * 32 * sizeof(uint32_t) + 3 * size + 64 + size_t(kGfWarps) * kWarpBytes;
-}
+size_t gf_smem_bytes(const GfDevice &d) { return gf_table_bytes(d.q, d.nroots) + size_t(kGfWarps) * kWarpBytes; }
 
 }  // namespace
 

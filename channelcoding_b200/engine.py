@@ -322,6 +322,42 @@ class Code:
                                                          C.addressof(c)))
         return c.as_dict()
 
+    def decode_chase(self, y, p, out=None):
+        """Chase-II with the p least reliable positions (extension, ccgpu_decode_llr_chase; binary BCH codes,
+        0 <= p <= 8) -> bits (frames, n) uint8, failed (frames,) uint8, chosen (frames,) uint8 [index of the returned
+        test pattern]; numpy or torch CUDA tensors like decode()"""
+        if _is_torch(y):
+            import torch
+            y = y.contiguous().view(-1, self.n)
+            frames = y.shape[0]
+            if out is None:
+                out = (torch.empty((frames, self.n), dtype=torch.uint8, device=y.device),
+                       torch.empty(frames, dtype=torch.uint8, device=y.device),
+                       torch.empty(frames, dtype=torch.uint8, device=y.device))
+        else:
+            y = np.ascontiguousarray(y, np.float32).reshape(-1, self.n)
+            frames = y.shape[0]
+            if out is None:
+                out = (np.empty((frames, self.n), np.uint8), np.empty(frames, np.uint8), np.empty(frames, np.uint8))
+        bits, failed, chosen = out
+        self.ctx._follow_torch(y, bits)
+        self.ctx._check(_lib.lib().ccgpu_decode_llr_chase(self.ctx._h, self._h, int(p), _ptr(y), frames, _ptr(bits),
+                                                          _ptr(failed), _ptr(chosen)))
+        return bits, failed, chosen
+
+    def awgn_point_chase(self, ebno_db, frames, p, seed=0, point=0, frame0=0, out=None):
+        """one Eb/N0 point decoded with Chase-II on the GPU (ccgpu_awgn_point_chase) -> counters.
+        out: optional torch uint64/int64 CUDA tensor of 8 slots that is accumulated into (no sync)."""
+        if out is not None:
+            self.ctx._follow_torch(out)
+            self.ctx._check(_lib.lib().ccgpu_awgn_point_chase(self.ctx._h, self._h, int(p), float(ebno_db), seed, point, frame0,
+                                                              frames, _ptr(out)))
+            return out
+        c = Counters()
+        self.ctx._check(_lib.lib().ccgpu_awgn_point_chase(self.ctx._h, self._h, int(p), float(ebno_db), seed, point, frame0,
+                                                          frames, C.addressof(c)))
+        return c.as_dict()
+
     def bitflip_point(self, weight, variant="MS", alpha=1.0, beta=0.0, max_iter=50,
                       stop_rule=STOP_REF_ZERO_OVERLAP, first=0, count=0, quant=None):
         """one error weight of bitflip_simulation (simulation.c++:156-213) -> counters"""
@@ -454,6 +490,12 @@ class GroupCode:
         c = Counters()
         self.group._check(_lib.lib().ccgpu_group_awgn_point_hard(self.group._h, self._arr, float(ebno_db), seed, point, frame0,
                                                                  frames, C.addressof(c)))
+        return c.as_dict()
+
+    def awgn_point_chase(self, ebno_db, frames, p, seed=0, point=0, frame0=0):
+        c = Counters()
+        self.group._check(_lib.lib().ccgpu_group_awgn_point_chase(self.group._h, self._arr, int(p), float(ebno_db), seed, point,
+                                                                  frame0, frames, C.addressof(c)))
         return c.as_dict()
 
     def awgn_point_mbbp(self, ebno_db, frames, shifts, variant="MS", alpha=1.0, beta=0.0, max_iter=50,

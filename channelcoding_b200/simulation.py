@@ -88,3 +88,16 @@ def gpu_point_fn(code, variant="MS", alpha=1.0, beta=0.0, max_iter=50, stop_rule
             code.ctx.sync()  # the launch is asynchronous on the context's stream, not on torch's
         return out
     return fn
+
+
+def chase_point_fn(code, p, seed=0):
+    """point_fn for awgn_sweep backed by ccgpu_awgn_point_chase (Chase-II with p test positions) on the code's device"""
+    import torch
+
+    def fn(ebno, point, frame0, frames):
+        out = torch.zeros(8, dtype=torch.int64, device="cuda:%d" % code.ctx.device)
+        if frames > 0:
+            code.awgn_point_chase(ebno, frames, p, seed=seed, point=point, frame0=frame0, out=out)
+            code.ctx.sync()
+        return out
+    return fn

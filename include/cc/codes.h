@@ -9,6 +9,7 @@
 //   cyclic::berlekamp_massey_tag / euklid_tag / PGZ    same names, same to_string()   codes/hard_decision.h:15-24
 //   cyclic::primitive_bch<q, Capability, Tag>          cc::primitive_bch<q, Capability, Tag>   codes/bch.h:16-161
 //   cyclic::rs<q, Capability, Tag>                     cc::rs<q, Capability, Tag>              codes/rs.h:6-94
+//   (extension) Chase-II                               cc::primitive_bch<q, Capability, chase_tag<P> >
 //     .correct<R>(vector<float|uint>)  .to_string()  .rate  ::n  ::t  .H<T>()           codes/cyclic.h:282-359
 //
 // Differences a user sees: every object holds a ccgpu context/code handle (one GPU, or every GPU of the current
@@ -141,6 +142,17 @@ struct fixed_offset_min_sum_tag : soft_decision_tag, fixed_point_tag {
 struct peterson_gorenstein_zierler_tag : hard_decision_tag { static std::string to_string() { return "PGZ"; } };
 struct berlekamp_massey_tag : hard_decision_tag { static std::string to_string() { return "BM"; } };
 struct euklid_tag : hard_decision_tag { static std::string to_string() { return "EUKLID"; } };
+
+// ---- extension: Chase-II (ccgpu_decode_llr_chase).  The hard decision plus 2^P test patterns over the P least reliable
+// positions, each decoded algebraically, the candidate closest to the channel values wins.  Neither a soft-decision
+// (min-sum) nor a hard-decision tag: it takes channel values and decodes algebraically.
+template <unsigned P> struct chase_tag : algorithm_tag {
+  static_assert(P <= 8, "Chase-II takes at most 8 test positions");
+  static constexpr unsigned p = P;
+  static std::string to_string() { return "CHASE" + std::to_string(P); }
+};
+template <typename Tag> struct is_chase_tag : std::false_type {};
+template <unsigned P> struct is_chase_tag<chase_tag<P> > : std::true_type {};
 
 // ---- one GPU context shared by every code object of the process (per device) ------------------------
 class gpu_error : public std::runtime_error {
@@ -309,6 +321,7 @@ protected:
 public:
   const double rate;  // public data member like cyclic.h:111
   static constexpr bool soft_tag = std::is_base_of<soft_decision_tag, Algorithm>::value;
+  static constexpr bool chase = is_chase_tag<Algorithm>::value;
 
   std::string to_string() const {  // cyclic.h:282-287
     char buf[96];
@@ -474,20 +487,62 @@ private:
   }
 };
 
+namespace detail {
+template <unsigned q, typename Capability> std::shared_ptr<code_handle> make_bch(int device) {
+  return code_handle::make(device, [](ccgpu_ctx *ctx, ccgpu_code **out) {
+    return ccgpu_bch_create(ctx, q, correction_capability<Capability>::kind, correction_capability<Capability>::raw, out);
+  });
+}
+}  // namespace detail
+
 // cyclic::primitive_bch<q, Capability, Sigma> -- codes/bch.h:16-161
 template <unsigned q, typename Capability, typename Sigma = peterson_gorenstein_zierler_tag>
 class primitive_bch : public cyclic_base<Sigma> {
-  static std::shared_ptr<detail::code_handle> make(int device) {
-    return detail::code_handle::make(device, [](ccgpu_ctx *ctx, ccgpu_code **out) {
-      return ccgpu_bch_create(ctx, q, correction_capability<Capability>::kind, correction_capability<Capability>::raw, out);
-    });
-  }
-
 public:
   static constexpr unsigned n = (1u << q) - 1;
   static constexpr unsigned t = correction_capability<Capability>::value;
   // device < 0: the process default (cc::set_default_device); under a current device_group the code lives on all its members
-  explicit primitive_bch(int device = -1) : cyclic_base<Sigma>(make(device)) {}
+  explicit primitive_bch(int device = -1) : cyclic_base<Sigma>(detail::make_bch<q, Capability>(device)) {}
+};
+
+// extension: the same code decoded with Chase-II over the P least reliable positions (ccgpu_decode_llr_chase)
+template <unsigned q, typename Capability, unsigned P>
+class primitive_bch<q, Capability, chase_tag<P> > : public cyclic_base<chase_tag<P> > {
+  using base = cyclic_base<chase_tag<P> >;
+
+public:
+  static constexpr unsigned n = (1u << q) - 1;
+  static constexpr unsigned t = correction_capability<Capability>::value;
+  explicit primitive_bch(int device = -1) : base(detail::make_bch<q, Capability>(device)) {}
+
+  // frames x n channel values -> frames x n bits; failed[f] = 1 where no test pattern decoded; chosen[f] (optional) is
+  // the index of the returned test pattern
+  void correct_batch(const float *y, uint64_t frames, uint8_t *bits, uint8_t *failed, uint8_t *chosen = nullptr) const {
+    this->h_->ctx->check(ccgpu_decode_llr_chase(this->h_->ctx->get(), this->h_->code, P, y, frames, bits, failed, chosen));
+  }
+  // one frame of channel values; throws decoding_failure when no test pattern decodes
+  template <typename Return_type = uint8_t, typename InputSequence>
+  std::vector<Return_type> correct(const InputSequence &b) const {
+    if (b.size() != n)
+      throw std::runtime_error("Channel code word has the wrong size (" + std::to_string(b.size()) + "). Expected " +
+                               std::to_string(n));
+    const std::vector<float> y(b.begin(), b.end());
+    std::vector<uint8_t> out(n);
+    uint8_t failed = 0;
+    correct_batch(y.data(), 1, out.data(), &failed);
+    if (failed) throw decoding_failure("Decoding failure");
+    return std::vector<Return_type>(out.begin(), out.end());
+  }
+  // one Eb/N0 point (simulation.c++:112-149) decoded with Chase-II on the device, sharded over the code's group if any
+  ccgpu_counters awgn_point(double ebno_db, uint64_t frames, uint64_t seed = 0, uint32_t point = 0, uint64_t frame0 = 0) const {
+    ccgpu_counters c{};
+    if (this->h_->grp)
+      this->h_->grp->check(ccgpu_group_awgn_point_chase(this->h_->grp->get(), this->h_->codes.data(), P, ebno_db, seed, point,
+                                                        frame0, frames, &c));
+    else
+      this->h_->ctx->check(ccgpu_awgn_point_chase(this->h_->ctx->get(), this->h_->code, P, ebno_db, seed, point, frame0, frames, &c));
+    return c;
+  }
 };
 
 // cyclic::rs<q, Capability, Sigma, N, Coding, mu, step> -- codes/rs.h:6-94

@@ -268,6 +268,24 @@ int ccgpu_awgn_point_uncoded(ccgpu_ctx *ctx, uint32_t n, double rate, double ebn
 int ccgpu_awgn_point_hard(ccgpu_ctx *ctx, const ccgpu_code *code, double ebno_db, uint64_t seed, uint32_t point,
                           uint64_t frame0, uint64_t frames, ccgpu_counters *out);
 
+/* EXTENSION (no reference implementation): Chase-II soft-decision decoding of binary primitive BCH codes.  Per frame:
+ *   h_c = (y_c < 0) as codes/codes.h:43-52 (0 for -0.0 and NaN);
+ *   u_0 .. u_{p-1}: the p columns with the smallest (bits of fabsf(y_c) as uint32, c), ascending (ties: lower column;
+ *   NaN sorts above +inf);
+ *   test word m (m = 0 .. 2^p - 1) is h with u_j flipped for every set bit j of m, decoded errors-only exactly as
+ *   ccgpu_gf_decode decodes it (bounded distance, same failure rules); a success x_m is a candidate;
+ *   D_m = sum of fabsf(y_c) over the columns where x_m != h, float32, c ascending, starting from +0.0;
+ *   the candidate with the smallest (bits of D_m as uint32, m) is returned.  Without a candidate: failed = 1,
+ *   bits = h, chosen = 0.  p = 0 is ccgpu_gf_decode of the hard decision.
+ * Binary BCH codes (t <= 31); 0 <= p <= 8 and p <= n.  bits frames x n, failed frames, chosen frames (nullable: index
+ * m of the returned test pattern).  Host or device pointers like ccgpu_decode_llr. */
+int ccgpu_decode_llr_chase(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t p, const float *y, uint64_t frames,
+                           uint8_t *bits, uint8_t *failed, uint8_t *chosen);
+/* one Eb/N0 point, frames [frame0, frame0 + frames) of the ccgpu_awgn_point noise stream, decoded with Chase-II on chip;
+ * only counters leave (iterations stays 0).  `out` host or device pointer as in ccgpu_awgn_point. */
+int ccgpu_awgn_point_chase(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t p, double ebno_db, uint64_t seed,
+                           uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
+
 /* one weight class of bitflip_simulation::operator() (simulation.c++:156-213): all C(n, weight)
  * inputs x = -2*bit + 1, decoded and counted; patterns [first, first + count) in the
  * lexicographic order of std::next_permutation (count 0 = all). */
@@ -327,12 +345,14 @@ int ccgpu_group_size(const ccgpu_group *group);
 ccgpu_ctx *ccgpu_group_ctx(const ccgpu_group *group, int member);
 const char *ccgpu_group_last_error(const ccgpu_group *group);
 int ccgpu_group_set_min_frames(ccgpu_group *group, uint64_t frames_per_member);
-/* the Monte-Carlo points of ccgpu_awgn_point / _hard / _mbbp / _uncoded / ccgpu_bitflip_point, sharded; `out` is a
+/* the Monte-Carlo points of ccgpu_awgn_point / _hard / _chase / _mbbp / _uncoded / ccgpu_bitflip_point, sharded; `out` is a
  * host pointer and holds the merged counters on return */
 int ccgpu_group_awgn_point(ccgpu_group *group, ccgpu_code *const *codes, const ccgpu_ms_params *params, double ebno_db,
                            uint64_t seed, uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
 int ccgpu_group_awgn_point_hard(ccgpu_group *group, ccgpu_code *const *codes, double ebno_db, uint64_t seed, uint32_t point,
                                 uint64_t frame0, uint64_t frames, ccgpu_counters *out);
+int ccgpu_group_awgn_point_chase(ccgpu_group *group, ccgpu_code *const *codes, uint32_t p, double ebno_db,
+                                 uint64_t seed, uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
 int ccgpu_group_awgn_point_mbbp(ccgpu_group *group, ccgpu_code *const *codes, const ccgpu_ms_params *params,
                                 const uint32_t *shifts, uint32_t n_bases, double ebno_db, uint64_t seed, uint32_t point,
                                 uint64_t frame0, uint64_t frames, ccgpu_counters *out);

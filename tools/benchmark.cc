@@ -9,7 +9,9 @@
 // Additions: --seed is honoured (the reference parses and drops it), --stop-rule ref|gf2 (stop test of the soft
 // decoders: the reference's integer zero-overlap rule or the GF(2) syndrome), --max-samples N, --errors W (bit-flip
 // weight, bitflips.c++ uses 6), --out DIR, --device D (first CUDA device), --gpus N (shard every point over N devices
-// D .. D+N-1 through a ccgpu_group; the counters, hence the logs, are identical to the one-GPU run).
+// D .. D+N-1 through a ccgpu_group; the counters, hence the logs, are identical to the one-GPU run),
+// --algorithm chase1 .. chase8 (Chase-II over 1 .. 8 test positions, "(n, l, dmin)-CHASE<P>.log"; built only when
+// named, never part of "all" or of the default selection).
 #include <getopt.h>
 
 #include <cmath>
@@ -34,6 +36,18 @@ template <unsigned Q, typename D> static void add_code(std::vector<decoder> &v) 
   v.emplace_back(primitive_bch<Q, D, self_correcting_2_min_sum_tag<50> >());
   v.emplace_back(primitive_bch<Q, D, normalized_2d_min_sum_tag<50> >());
 }
+// Chase-II decoders (extension): only built when --algorithm chase<P> asks for them, never part of "all"
+template <unsigned Q, unsigned P> static void add_chase_power(std::vector<decoder> &v) {
+  v.emplace_back(primitive_bch<Q, dmin<3>, chase_tag<P> >());
+  v.emplace_back(primitive_bch<Q, dmin<5>, chase_tag<P> >());
+  v.emplace_back(primitive_bch<Q, dmin<7>, chase_tag<P> >());
+  v.emplace_back(primitive_bch<Q, dmin<9>, chase_tag<P> >());
+}
+template <unsigned P> static void add_chase(std::vector<decoder> &v) {
+  add_chase_power<5, P>(v);
+  add_chase_power<6, P>(v);
+  add_chase_power<7, P>(v);
+}
 template <unsigned Q> static void add_power(std::vector<decoder> &v) {
   add_code<Q, dmin<3> >(v);
   add_code<Q, dmin<5> >(v);
@@ -43,7 +57,8 @@ template <unsigned Q> static void add_power(std::vector<decoder> &v) {
 
 [[noreturn]] static void usage() {
   std::cout << "--simulation [awgn|bitflip]  choose the simulation (default awgn)\n"
-               "--algorithm <ms|nms|oms|scms1|scms2|2dnms|bm|pgz|euklid|all>   (repeatable)\n"
+               "--algorithm <ms|nms|oms|scms1|scms2|2dnms|bm|pgz|euklid|all|chase1..chase8>   (repeatable;\n"
+               "             Chase-II only when named, awgn only)\n"
                "--k <5|6|7|all>   code length n = 2^k - 1   (repeatable)\n"
                "--dmin <3|5|7|9|all>                          (repeatable)\n"
                "--seed <num>  --seed-time  --threads <num>\n"
@@ -108,6 +123,10 @@ int main(int argc, char *const argv[]) {
   add_power<5>(decoders);
   add_power<6>(decoders);
   add_power<7>(decoders);
+  static void (*const chase[])(std::vector<decoder> &) = { add_chase<1>, add_chase<2>, add_chase<3>, add_chase<4>,
+                                                           add_chase<5>, add_chase<6>, add_chase<7>, add_chase<8> };
+  for (unsigned p = 1; p <= 8; ++p)
+    if (algorithms.count("chase" + std::to_string(p))) chase[p - 1](decoders);
 
   // selection by parsing to_string(), exactly like benchmark.c++:214-240
   std::vector<const decoder *> chosen;

@@ -2,6 +2,7 @@
 """tools/sweep.py -- Eb/N0 waterfall sweep sharded over GPUs (BASELINE.json config 5).
 
     python tools/sweep.py --q 8 --t 18 --variant NMS --alpha 0.8 --ebno-from 0 --ebno-to 8 --ebno-step 0.5
+    python tools/sweep.py --q 6 --t 5 --chase 4 ...      # Chase-II over the 4 least reliable positions
     torchrun --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 tools/sweep.py ...
 
 Every Eb/N0 point is simulated in rounds of --batch frames (split evenly over the ranks by global frame
@@ -34,6 +35,8 @@ def main():
     ap.add_argument("--min-errors", type=int, default=100)
     ap.add_argument("--max-frames", type=float, default=1e9)
     ap.add_argument("--seed", type=int, default=0)
+    ap.add_argument("--chase", type=int, default=None, metavar="P",
+                    help="decode with Chase-II over the P least reliable positions (0..8) instead of the min-sum variant")
     a = ap.parse_args()
 
     import torch
@@ -61,8 +64,11 @@ def main():
         while True:
             first, count = shard_range(a.batch, world, rank)
             part = torch.zeros(8, dtype=torch.int64, device=dev)
-            code.awgn_point(eb, count, a.variant, a.alpha, a.beta, a.max_iter, a.stop_rule, seed=a.seed, point=point,
-                            frame0=done + first, out=part)
+            if a.chase is None:
+                code.awgn_point(eb, count, a.variant, a.alpha, a.beta, a.max_iter, a.stop_rule, seed=a.seed, point=point,
+                                frame0=done + first, out=part)
+            else:
+                code.awgn_point_chase(eb, count, a.chase, seed=a.seed, point=point, frame0=done + first, out=part)
             if world > 1:
                 dist.all_reduce(part, op=dist.ReduceOp.SUM)  # the one collective of the path
             total += part
@@ -72,7 +78,7 @@ def main():
                 break
         el = time.perf_counter() - t0
         if rank == 0:
-            print(json.dumps({"code": code.to_string(a.variant), "ebno_db": eb, "frames": c[0], "frame_errors": c[1],
+            print(json.dumps({"code": code.to_string(a.variant if a.chase is None else "CHASE%d" % a.chase), "ebno_db": eb, "frames": c[0], "frame_errors": c[1],
                               "bit_errors": c[2], "wer": c[1] / c[0], "ber": c[2] / c[0] / code.n,
                               "avg_iterations": c[3] / c[0], "failures": c[4], "undetected": c[5], "n_gpus": world,
                               "seconds": el, "frames_per_s": c[0] / el}), flush=True)
