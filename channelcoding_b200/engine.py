@@ -282,25 +282,32 @@ class Code:
         return c.as_dict()
 
     def decode_mbbp(self, y, shifts, variant="MS", alpha=1.0, beta=0.0, max_iter=50, stop_rule=STOP_REF_ZERO_OVERLAP,
-                    want_L=True):
+                    want_L=True, out=None):
         """multiple-bases decoding (extension, ccgpu_decode_llr_mbbp): every frame is decoded once per rotation in
-        `shifts`, the best converged candidate is returned -> bits, L, iter, failed, chosen"""
+        `shifts`, the best converged candidate is returned -> bits, L, iter, failed, chosen.
+        out: optional (bits, L, iter, failed, chosen) buffers like decode()'s; L, iter and chosen may be None"""
         p = ms_params(variant, alpha, beta, max_iter, stop_rule)
         sh = np.ascontiguousarray(shifts, np.uint32)
         if _is_torch(y):
             import torch
             y = y.contiguous().view(-1, self.n)
             frames = y.shape[0]
-            mk = lambda shape, dt: torch.empty(shape, dtype=dt, device=y.device)  # noqa: E731
-            bits, it, failed, chosen = mk((frames, self.n), torch.uint8), mk(frames, torch.uint8), mk(frames, torch.uint8), mk(frames, torch.uint8)
-            L = mk((frames, self.n), torch.float32) if want_L else None
+            if out is None:
+                mk = lambda shape, dt: torch.empty(shape, dtype=dt, device=y.device)  # noqa: E731
+                bits, it, failed, chosen = mk((frames, self.n), torch.uint8), mk(frames, torch.uint8), mk(frames, torch.uint8), mk(frames, torch.uint8)
+                L = mk((frames, self.n), torch.float32) if want_L else None
+            else:
+                bits, L, it, failed, chosen = out
         else:
             y = np.ascontiguousarray(y, np.float32).reshape(-1, self.n)
             frames = y.shape[0]
-            bits, it, failed, chosen = (np.empty((frames, self.n), np.uint8), np.empty(frames, np.uint8),
-                                        np.empty(frames, np.uint8), np.empty(frames, np.uint8))
-            L = np.empty((frames, self.n), np.float32) if want_L else None
-        self.ctx._follow_torch(y)
+            if out is None:
+                bits, it, failed, chosen = (np.empty((frames, self.n), np.uint8), np.empty(frames, np.uint8),
+                                            np.empty(frames, np.uint8), np.empty(frames, np.uint8))
+                L = np.empty((frames, self.n), np.float32) if want_L else None
+            else:
+                bits, L, it, failed, chosen = out
+        self.ctx._follow_torch(y, bits)
         self.ctx._check(_lib.lib().ccgpu_decode_llr_mbbp(self.ctx._h, self._h, C.byref(p), sh.ctypes.data, len(sh), _ptr(y),
                                                          frames, _ptr(bits), _ptr(L), _ptr(it), _ptr(failed), _ptr(chosen)))
         return bits, L, it, failed, chosen

@@ -1,6 +1,7 @@
 """Full-size runs of the BASELINE.json configurations, checked through size-independent properties
-(the oracle cannot follow at these sizes): shard-sum linearity of the counters, statistical agreement with
-a small oracle-checked run, all-zero-codeword round trips for the linear RS code."""
+(the per-frame outputs at the benchmarked batch sizes are checked against the oracle in tests/test_gpu_scale.py):
+shard-sum linearity of the counters, statistical agreement with a small oracle-checked run, all-zero-codeword round
+trips for the linear RS code."""
 import math
 
 import numpy as np
