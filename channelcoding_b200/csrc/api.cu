@@ -8,6 +8,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <initializer_list>
 #include <mutex>
 #include <new>
 #include <string>
@@ -51,7 +52,6 @@ struct ccgpu_ctx {
   // buffer each), so the H2D copy of chunk i+1 and the D2H copy of chunk i-1 overlap the decode
   // of chunk i
   cudaStream_t slot_stream[kSlots] = {};
-  cudaEvent_t slot_done[kSlots] = {};
   cudaEvent_t main_ready = nullptr;
   void *slot_buf[kSlots] = {};
   size_t slot_bytes = 0;
@@ -101,12 +101,41 @@ bool is_device_ptr(const void *p) {
   }
   return a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged;
 }
+// whether every non-null pointer of `ptrs` is device memory (dev) or every one is host memory (!dev)
+bool same_residency(bool dev, std::initializer_list<const void *> ptrs) {
+  for (const void *p : ptrs)
+    if (p && is_device_ptr(p) != dev) return false;
+  return true;
+}
+
+int check_code(ccgpu_ctx *ctx, const ccgpu_code *code) {
+  return code->ctx == ctx ? CCGPU_OK : fail(ctx, CCGPU_ERR_INVALID, "code was not created on this context");
+}
+
+// grid of a grid-stride kernel with one thread (or warp) per item and `per_cta` items per CTA, at most `per_sm` CTAs
+// per SM
+unsigned grid_for(const ccgpu_ctx *ctx, uint64_t items, unsigned per_cta, unsigned per_sm = 16) {
+  return static_cast<unsigned>(
+      std::max<uint64_t>(1, std::min<uint64_t>((items + per_cta - 1) / per_cta, uint64_t(ctx->sm_count) * per_sm)));
+}
+
+size_t align256(size_t v) { return (v + 255) & ~size_t(255); }
+// Cuts typed pieces, each 256-byte aligned, out of a device buffer in order.  On a null base it hands out null
+// pointers and only adds up the size: the size a buffer is allocated with comes from the code that cuts it.
+struct Arena {
+  char *base = nullptr;
+  size_t used = 0;
+  template <class T> T *take(size_t count, bool present = true) {
+    if (!present) return nullptr;
+    T *p = base ? reinterpret_cast<T *>(base + used) : nullptr;
+    used += align256(count * sizeof(T));
+    return p;
+  }
+};
 
 int ensure_slots(ccgpu_ctx *ctx, size_t bytes) {
-  for (int s = 0; s < kSlots; ++s) {
+  for (int s = 0; s < kSlots; ++s)
     if (!ctx->slot_stream[s]) CU(cudaStreamCreateWithFlags(&ctx->slot_stream[s], cudaStreamNonBlocking));
-    if (!ctx->slot_done[s]) CU(cudaEventCreateWithFlags(&ctx->slot_done[s], cudaEventDisableTiming));
-  }
   if (!ctx->main_ready) CU(cudaEventCreateWithFlags(&ctx->main_ready, cudaEventDisableTiming));
   if (bytes <= ctx->slot_bytes) return CCGPU_OK;
   for (int s = 0; s < kSlots; ++s) {
@@ -119,14 +148,80 @@ int ensure_slots(ccgpu_ctx *ctx, size_t bytes) {
   return CCGPU_OK;
 }
 
-int ensure_stage(ccgpu_ctx *ctx, size_t bytes) {
-  if (bytes <= ctx->d_stage_bytes) return CCGPU_OK;
-  if (ctx->d_stage) cudaFree(ctx->d_stage);
-  ctx->d_stage = nullptr;
-  ctx->d_stage_bytes = 0;
-  const size_t want = std::max(bytes, size_t(1) << 20);
-  CU(cudaMalloc(&ctx->d_stage, want));
-  ctx->d_stage_bytes = want;
+// grows the stage arena to fit the layout that cut(Arena &) cuts, then cuts it there
+template <class Cut>
+int cut_stage(ccgpu_ctx *ctx, Cut &&cut) {
+  Arena size;
+  cut(size);
+  if (size.used > ctx->d_stage_bytes) {
+    if (ctx->d_stage) cudaFree(ctx->d_stage);
+    ctx->d_stage = nullptr;
+    ctx->d_stage_bytes = 0;
+    const size_t want = std::max(size.used, size_t(1) << 20);
+    CU(cudaMalloc(&ctx->d_stage, want));
+    ctx->d_stage_bytes = want;
+  }
+  Arena a{static_cast<char *>(ctx->d_stage)};
+  cut(a);
+  return CCGPU_OK;
+}
+
+// one per-frame field of a call whose buffers are in host memory
+struct HostField {
+  size_t bytes;      // per frame
+  const void *host;  // nullptr: the caller left this field out
+  bool out;          // copied back after the launch (else copied in before it)
+};
+
+// Decodes `frames` frames from and into host buffers.  Chunks rotate over the kSlots staging slots, so that the
+// copy-in of one chunk, the decode of the next and the copy-out of a third overlap.  launch(dev, nf, stream, slot)
+// runs nf frames on `stream` over the slot's device copies dev[i] of the fields (nullptr where a field is absent).
+template <size_t N, class Launch>
+int host_pipeline(ccgpu_ctx *ctx, uint64_t frames, const HostField (&fields)[N], Launch &&launch) {
+  size_t per_frame = 0;
+  for (const HostField &f : fields) per_frame += f.host ? f.bytes : 0;
+  const uint64_t chunk = std::max<uint64_t>(1024, std::min<uint64_t>((frames + 15) / 16, (size_t(32) << 20) / per_frame));
+  void *dev[N];
+  auto cut = [&](void *base) {
+    Arena a{static_cast<char *>(base)};
+    for (size_t i = 0; i < N; ++i) dev[i] = a.take<char>(chunk * fields[i].bytes, fields[i].host != nullptr);
+    return a.used;
+  };
+  int rc = ensure_slots(ctx, cut(nullptr));
+  if (rc) return rc;
+  CU(cudaEventRecord(ctx->main_ready, ctx->stream));
+  for (int s = 0; s < kSlots; ++s) CU(cudaStreamWaitEvent(ctx->slot_stream[s], ctx->main_ready, 0));
+  int slot = 0;
+  for (uint64_t f0 = 0; f0 < frames; f0 += chunk, slot = (slot + 1) % kSlots) {
+    const uint64_t nf = std::min(chunk, frames - f0);
+    cudaStream_t st = ctx->slot_stream[slot];
+    cut(ctx->slot_buf[slot]);
+    for (size_t i = 0; i < N; ++i)
+      if (fields[i].host && !fields[i].out)
+        CU(cudaMemcpyAsync(dev[i], static_cast<const char *>(fields[i].host) + f0 * fields[i].bytes, nf * fields[i].bytes,
+                           cudaMemcpyHostToDevice, st));
+    rc = launch(dev, nf, st, slot);
+    if (rc) return rc;
+    for (size_t i = 0; i < N; ++i)
+      if (fields[i].host && fields[i].out)
+        CU(cudaMemcpyAsync(static_cast<char *>(const_cast<void *>(fields[i].host)) + f0 * fields[i].bytes, dev[i],
+                           nf * fields[i].bytes, cudaMemcpyDeviceToHost, st));
+  }
+  for (int s = 0; s < kSlots; ++s) CU(cudaStreamSynchronize(ctx->slot_stream[s]));
+  return CCGPU_OK;
+}
+
+// Runs body(counters) on the device counters (ccgpu_counters layout) to accumulate into: `out` itself when it is
+// device memory, else the context's scratch counters, zeroed before and copied into *out after.
+template <class Body>
+int with_counters(ccgpu_ctx *ctx, ccgpu_counters *out, Body &&body) {
+  if (is_device_ptr(out)) return body(reinterpret_cast<unsigned long long *>(out));
+  CU(cudaMemsetAsync(ctx->d_counters, 0, sizeof(ccgpu_counters), ctx->stream));
+  const int rc = body(ctx->d_counters);
+  if (rc) return rc;
+  CU(cudaMemcpyAsync(ctx->h_counters, ctx->d_counters, sizeof(ccgpu_counters), cudaMemcpyDeviceToHost, ctx->stream));
+  CU(cudaStreamSynchronize(ctx->stream));
+  *out = *ctx->h_counters;
   return CCGPU_OK;
 }
 
@@ -467,19 +562,24 @@ void select_cyclic(ccgpu_code *c) {
   }
 }
 
-int finish_code(ccgpu_ctx *ctx, ccgpu_code *c) {
-  c->ctx = ctx;
+// everything derived from H: shape, coverage, column weight and, on a context, the kernel choice and the CSR tables
+int refresh_H(ccgpu_code *c) {
   c->shape = analyse_H(c->spec.H.data(), c->spec.rows, c->spec.n);
   c->all_columns_covered = columns_covered(c->spec);
   c->max_col_weight = max_column_weight(c->spec);
-  if (!ctx) return CCGPU_OK;  // host-only description: no device tables, no decoding
+  if (!c->ctx) return CCGPU_OK;  // host-only description: no device tables, no decoding
   select_cyclic(c);
-  int rc = ms_csr_upload(c->spec.H.data(), c->spec.rows, c->spec.n, &c->csr);
-  if (rc != 0) return fail(ctx, CCGPU_ERR_CUDA, "ms_csr_upload failed");
-  if (c->spec.family != 2) {
-    rc = gf_upload(c->spec, &c->gf);
-    if (rc != 0) return fail(ctx, CCGPU_ERR_CUDA, "gf_upload failed");
-  }
+  ms_csr_free(&c->csr);
+  if (ms_csr_upload(c->spec.H.data(), c->spec.rows, c->spec.n, &c->csr) != 0)
+    return fail(c->ctx, CCGPU_ERR_CUDA, "ms_csr_upload failed");
+  return CCGPU_OK;
+}
+
+int finish_code(ccgpu_ctx *ctx, ccgpu_code *c) {
+  c->ctx = ctx;
+  const int rc = refresh_H(c);
+  if (rc || !ctx || c->spec.family == 2) return rc;
+  if (gf_upload(c->spec, &c->gf) != 0) return fail(ctx, CCGPU_ERR_CUDA, "gf_upload failed");
   return CCGPU_OK;
 }
 
@@ -575,121 +675,118 @@ int launch_ms(ccgpu_ctx *ctx, const ccgpu_code *c, const ccgpu_ms_params *p, MsP
     const int rc = check_params_q(ctx, c, p);
     if (rc) return rc;
   }
+  const MsCyclicEntry *e;
+  uint64_t per_cta;
+  int grid_max;
+  size_t smem;
   // small codes: one lane per frame (ms_cyclic_lane.cuh) for frames from HBM or the Philox channel; the exhaustive
   // bit-flip source and the self-correcting flavour stay on the warp kernel
   if (ctx->opt_lane != 0 && c->lane[vn] && mp.src != SRC_BITFLIP) {
-    const MsCyclicEntry *e = c->lane[vn];
-    const uint64_t want = (mp.frames + e->threads - 1) / e->threads;
-    const unsigned grid = static_cast<unsigned>(std::min<uint64_t>(want, c->lane_grid_max[vn]));
-    CU(cudaMemsetAsync(work, 0, sizeof(unsigned long long), stream));
-    mp.work = work;
-    const uint64_t warps = uint64_t(grid) * (e->threads / 32);
-    unsigned shift = 0;
-    while ((uint64_t(1) << shift) < 4 * warps) ++shift;
-    mp.work_batch = ctx->opt_work_batch > 0 ? static_cast<unsigned>(ctx->opt_work_batch) : 32;
-    mp.work_shift = shift;
-    void *args[] = { &mp };
-    CU(cudaLaunchKernel(reinterpret_cast<const void *>(e->fn), dim3(grid), dim3(e->threads), args, size_t(e->dyn_smem), stream));
-    ctx->launches++;
-    return CCGPU_OK;
-  }
-  // the QUICK instantiation retires all-positive frames without iterating (ms_cyclic.cuh); it pays when such frames
-  // are frequent, i.e. in Monte-Carlo points at high Eb/N0 (the hint is set by ccgpu_awgn_point; CCGPU_QUICK=0/1
-  // overrides it for every path, which is how the parity tests drive both instantiations over the same inputs)
-  // the fixed-point kernels test for all-positive frames at run time when the hint is set; with several frames per
-  // warp all of them must be all-positive at once, which is rare: measured slower there (profiles/r2_notes.md)
-  if (vn == VN_FIX && c->cyc[VN_FIX] && !c->cyc[VN_FIX]->cta && c->cyc[VN_FIX]->fpw != 1) mp.quick_hint = 0;
-  // the float CTA kernel screens groups of frames at any Eb/N0 (ms_cyclic_cta.cuh, grouped mode): no cost where no frame
-  // is all-positive, measured in profiles/r2_notes.md
-  if (c->cyc[vn] && c->cyc[vn]->cta && mp.src == SRC_PHILOX) mp.quick_hint = 1;
-  if (ctx->opt_quick >= 0) mp.quick_hint = ctx->opt_quick;
-  const int vq = (mp.quick_hint && vn != VN_SPA && vn != VN_FIX && mp.L == nullptr && p->stop_rule != CCGPU_STOP_NONE && c->cyc[vn + VN_QUICK] &&
-                  c->cyc[vn] && !c->cyc[vn]->cta && c->cyc[vn + VN_QUICK]->k == c->cyc[vn]->k && c->cyc[vn + VN_QUICK]->fpw == 1)
-                     ? vn + VN_QUICK
-                     : vn;
-  if (c->cyc[vq]) {
-    const MsCyclicEntry *e = c->cyc[vq];
-    const uint64_t per_cta = (e->cta ? 1 : uint64_t(kMsThreads / 32) * e->fpw) * e->slots;
-    const uint64_t want = (mp.frames + per_cta - 1) / per_cta;
-    const unsigned grid = static_cast<unsigned>(std::min<uint64_t>(want, c->grid_max[vq]));
-    CU(cudaMemsetAsync(work, 0, sizeof(unsigned long long), stream));
-    mp.work = work;
-    {  // guided self-scheduling of the frame queue: a warp takes up to 32 frame indices per atomic while more than
-       // 4 x 32 frames per warp are left, fewer towards the end (work_shift = log2(4 x warps))
-      const uint64_t warps = uint64_t(grid) * (e->threads / 32);
-      unsigned shift = 0;
-      while ((uint64_t(1) << shift) < 4 * warps) ++shift;
-      mp.work_batch = 32;
-      mp.work_shift = shift;
-      if (ctx->opt_work_batch > 0) mp.work_batch = static_cast<unsigned>(ctx->opt_work_batch);
+    e = c->lane[vn];
+    per_cta = e->threads;
+    grid_max = c->lane_grid_max[vn];
+    smem = size_t(e->dyn_smem);
+  } else {
+    // the QUICK instantiation retires all-positive frames without iterating (ms_cyclic.cuh); it pays when such frames
+    // are frequent, i.e. in Monte-Carlo points at high Eb/N0 (the hint is set by ccgpu_awgn_point; CCGPU_QUICK=0/1
+    // overrides it for every path, which is how the parity tests drive both instantiations over the same inputs)
+    // the fixed-point kernels test for all-positive frames at run time when the hint is set; with several frames per
+    // warp all of them must be all-positive at once, which is rare: measured slower there (profiles/r2_notes.md)
+    if (vn == VN_FIX && c->cyc[VN_FIX] && !c->cyc[VN_FIX]->cta && c->cyc[VN_FIX]->fpw != 1) mp.quick_hint = 0;
+    // the float CTA kernel screens groups of frames at any Eb/N0 (ms_cyclic_cta.cuh, grouped mode): no cost where no
+    // frame is all-positive, measured in profiles/r2_notes.md
+    if (c->cyc[vn] && c->cyc[vn]->cta && mp.src == SRC_PHILOX) mp.quick_hint = 1;
+    if (ctx->opt_quick >= 0) mp.quick_hint = ctx->opt_quick;
+    const int vq = (mp.quick_hint && vn != VN_SPA && vn != VN_FIX && mp.L == nullptr && p->stop_rule != CCGPU_STOP_NONE && c->cyc[vn + VN_QUICK] &&
+                    c->cyc[vn] && !c->cyc[vn]->cta && c->cyc[vn + VN_QUICK]->k == c->cyc[vn]->k && c->cyc[vn + VN_QUICK]->fpw == 1)
+                       ? vn + VN_QUICK
+                       : vn;
+    e = c->cyc[vq];
+    if (!e) {
+      const int rc = ms_csr_launch(c->csr, mp, ctx->sm_count, stream);
+      if (rc == -3) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "parity-check matrix too large for the CSR kernel");
+      if (rc != 0) return cuda_fail(ctx, cudaGetLastError(), "ms_csr_launch");
+      ctx->launches++;
+      return CCGPU_OK;
     }
-    void *args[] = { &mp };
-    CU(cudaLaunchKernel(reinterpret_cast<const void *>(e->fn), dim3(grid), dim3(e->threads), args, c->smem[vq], stream));
-    ctx->launches++;
-    return CCGPU_OK;
+    per_cta = (e->cta ? 1 : uint64_t(kMsThreads / 32) * e->fpw) * e->slots;
+    grid_max = c->grid_max[vq];
+    smem = c->smem[vq];
   }
-  int rc = ms_csr_launch(c->csr, mp, ctx->sm_count, stream);
-  if (rc == -3) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "parity-check matrix too large for the CSR kernel");
-  if (rc != 0) return cuda_fail(ctx, cudaGetLastError(), "ms_csr_launch");
+  const unsigned grid = static_cast<unsigned>(std::min<uint64_t>((mp.frames + per_cta - 1) / per_cta, grid_max));
+  CU(cudaMemsetAsync(work, 0, sizeof(unsigned long long), stream));
+  mp.work = work;
+  // guided self-scheduling of the frame queue: a warp takes up to 32 frame indices per atomic while more than
+  // 4 x 32 frames per warp are left, fewer towards the end (work_shift = log2(4 x warps))
+  const uint64_t warps = uint64_t(grid) * (e->threads / 32);
+  unsigned shift = 0;
+  while ((uint64_t(1) << shift) < 4 * warps) ++shift;
+  mp.work_batch = ctx->opt_work_batch > 0 ? static_cast<unsigned>(ctx->opt_work_batch) : 32;
+  mp.work_shift = shift;
+  void *args[] = { &mp };
+  CU(cudaLaunchKernel(reinterpret_cast<const void *>(e->fn), dim3(grid), dim3(e->threads), args, smem, stream));
   ctx->launches++;
   return CCGPU_OK;
 }
 
 
-// multiple-bases decoding of `frames` frames whose channel values are in device memory (d_y).  Work buffers come
-// from the stage arena starting at `arena`; outputs are device pointers (L / iter / chosen nullable); when
-// `counters` is given the Monte-Carlo statistics of the all-zero codeword are accumulated as well.
-size_t align256(size_t v) { return (v + 255) & ~size_t(255); }
-size_t mbbp_work_bytes(size_t n, uint32_t nb, uint64_t frames, bool want_L) {
-  return align256(nb * frames * n * sizeof(float)) + (want_L ? align256(nb * frames * n * sizeof(float)) : 0) +
-         align256(nb * frames * n) + 2 * align256(nb * frames) + align256(nb * sizeof(uint32_t));
+// work buffers of multiple-bases decoding: every candidate of `frames` frames, and the rotations
+struct MbbpWork {
+  float *rolled, *L_b;  // L_b only when the caller wants L
+  uint8_t *bits_b, *iter_b, *failed_b;
+  uint32_t *shifts;
+};
+MbbpWork cut_mbbp_work(Arena &a, size_t n, uint32_t nb, uint64_t frames, bool want_L) {
+  return { a.take<float>(nb * frames * n), a.take<float>(nb * frames * n, want_L), a.take<uint8_t>(nb * frames * n),
+           a.take<uint8_t>(nb * frames),   a.take<uint8_t>(nb * frames),           a.take<uint32_t>(nb) };
 }
+// the stage arena of one chunk of multiple-bases decoding: channel values and outputs (iter and chosen also stand in
+// for the ones a device caller leaves out), then the work buffers
+struct MbbpStage {
+  float *y, *L;  // L only when the caller wants L
+  uint8_t *bits, *iter, *failed, *chosen;
+  MbbpWork work;
+};
+MbbpStage cut_mbbp_stage(Arena &a, size_t n, uint32_t nb, uint64_t frames, bool want_L) {
+  return { a.take<float>(frames * n), a.take<float>(frames * n, want_L), a.take<uint8_t>(frames * n),
+           a.take<uint8_t>(frames),   a.take<uint8_t>(frames),           a.take<uint8_t>(frames),
+           cut_mbbp_work(a, n, nb, frames, want_L) };
+}
+
+// multiple-bases decoding of `frames` frames whose channel values are in device memory (d_y), in the work buffers
+// `w` cut for at least `frames` frames; outputs are device pointers (L / iter nullable, L only if w has L_b); when
+// `counters` is given the Monte-Carlo statistics of the all-zero codeword are accumulated as well.
 int mbbp_run(ccgpu_ctx *ctx, const ccgpu_code *code, const ccgpu_ms_params *params, const uint32_t *shifts, uint32_t nb,
-             const float *d_y, uint64_t frames, char *arena, uint8_t *d_bits, float *d_L, uint8_t *d_iter,
+             const float *d_y, uint64_t frames, const MbbpWork &w, uint8_t *d_bits, float *d_L, uint8_t *d_iter,
              uint8_t *d_failed, uint8_t *d_chosen, unsigned long long *counters) {
   const size_t n = code->spec.n;
-  float *rolled = reinterpret_cast<float *>(arena);
-  arena += align256(nb * frames * n * sizeof(float));
-  float *L_b = nullptr;
-  if (d_L) {
-    L_b = reinterpret_cast<float *>(arena);
-    arena += align256(nb * frames * n * sizeof(float));
-  }
-  uint8_t *bits_b = reinterpret_cast<uint8_t *>(arena);
-  arena += align256(nb * frames * n);
-  uint8_t *iter_b = reinterpret_cast<uint8_t *>(arena);
-  arena += align256(nb * frames);
-  uint8_t *failed_b = reinterpret_cast<uint8_t *>(arena);
-  arena += align256(nb * frames);
-  uint32_t *d_shifts = reinterpret_cast<uint32_t *>(arena);
-  CU(cudaMemcpyAsync(d_shifts, shifts, nb * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
-  const unsigned wide = static_cast<unsigned>(std::min<uint64_t>((nb * frames * n + 255) / 256, uint64_t(ctx->sm_count) * 16));
-  mbbp_roll_kernel<<<std::max(1u, wide), 256, 0, ctx->stream>>>(d_y, rolled, d_shifts, static_cast<uint32_t>(n), nb, frames);
+  CU(cudaMemcpyAsync(w.shifts, shifts, nb * sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
+  mbbp_roll_kernel<<<grid_for(ctx, nb * frames * n, 256), 256, 0, ctx->stream>>>(d_y, w.rolled, w.shifts,
+                                                                                static_cast<uint32_t>(n), nb, frames);
   CU(cudaGetLastError());
   MsParams mp{};
   fill_decoder(mp, code, params);
   mp.src = SRC_HBM;
   mp.frames = nb * frames;
-  mp.y = rolled;
-  mp.bits = bits_b;
-  mp.L = L_b;
-  mp.iter = iter_b;
-  mp.failed = failed_b;
+  mp.y = w.rolled;
+  mp.bits = w.bits_b;
+  mp.L = w.L_b;
+  mp.iter = w.iter_b;
+  mp.failed = w.failed_b;
   const int rc = launch_ms(ctx, code, params, mp);
   if (rc) return rc;
-  const unsigned per_frame = static_cast<unsigned>(std::min<uint64_t>((frames + 127) / 128, uint64_t(ctx->sm_count) * 16));
-  mbbp_select_kernel<<<std::max(1u, per_frame), 128, 0, ctx->stream>>>(d_y, bits_b, iter_b, failed_b, d_shifts,
-                                                                      static_cast<uint32_t>(n), nb, params->max_iter, frames,
-                                                                      d_chosen, d_iter, d_failed, counters);
+  mbbp_select_kernel<<<grid_for(ctx, frames, 128), 128, 0, ctx->stream>>>(d_y, w.bits_b, w.iter_b, w.failed_b, w.shifts,
+                                                                         static_cast<uint32_t>(n), nb, params->max_iter,
+                                                                         frames, d_chosen, d_iter, d_failed, counters);
   CU(cudaGetLastError());
-  const unsigned narrow = static_cast<unsigned>(std::min<uint64_t>((frames * n + 255) / 256, uint64_t(ctx->sm_count) * 16));
-  mbbp_unroll_kernel<<<std::max(1u, narrow), 256, 0, ctx->stream>>>(bits_b, L_b, d_chosen, d_shifts, static_cast<uint32_t>(n), nb,
-                                                                    frames, d_bits, d_L);
+  mbbp_unroll_kernel<<<grid_for(ctx, frames * n, 256), 256, 0, ctx->stream>>>(w.bits_b, w.L_b, d_chosen, w.shifts,
+                                                                              static_cast<uint32_t>(n), nb, frames, d_bits,
+                                                                              d_L);
   CU(cudaGetLastError());
   ctx->launches += 3;
   if (counters) {
-    count_words_kernel<<<static_cast<unsigned>(std::min<uint64_t>((frames + 7) / 8, uint64_t(ctx->sm_count) * 8)), 256, 0,
-                         ctx->stream>>>(d_bits, d_failed, static_cast<uint32_t>(n), frames, counters);
+    count_words_kernel<<<grid_for(ctx, frames, 8, 8), 256, 0, ctx->stream>>>(d_bits, d_failed, static_cast<uint32_t>(n),
+                                                                             frames, counters);
     CU(cudaGetLastError());
     ctx->launches++;
   }
@@ -748,7 +845,6 @@ void ccgpu_destroy(ccgpu_ctx *ctx) {
       cudaStreamSynchronize(ctx->slot_stream[s]);
       cudaStreamDestroy(ctx->slot_stream[s]);
     }
-    if (ctx->slot_done[s]) cudaEventDestroy(ctx->slot_done[s]);
     if (ctx->slot_buf[s]) cudaFree(ctx->slot_buf[s]);
   }
   if (ctx->main_ready) cudaEventDestroy(ctx->main_ready);
@@ -873,18 +969,11 @@ int ccgpu_code_set_rows(ccgpu_code *code, uint32_t rows) {
   } catch (const std::exception &e) {
     return fail(ctx, CCGPU_ERR_INVALID, e.what());
   }
-  code->shape = analyse_H(code->spec.H.data(), code->spec.rows, code->spec.n);
-  code->all_columns_covered = columns_covered(code->spec);
-  code->max_col_weight = max_column_weight(code->spec);
-  if (!ctx) return CCGPU_OK;
-  cudaSetDevice(ctx->device);
-  cudaStreamSynchronize(ctx->stream);
-  ms_csr_free(&code->csr);
-  code->shape = analyse_H(code->spec.H.data(), code->spec.rows, code->spec.n);
-  select_cyclic(code);
-  if (ms_csr_upload(code->spec.H.data(), code->spec.rows, code->spec.n, &code->csr) != 0)
-    return fail(ctx, CCGPU_ERR_CUDA, "ms_csr_upload failed");
-  return CCGPU_OK;
+  if (ctx) {  // the kernels of earlier calls may still read the CSR tables
+    cudaSetDevice(ctx->device);
+    cudaStreamSynchronize(ctx->stream);
+  }
+  return refresh_H(code);
 }
 
 void ccgpu_code_destroy(ccgpu_code *code) {
@@ -1075,10 +1164,8 @@ static int decode_llr_impl(ccgpu_ctx *ctx, const ccgpu_code *code, const ccgpu_m
   fill_decoder(mp, code, params);
   mp.src = SRC_HBM;
   mp.frames = frames;
-  const bool dev = is_device_ptr(y);
-  if (dev) {
-    if ((bits && !is_device_ptr(bits)) || (failed && !is_device_ptr(failed)) || (L && !is_device_ptr(L)) ||
-        (iter && !is_device_ptr(iter)) || (packed && !is_device_ptr(packed)) || (status && !is_device_ptr(status)))
+  if (is_device_ptr(y)) {
+    if (!same_residency(true, {bits, failed, L, iter, packed, status}))
       return fail(ctx, CCGPU_ERR_INVALID, "y is a device pointer: every output must be one too");
     mp.y = y;
     mp.bits = bits;
@@ -1089,65 +1176,34 @@ static int decode_llr_impl(ccgpu_ctx *ctx, const ccgpu_code *code, const ccgpu_m
     mp.status = status;
     return launch_ms(ctx, code, params, mp);
   }
-  // host buffers: chunks rotate over the staging slots so that copies and decoding overlap
-  const size_t per_frame = n * sizeof(float) + (L ? n * sizeof(float) : 0) + (packed ? npw * sizeof(uint32_t) : 0) +
-                           (bits ? n : 0) + (iter ? 1 : 0) + (failed ? 1 : 0) + (status ? 1 : 0);
-  const uint64_t chunk = std::max<uint64_t>(1024, std::min<uint64_t>((frames + 15) / 16, (size_t(32) << 20) / per_frame));
-  rc = ensure_slots(ctx, chunk * per_frame + 256);
-  if (rc) return rc;
-  CU(cudaEventRecord(ctx->main_ready, ctx->stream));
-  for (int s = 0; s < kSlots; ++s) CU(cudaStreamWaitEvent(ctx->slot_stream[s], ctx->main_ready, 0));
-  int slot = 0;
-  for (uint64_t f0 = 0; f0 < frames; f0 += chunk, slot = (slot + 1) % kSlots) {
-    const uint64_t nf = std::min(chunk, frames - f0);
-    cudaStream_t st = ctx->slot_stream[slot];
-    char *at = static_cast<char *>(ctx->slot_buf[slot]);  // 4-byte fields first
-    float *d_y = reinterpret_cast<float *>(at);
-    at += chunk * n * sizeof(float);
-    float *d_L = L ? reinterpret_cast<float *>(at) : nullptr;
-    at += L ? chunk * n * sizeof(float) : 0;
-    uint32_t *d_packed = packed ? reinterpret_cast<uint32_t *>(at) : nullptr;
-    at += packed ? chunk * npw * sizeof(uint32_t) : 0;
-    uint8_t *d_bits = bits ? reinterpret_cast<uint8_t *>(at) : nullptr;
-    at += bits ? chunk * n : 0;
-    uint8_t *d_iter = iter ? reinterpret_cast<uint8_t *>(at) : nullptr;
-    at += iter ? chunk : 0;
-    uint8_t *d_failed = failed ? reinterpret_cast<uint8_t *>(at) : nullptr;
-    at += failed ? chunk : 0;
-    uint8_t *d_status = status ? reinterpret_cast<uint8_t *>(at) : nullptr;
-    CU(cudaMemcpyAsync(d_y, y + f0 * n, nf * n * sizeof(float), cudaMemcpyHostToDevice, st));
-    mp.y = d_y;
-    mp.bits = d_bits;
-    mp.L = d_L;
-    mp.iter = d_iter;
-    mp.failed = d_failed;
-    mp.packed = d_packed;
-    mp.status = d_status;
+  const HostField fields[] = { { n * sizeof(float), y, false },       { n * sizeof(float), L, true },
+                               { npw * sizeof(uint32_t), packed, true }, { n, bits, true },
+                               { 1, iter, true },                      { 1, failed, true },
+                               { 1, status, true } };
+  return host_pipeline(ctx, frames, fields, [&](void *const *d, uint64_t nf, cudaStream_t, int slot) {
+    mp.y = static_cast<const float *>(d[0]);
+    mp.L = static_cast<float *>(d[1]);
+    mp.packed = static_cast<uint32_t *>(d[2]);
+    mp.bits = static_cast<uint8_t *>(d[3]);
+    mp.iter = static_cast<uint8_t *>(d[4]);
+    mp.failed = static_cast<uint8_t *>(d[5]);
+    mp.status = static_cast<uint8_t *>(d[6]);
     mp.frames = nf;
-    rc = launch_ms(ctx, code, params, mp, slot);
-    if (rc) return rc;
-    if (bits) CU(cudaMemcpyAsync(bits + f0 * n, d_bits, nf * n, cudaMemcpyDeviceToHost, st));
-    if (L) CU(cudaMemcpyAsync(L + f0 * n, d_L, nf * n * sizeof(float), cudaMemcpyDeviceToHost, st));
-    if (iter) CU(cudaMemcpyAsync(iter + f0, d_iter, nf, cudaMemcpyDeviceToHost, st));
-    if (failed) CU(cudaMemcpyAsync(failed + f0, d_failed, nf, cudaMemcpyDeviceToHost, st));
-    if (packed) CU(cudaMemcpyAsync(packed + f0 * npw, d_packed, nf * npw * sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-    if (status) CU(cudaMemcpyAsync(status + f0, d_status, nf, cudaMemcpyDeviceToHost, st));
-  }
-  for (int s = 0; s < kSlots; ++s) CU(cudaStreamSynchronize(ctx->slot_stream[s]));
-  return CCGPU_OK;
+    return launch_ms(ctx, code, params, mp, slot);
+  });
 }
 
 int ccgpu_decode_llr(ccgpu_ctx *ctx, const ccgpu_code *code, const ccgpu_ms_params *params, const float *y,
                      uint64_t frames, uint8_t *bits, float *L, uint8_t *iter, uint8_t *failed) {
   if (!ctx || !code || !y || !bits || !failed) return fail(ctx, CCGPU_ERR_INVALID, "null argument");
-  if (code->ctx != ctx) return fail(ctx, CCGPU_ERR_INVALID, "code was not created on this context");
+  if (int rc = check_code(ctx, code)) return rc;
   return decode_llr_impl(ctx, code, params, y, frames, bits, L, iter, failed, nullptr, nullptr);
 }
 
 int ccgpu_decode_llr_packed(ccgpu_ctx *ctx, const ccgpu_code *code, const ccgpu_ms_params *params, const float *y,
                             uint64_t frames, uint32_t *packed, uint8_t *status) {
   if (!ctx || !code || !y || !packed || !status) return fail(ctx, CCGPU_ERR_INVALID, "null argument");
-  if (code->ctx != ctx) return fail(ctx, CCGPU_ERR_INVALID, "code was not created on this context");
+  if (int rc = check_code(ctx, code)) return rc;
   return decode_llr_impl(ctx, code, params, y, frames, nullptr, nullptr, nullptr, nullptr, packed, status);
 }
 
@@ -1160,9 +1216,8 @@ int ccgpu_awgn_llr(ccgpu_ctx *ctx, uint32_t n, double sigma, uint64_t seed, uint
   const bool dev = is_device_ptr(y);
   float *d_y = y;
   if (!dev) {
-    const int rc = ensure_stage(ctx, frames * n * sizeof(float));
+    const int rc = cut_stage(ctx, [&](Arena &a) { d_y = a.take<float>(frames * n); });
     if (rc) return rc;
-    d_y = static_cast<float *>(ctx->d_stage);
   }
   const int rc = launch_awgn(ctx, d_y, n, static_cast<float>(sigma), seed, point, frame0, frames);
   if (rc) return rc;
@@ -1173,27 +1228,10 @@ int ccgpu_awgn_llr(ccgpu_ctx *ctx, uint32_t n, double sigma, uint64_t seed, uint
   return CCGPU_OK;
 }
 
-static int counted_launch(ccgpu_ctx *ctx, const ccgpu_code *code, const ccgpu_ms_params *params, MsParams mp,
-                          ccgpu_counters *out) {
-  const bool dev = is_device_ptr(out);
-  if (dev) {
-    mp.counters = reinterpret_cast<unsigned long long *>(out);
-    return launch_ms(ctx, code, params, mp);
-  }
-  CU(cudaMemsetAsync(ctx->d_counters, 0, sizeof(ccgpu_counters), ctx->stream));
-  mp.counters = ctx->d_counters;
-  const int rc = launch_ms(ctx, code, params, mp);
-  if (rc) return rc;
-  CU(cudaMemcpyAsync(ctx->h_counters, ctx->d_counters, sizeof(ccgpu_counters), cudaMemcpyDeviceToHost, ctx->stream));
-  CU(cudaStreamSynchronize(ctx->stream));
-  *out = *ctx->h_counters;
-  return CCGPU_OK;
-}
-
 int ccgpu_awgn_point(ccgpu_ctx *ctx, const ccgpu_code *code, const ccgpu_ms_params *params, double ebno_db,
                      uint64_t seed, uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out) {
   if (!ctx || !code || !out) return fail(ctx, CCGPU_ERR_INVALID, "null argument");
-  if (code->ctx != ctx) return fail(ctx, CCGPU_ERR_INVALID, "code was not created on this context");
+  if (int rc = check_code(ctx, code)) return rc;
   std::lock_guard<std::mutex> g(ctx->mu);
   int rc = check_params(ctx, params);
   if (rc) return rc;
@@ -1223,14 +1261,17 @@ int ccgpu_awgn_point(ccgpu_ctx *ctx, const ccgpu_code *code, const ccgpu_ms_para
   mp.point = point;
   mp.frame0 = frame0;
   mp.frames = frames;
-  return counted_launch(ctx, code, params, mp, out);
+  return with_counters(ctx, out, [&](unsigned long long *counters) {
+    mp.counters = counters;
+    return launch_ms(ctx, code, params, mp);
+  });
 }
 
 int ccgpu_decode_llr_mbbp(ccgpu_ctx *ctx, const ccgpu_code *code, const ccgpu_ms_params *params, const uint32_t *shifts,
                           uint32_t n_bases, const float *y, uint64_t frames, uint8_t *bits, float *L, uint8_t *iter,
                           uint8_t *failed, uint8_t *chosen) {
   if (!ctx || !code || !y || !bits || !failed) return fail(ctx, CCGPU_ERR_INVALID, "null argument");
-  if (code->ctx != ctx) return fail(ctx, CCGPU_ERR_INVALID, "code was not created on this context");
+  if (int rc = check_code(ctx, code)) return rc;
   std::lock_guard<std::mutex> g(ctx->mu);
   int rc = check_params(ctx, params);
   if (rc) return rc;
@@ -1240,39 +1281,31 @@ int ccgpu_decode_llr_mbbp(ccgpu_ctx *ctx, const ccgpu_code *code, const ccgpu_ms
   CU(cudaSetDevice(ctx->device));
   const size_t n = code->spec.n;
   const bool dev = is_device_ptr(y);
-  if (dev && (!is_device_ptr(bits) || !is_device_ptr(failed) || (L && !is_device_ptr(L)) || (iter && !is_device_ptr(iter)) ||
-              (chosen && !is_device_ptr(chosen))))
+  if (dev && !same_residency(true, {bits, failed, L, iter, chosen}))
     return fail(ctx, CCGPU_ERR_INVALID, "y is a device pointer: every output must be one too");
   // chunks bound the work arena (all candidates of a chunk are decoded in one launch)
-  const size_t per_frame = mbbp_work_bytes(n, n_bases, 1, L != nullptr) / 1 + n * (sizeof(float) * 2 + 1) + 3;
+  Arena one;
+  cut_mbbp_work(one, n, n_bases, 1, L != nullptr);
+  const size_t per_frame = one.used + n * (sizeof(float) * 2 + 1) + 3;
   const uint64_t chunk = std::max<uint64_t>(1, std::min<uint64_t>(frames, (size_t(512) << 20) / per_frame));
-  const size_t io = align256(chunk * n * sizeof(float)) * 2 + align256(chunk * n) + 3 * align256(chunk);
-  rc = ensure_stage(ctx, io + mbbp_work_bytes(n, n_bases, chunk, L != nullptr) + 4096);
+  MbbpStage s;
+  rc = cut_stage(ctx, [&](Arena &a) { s = cut_mbbp_stage(a, n, n_bases, chunk, L != nullptr); });
   if (rc) return rc;
-  char *base = static_cast<char *>(ctx->d_stage);
-  float *s_y = reinterpret_cast<float *>(base);
-  float *s_L = reinterpret_cast<float *>(base + align256(chunk * n * sizeof(float)));
-  uint8_t *s_bits = reinterpret_cast<uint8_t *>(base + 2 * align256(chunk * n * sizeof(float)));
-  uint8_t *s_iter = s_bits + align256(chunk * n);
-  uint8_t *s_failed = s_iter + align256(chunk);
-  uint8_t *s_chosen = s_failed + align256(chunk);
-  char *arena = base + io;
   for (uint64_t f0 = 0; f0 < frames; f0 += chunk) {
     const uint64_t nf = std::min(chunk, frames - f0);
     if (dev) {
-      rc = mbbp_run(ctx, code, params, shifts, n_bases, y + f0 * n, nf, arena, bits + f0 * n, L ? L + f0 * n : nullptr,
-                    iter ? iter + f0 : s_iter, failed + f0, chosen ? chosen + f0 : s_chosen, nullptr);
+      rc = mbbp_run(ctx, code, params, shifts, n_bases, y + f0 * n, nf, s.work, bits + f0 * n, L ? L + f0 * n : nullptr,
+                    iter ? iter + f0 : s.iter, failed + f0, chosen ? chosen + f0 : s.chosen, nullptr);
       if (rc) return rc;
     } else {
-      CU(cudaMemcpyAsync(s_y, y + f0 * n, nf * n * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-      rc = mbbp_run(ctx, code, params, shifts, n_bases, s_y, nf, arena, s_bits, L ? s_L : nullptr, s_iter, s_failed, s_chosen,
-                    nullptr);
+      CU(cudaMemcpyAsync(s.y, y + f0 * n, nf * n * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
+      rc = mbbp_run(ctx, code, params, shifts, n_bases, s.y, nf, s.work, s.bits, s.L, s.iter, s.failed, s.chosen, nullptr);
       if (rc) return rc;
-      CU(cudaMemcpyAsync(bits + f0 * n, s_bits, nf * n, cudaMemcpyDeviceToHost, ctx->stream));
-      if (L) CU(cudaMemcpyAsync(L + f0 * n, s_L, nf * n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-      if (iter) CU(cudaMemcpyAsync(iter + f0, s_iter, nf, cudaMemcpyDeviceToHost, ctx->stream));
-      CU(cudaMemcpyAsync(failed + f0, s_failed, nf, cudaMemcpyDeviceToHost, ctx->stream));
-      if (chosen) CU(cudaMemcpyAsync(chosen + f0, s_chosen, nf, cudaMemcpyDeviceToHost, ctx->stream));
+      CU(cudaMemcpyAsync(bits + f0 * n, s.bits, nf * n, cudaMemcpyDeviceToHost, ctx->stream));
+      if (L) CU(cudaMemcpyAsync(L + f0 * n, s.L, nf * n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+      if (iter) CU(cudaMemcpyAsync(iter + f0, s.iter, nf, cudaMemcpyDeviceToHost, ctx->stream));
+      CU(cudaMemcpyAsync(failed + f0, s.failed, nf, cudaMemcpyDeviceToHost, ctx->stream));
+      if (chosen) CU(cudaMemcpyAsync(chosen + f0, s.chosen, nf, cudaMemcpyDeviceToHost, ctx->stream));
       CU(cudaStreamSynchronize(ctx->stream));  // the staging buffers are reused by the next chunk
     }
   }
@@ -1283,43 +1316,33 @@ int ccgpu_awgn_point_mbbp(ccgpu_ctx *ctx, const ccgpu_code *code, const ccgpu_ms
                           uint32_t n_bases, double ebno_db, uint64_t seed, uint32_t point, uint64_t frame0, uint64_t frames,
                           ccgpu_counters *out) {
   if (!ctx || !code || !out) return fail(ctx, CCGPU_ERR_INVALID, "null argument");
-  if (code->ctx != ctx) return fail(ctx, CCGPU_ERR_INVALID, "code was not created on this context");
+  if (int rc = check_code(ctx, code)) return rc;
   std::lock_guard<std::mutex> g(ctx->mu);
   int rc = check_params(ctx, params);
   if (rc) return rc;
   rc = check_bases(ctx, code, shifts, n_bases);
   if (rc) return rc;
   CU(cudaSetDevice(ctx->device));
-  const size_t n = code->spec.n;
-  const bool dev = is_device_ptr(out);
-  unsigned long long *counters = dev ? reinterpret_cast<unsigned long long *>(out) : ctx->d_counters;
-  if (!dev) CU(cudaMemsetAsync(ctx->d_counters, 0, sizeof(ccgpu_counters), ctx->stream));
-  const size_t per_frame = mbbp_work_bytes(n, n_bases, 1, false) + n * (sizeof(float) + 1) + 3;
-  const uint64_t chunk = std::max<uint64_t>(4, std::min<uint64_t>(std::max<uint64_t>(frames, 4), (size_t(512) << 20) / per_frame) & ~uint64_t(3));
-  const size_t io = align256(chunk * n * sizeof(float)) + align256(chunk * n) + 3 * align256(chunk);
-  rc = ensure_stage(ctx, io + mbbp_work_bytes(n, n_bases, chunk, false) + 4096);
-  if (rc) return rc;
-  char *base = static_cast<char *>(ctx->d_stage);
-  float *s_y = reinterpret_cast<float *>(base);
-  uint8_t *s_bits = reinterpret_cast<uint8_t *>(base + align256(chunk * n * sizeof(float)));
-  uint8_t *s_iter = s_bits + align256(chunk * n);
-  uint8_t *s_failed = s_iter + align256(chunk);
-  uint8_t *s_chosen = s_failed + align256(chunk);
-  const float sigma = static_cast<float>(ccgpu_sigma(code->spec.rate, ebno_db));
   if (params->variant == CCGPU_SPA) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "multiple-bases points take the min-sum variants");
-  for (uint64_t f0 = 0; f0 < frames; f0 += chunk) {
-    const uint64_t nf = std::min(chunk, frames - f0);
-    rc = launch_awgn(ctx, s_y, static_cast<uint32_t>(n), sigma, seed, point, frame0 + f0, nf);
+  const size_t n = code->spec.n;
+  Arena one;
+  cut_mbbp_work(one, n, n_bases, 1, false);
+  const size_t per_frame = one.used + n * (sizeof(float) + 1) + 3;
+  const uint64_t chunk = std::max<uint64_t>(4, std::min<uint64_t>(std::max<uint64_t>(frames, 4), (size_t(512) << 20) / per_frame) & ~uint64_t(3));
+  const float sigma = static_cast<float>(ccgpu_sigma(code->spec.rate, ebno_db));
+  return with_counters(ctx, out, [&](unsigned long long *counters) -> int {
+    MbbpStage s;
+    rc = cut_stage(ctx, [&](Arena &a) { s = cut_mbbp_stage(a, n, n_bases, chunk, false); });
     if (rc) return rc;
-    rc = mbbp_run(ctx, code, params, shifts, n_bases, s_y, nf, base + io, s_bits, nullptr, s_iter, s_failed, s_chosen, counters);
-    if (rc) return rc;
-  }
-  if (!dev) {
-    CU(cudaMemcpyAsync(ctx->h_counters, ctx->d_counters, sizeof(ccgpu_counters), cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    *out = *ctx->h_counters;
-  }
-  return CCGPU_OK;
+    for (uint64_t f0 = 0; f0 < frames; f0 += chunk) {
+      const uint64_t nf = std::min(chunk, frames - f0);
+      rc = launch_awgn(ctx, s.y, static_cast<uint32_t>(n), sigma, seed, point, frame0 + f0, nf);
+      if (rc) return rc;
+      rc = mbbp_run(ctx, code, params, shifts, n_bases, s.y, nf, s.work, s.bits, nullptr, s.iter, s.failed, s.chosen, counters);
+      if (rc) return rc;
+    }
+    return CCGPU_OK;
+  });
 }
 
 int ccgpu_awgn_point_uncoded(ccgpu_ctx *ctx, uint32_t n, double rate, double ebno_db, uint64_t seed, uint32_t point,
@@ -1328,28 +1351,21 @@ int ccgpu_awgn_point_uncoded(ccgpu_ctx *ctx, uint32_t n, double rate, double ebn
   if (!(rate > 0.0)) return fail(ctx, CCGPU_ERR_INVALID, "rate must be positive");
   std::lock_guard<std::mutex> g(ctx->mu);
   CU(cudaSetDevice(ctx->device));
-  const bool dev = is_device_ptr(out);
-  unsigned long long *counters = dev ? reinterpret_cast<unsigned long long *>(out) : ctx->d_counters;
-  if (!dev) CU(cudaMemsetAsync(ctx->d_counters, 0, sizeof(ccgpu_counters), ctx->stream));
-  if (frames) {
-    const unsigned grid = static_cast<unsigned>(std::min<uint64_t>((frames + 7) / 8, uint64_t(ctx->sm_count) * 8));
-    awgn_uncoded_kernel<<<grid, 256, 0, ctx->stream>>>(n, static_cast<float>(ccgpu_sigma(rate, ebno_db)), philox_round_keys(seed),
-                                                       point, frame0, frames, counters);
-    CU(cudaGetLastError());
-    ctx->launches++;
-  }
-  if (!dev) {
-    CU(cudaMemcpyAsync(ctx->h_counters, ctx->d_counters, sizeof(ccgpu_counters), cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    *out = *ctx->h_counters;
-  }
-  return CCGPU_OK;
+  return with_counters(ctx, out, [&](unsigned long long *counters) -> int {
+    if (frames) {
+      awgn_uncoded_kernel<<<grid_for(ctx, frames, 8, 8), 256, 0, ctx->stream>>>(
+          n, static_cast<float>(ccgpu_sigma(rate, ebno_db)), philox_round_keys(seed), point, frame0, frames, counters);
+      CU(cudaGetLastError());
+      ctx->launches++;
+    }
+    return CCGPU_OK;
+  });
 }
 
 int ccgpu_bitflip_point(ccgpu_ctx *ctx, const ccgpu_code *code, const ccgpu_ms_params *params, uint32_t weight,
                         uint64_t first, uint64_t count, ccgpu_counters *out) {
   if (!ctx || !code || !out) return fail(ctx, CCGPU_ERR_INVALID, "null argument");
-  if (code->ctx != ctx) return fail(ctx, CCGPU_ERR_INVALID, "code was not created on this context");
+  if (int rc = check_code(ctx, code)) return rc;
   std::lock_guard<std::mutex> g(ctx->mu);
   int rc = check_params(ctx, params);
   if (rc) return rc;
@@ -1368,14 +1384,24 @@ int ccgpu_bitflip_point(ccgpu_ctx *ctx, const ccgpu_code *code, const ccgpu_ms_p
   mp.flip_weight = weight;
   mp.frame0 = first;
   mp.frames = count;
-  return counted_launch(ctx, code, params, mp, out);
+  return with_counters(ctx, out, [&](unsigned long long *counters) {
+    mp.counters = counters;
+    return launch_ms(ctx, code, params, mp);
+  });
+}
+
+static int gf_rc(ccgpu_ctx *ctx, int rc) {
+  if (rc == -3) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "code not supported by the algebraic kernel (t <= 31, 2t <= 64, step = 1)");
+  if (rc != 0) return cuda_fail(ctx, cudaGetLastError(), "gf_launch");
+  ctx->launches++;
+  return CCGPU_OK;
 }
 
 int ccgpu_gf_decode_erasures(ccgpu_ctx *ctx, const ccgpu_code *code, const uint8_t *words, uint64_t count,
                              const uint8_t *erasure_pos, const uint8_t *erasure_cnt, uint32_t max_erasures,
                              uint8_t *corrected, uint8_t *n_errors, uint8_t *failed) {
   if (!ctx || !code || !words || !corrected || !failed) return fail(ctx, CCGPU_ERR_INVALID, "null argument");
-  if (code->ctx != ctx) return fail(ctx, CCGPU_ERR_INVALID, "code was not created on this context");
+  if (int rc = check_code(ctx, code)) return rc;
   if (code->spec.family == 2) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "algebraic decoding needs a BCH/RS code");
   if ((erasure_pos == nullptr) != (erasure_cnt == nullptr)) return fail(ctx, CCGPU_ERR_INVALID, "erasure_pos and erasure_cnt go together");
   if (erasure_pos && (max_erasures == 0 || max_erasures > 30)) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "max_erasures must be in 1..30");
@@ -1383,52 +1409,20 @@ int ccgpu_gf_decode_erasures(ccgpu_ctx *ctx, const ccgpu_code *code, const uint8
   if (count == 0) return CCGPU_OK;
   CU(cudaSetDevice(ctx->device));
   const size_t n = code->spec.n;
-  const size_t me = erasure_pos ? max_erasures : 0;
-  const bool dev = is_device_ptr(words);
-  auto launch = [&](const uint8_t *w, uint64_t cnt, const uint8_t *ep, const uint8_t *ec, uint8_t *out, uint8_t *ne, uint8_t *fl,
-                    cudaStream_t st) -> int {
-    const int rc = gf_launch(code->gf, w, cnt, ep, ec, static_cast<int>(me), out, ne, fl, ctx->sm_count, st);
-    if (rc == -3) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "code not supported by the algebraic kernel (t <= 31, 2t <= 64, step = 1)");
-    if (rc != 0) return cuda_fail(ctx, cudaGetLastError(), "gf_launch");
-    ctx->launches++;
-    return CCGPU_OK;
-  };
-  if (dev) {
-    if (!is_device_ptr(corrected) || !is_device_ptr(failed) || (n_errors && !is_device_ptr(n_errors)) ||
-        (erasure_pos && (!is_device_ptr(erasure_pos) || !is_device_ptr(erasure_cnt))))
+  const int me = erasure_pos ? static_cast<int>(max_erasures) : 0;
+  if (is_device_ptr(words)) {
+    if (!same_residency(true, {corrected, failed, n_errors, erasure_pos, erasure_cnt}))
       return fail(ctx, CCGPU_ERR_INVALID, "words is a device pointer: every other buffer must be one too");
-    return launch(words, count, erasure_pos, erasure_cnt, corrected, n_errors, failed, ctx->stream);
+    return gf_rc(ctx, gf_launch(code->gf, words, count, erasure_pos, erasure_cnt, me, corrected, n_errors, failed,
+                                ctx->sm_count, ctx->stream));
   }
-  // host buffers: chunks alternate between two slots so that copies and decoding overlap
-  const size_t per_word = 2 * n + 2 + me + (me ? 1 : 0);
-  const uint64_t chunk = std::max<uint64_t>(1024, std::min<uint64_t>((count + 15) / 16, (size_t(32) << 20) / per_word));
-  int rc = ensure_slots(ctx, chunk * per_word + 256);
-  if (rc) return rc;
-  CU(cudaEventRecord(ctx->main_ready, ctx->stream));
-  for (int s = 0; s < kSlots; ++s) CU(cudaStreamWaitEvent(ctx->slot_stream[s], ctx->main_ready, 0));
-  int slot = 0;
-  for (uint64_t w0 = 0; w0 < count; w0 += chunk, slot = (slot + 1) % kSlots) {
-    const uint64_t nw = std::min(chunk, count - w0);
-    cudaStream_t st = ctx->slot_stream[slot];
-    uint8_t *d_in = static_cast<uint8_t *>(ctx->slot_buf[slot]);
-    uint8_t *d_out = d_in + chunk * n;
-    uint8_t *d_ne = d_out + chunk * n;
-    uint8_t *d_fail = d_ne + chunk;
-    uint8_t *d_ep = me ? d_fail + chunk : nullptr;
-    uint8_t *d_ec = me ? d_ep + chunk * me : nullptr;
-    CU(cudaMemcpyAsync(d_in, words + w0 * n, nw * n, cudaMemcpyHostToDevice, st));
-    if (me) {
-      CU(cudaMemcpyAsync(d_ep, erasure_pos + w0 * me, nw * me, cudaMemcpyHostToDevice, st));
-      CU(cudaMemcpyAsync(d_ec, erasure_cnt + w0, nw, cudaMemcpyHostToDevice, st));
-    }
-    rc = launch(d_in, nw, d_ep, d_ec, d_out, d_ne, d_fail, st);
-    if (rc) return rc;
-    CU(cudaMemcpyAsync(corrected + w0 * n, d_out, nw * n, cudaMemcpyDeviceToHost, st));
-    if (n_errors) CU(cudaMemcpyAsync(n_errors + w0, d_ne, nw, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(failed + w0, d_fail, nw, cudaMemcpyDeviceToHost, st));
-  }
-  for (int s = 0; s < kSlots; ++s) CU(cudaStreamSynchronize(ctx->slot_stream[s]));
-  return CCGPU_OK;
+  const HostField fields[] = { { n, words, false },  { size_t(me), erasure_pos, false }, { 1, erasure_cnt, false },
+                               { n, corrected, true }, { 1, n_errors, true },             { 1, failed, true } };
+  return host_pipeline(ctx, count, fields, [&](void *const *d, uint64_t nw, cudaStream_t st, int) {
+    return gf_rc(ctx, gf_launch(code->gf, static_cast<const uint8_t *>(d[0]), nw, static_cast<const uint8_t *>(d[1]),
+                                static_cast<const uint8_t *>(d[2]), me, static_cast<uint8_t *>(d[3]),
+                                static_cast<uint8_t *>(d[4]), static_cast<uint8_t *>(d[5]), ctx->sm_count, st));
+  });
 }
 
 int ccgpu_gf_decode_erasures_pgz(ccgpu_ctx *ctx, const ccgpu_code *code, const uint8_t *words, uint64_t count,
@@ -1436,7 +1430,7 @@ int ccgpu_gf_decode_erasures_pgz(ccgpu_ctx *ctx, const ccgpu_code *code, const u
                                  uint8_t *corrected, uint8_t *n_errors, uint8_t *failed) {
   if (!ctx || !code || !words || !corrected || !failed || !erasure_pos || !erasure_cnt)
     return fail(ctx, CCGPU_ERR_INVALID, "null argument");
-  if (code->ctx != ctx) return fail(ctx, CCGPU_ERR_INVALID, "code was not created on this context");
+  if (int rc = check_code(ctx, code)) return rc;
   if (code->spec.family != 0) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "the zero/one fill rule is for binary BCH codes");
   if (max_erasures == 0 || max_erasures > 255) return fail(ctx, CCGPU_ERR_INVALID, "max_erasures must be in 1..255");
   std::lock_guard<std::mutex> g(ctx->mu);
@@ -1444,25 +1438,25 @@ int ccgpu_gf_decode_erasures_pgz(ccgpu_ctx *ctx, const ccgpu_code *code, const u
   CU(cudaSetDevice(ctx->device));
   const size_t n = code->spec.n, me = max_erasures;
   const bool dev = is_device_ptr(words);
-  if (dev && (!is_device_ptr(corrected) || !is_device_ptr(failed) || (n_errors && !is_device_ptr(n_errors)) ||
-              !is_device_ptr(erasure_pos) || !is_device_ptr(erasure_cnt)))
+  if (dev && !same_residency(true, {corrected, failed, n_errors, erasure_pos, erasure_cnt}))
     return fail(ctx, CCGPU_ERR_INVALID, "words is a device pointer: every other buffer must be one too");
   const size_t per_word = 4 * n + 4 + (dev ? 0 : 2 * n + 3 + me);
   const uint64_t chunk = std::max<uint64_t>(1, std::min<uint64_t>(count, (size_t(256) << 20) / per_word));
-  const size_t work = 2 * align256(2 * chunk * n) + 2 * align256(2 * chunk);
-  const size_t staging = dev ? 0 : 2 * align256(chunk * n) + 3 * align256(chunk) + align256(chunk * me);
-  int rc = ensure_stage(ctx, work + staging + 256);
+  // both fills of every word, the decoder's outputs for them, then the staging of host buffers
+  uint8_t *d_fill, *d_cand, *d_cne, *d_cfail, *s_in, *s_out, *s_ne, *s_fail, *s_ec, *s_ep;
+  int rc = cut_stage(ctx, [&](Arena &a) {
+    d_fill = a.take<uint8_t>(2 * chunk * n);
+    d_cand = a.take<uint8_t>(2 * chunk * n);
+    d_cne = a.take<uint8_t>(2 * chunk);
+    d_cfail = a.take<uint8_t>(2 * chunk);
+    s_in = a.take<uint8_t>(chunk * n, !dev);
+    s_out = a.take<uint8_t>(chunk * n, !dev);
+    s_ne = a.take<uint8_t>(chunk, !dev);
+    s_fail = a.take<uint8_t>(chunk, !dev);
+    s_ec = a.take<uint8_t>(chunk, !dev);
+    s_ep = a.take<uint8_t>(chunk * me, !dev);
+  });
   if (rc) return rc;
-  uint8_t *d_fill = static_cast<uint8_t *>(ctx->d_stage);  // both fills of every word, then the decoder's outputs for them
-  uint8_t *d_cand = d_fill + align256(2 * chunk * n);
-  uint8_t *d_cne = d_cand + align256(2 * chunk * n);
-  uint8_t *d_cfail = d_cne + align256(2 * chunk);
-  uint8_t *s_in = d_cfail + align256(2 * chunk);  // staging for host buffers
-  uint8_t *s_out = s_in + align256(chunk * n);
-  uint8_t *s_ne = s_out + align256(chunk * n);
-  uint8_t *s_fail = s_ne + align256(chunk);
-  uint8_t *s_ec = s_fail + align256(chunk);
-  uint8_t *s_ep = s_ec + align256(chunk);
   for (uint64_t w0 = 0; w0 < count; w0 += chunk) {
     const uint64_t nw = std::min(chunk, count - w0);
     const uint8_t *in = words + w0 * n, *ep = erasure_pos + w0 * me, *ec = erasure_cnt + w0;
@@ -1473,16 +1467,15 @@ int ccgpu_gf_decode_erasures_pgz(ccgpu_ctx *ctx, const ccgpu_code *code, const u
       CU(cudaMemcpyAsync(s_ec, ec, nw, cudaMemcpyHostToDevice, ctx->stream));
       in = s_in, ep = s_ep, ec = s_ec, out = s_out, ne = s_ne, fl = s_fail;
     }
-    const unsigned grid = static_cast<unsigned>(std::min<uint64_t>((nw * n + 255) / 256, uint64_t(ctx->sm_count) * 16));
+    const unsigned grid = grid_for(ctx, nw * n, 256);
     pgz_fill_kernel<<<grid, 256, 0, ctx->stream>>>(in, ep, ec, static_cast<uint32_t>(me), static_cast<uint32_t>(n), nw, d_fill);
     CU(cudaGetLastError());
-    const int grc = gf_launch(code->gf, d_fill, 2 * nw, nullptr, nullptr, 0, d_cand, d_cne, d_cfail, ctx->sm_count, ctx->stream);
-    if (grc == -3) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "code not supported by the algebraic kernel (t <= 31, 2t <= 64, step = 1)");
-    if (grc != 0) return cuda_fail(ctx, cudaGetLastError(), "gf_launch");
+    rc = gf_rc(ctx, gf_launch(code->gf, d_fill, 2 * nw, nullptr, nullptr, 0, d_cand, d_cne, d_cfail, ctx->sm_count, ctx->stream));
+    if (rc) return rc;
     pgz_select_kernel<<<grid, 256, 0, ctx->stream>>>(in, d_cand, d_cne, d_cfail, ec, code->spec.t, static_cast<uint32_t>(n), nw, out,
                                                      ne, fl);
     CU(cudaGetLastError());
-    ctx->launches += 3;
+    ctx->launches += 2;
     if (!dev) {
       CU(cudaMemcpyAsync(corrected + w0 * n, s_out, nw * n, cudaMemcpyDeviceToHost, ctx->stream));
       if (n_errors) CU(cudaMemcpyAsync(n_errors + w0, s_ne, nw, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1501,47 +1494,41 @@ int ccgpu_gf_decode(ccgpu_ctx *ctx, const ccgpu_code *code, const uint8_t *words
 int ccgpu_awgn_point_hard(ccgpu_ctx *ctx, const ccgpu_code *code, double ebno_db, uint64_t seed, uint32_t point,
                           uint64_t frame0, uint64_t frames, ccgpu_counters *out) {
   if (!ctx || !code || !out) return fail(ctx, CCGPU_ERR_INVALID, "null argument");
-  if (code->ctx != ctx) return fail(ctx, CCGPU_ERR_INVALID, "code was not created on this context");
+  if (int rc = check_code(ctx, code)) return rc;
   if (code->spec.family != 0) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "hard-decision AWGN points need a binary BCH code");
   std::lock_guard<std::mutex> g(ctx->mu);
   CU(cudaSetDevice(ctx->device));
   const size_t n = code->spec.n;
-  const bool dev = is_device_ptr(out);
-  unsigned long long *counters = dev ? reinterpret_cast<unsigned long long *>(out) : ctx->d_counters;
-  if (!dev) CU(cudaMemsetAsync(ctx->d_counters, 0, sizeof(ccgpu_counters), ctx->stream));
   const uint64_t chunk = std::min<uint64_t>(std::max<uint64_t>(frames, 1), uint64_t(1) << 22);
-  int rc = ensure_stage(ctx, chunk * (2 * n + 2) + 64);
-  if (rc) return rc;
-  uint8_t *d_words = static_cast<uint8_t *>(ctx->d_stage);
-  uint8_t *d_out = d_words + chunk * n;
-  uint8_t *d_ne = d_out + chunk * n;
-  uint8_t *d_fail = d_ne + chunk;
   const float sigma = static_cast<float>(ccgpu_sigma(code->spec.rate, ebno_db));
-  for (uint64_t f0 = 0; f0 < frames; f0 += chunk) {
-    const uint64_t nf = std::min(chunk, frames - f0);
-    const uint64_t blocks = (nf * ((n + 3) / 4) + kAwgnThreads - 1) / kAwgnThreads;
-    awgn_hard_kernel<<<static_cast<unsigned>(std::min<uint64_t>(blocks, uint64_t(ctx->sm_count) * 16)), kAwgnThreads, 0,
-                       ctx->stream>>>(d_words, static_cast<uint32_t>(n), sigma, seed, point, frame0 + f0, nf);
-    CU(cudaGetLastError());
-    rc = gf_launch(code->gf, d_words, nf, nullptr, nullptr, 0, d_out, d_ne, d_fail, ctx->sm_count, ctx->stream);
-    if (rc == -3) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "code not supported by the algebraic kernel");
-    if (rc != 0) return cuda_fail(ctx, cudaGetLastError(), "gf_launch");
-    count_words_kernel<<<static_cast<unsigned>(std::min<uint64_t>((nf + 7) / 8, uint64_t(ctx->sm_count) * 8)), 256, 0, ctx->stream>>>(
-        d_out, d_fail, static_cast<uint32_t>(n), nf, counters);
-    CU(cudaGetLastError());
-    ctx->launches += 3;
-  }
-  if (!dev) {
-    CU(cudaMemcpyAsync(ctx->h_counters, ctx->d_counters, sizeof(ccgpu_counters), cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    *out = *ctx->h_counters;
-  }
-  return CCGPU_OK;
+  return with_counters(ctx, out, [&](unsigned long long *counters) -> int {
+    uint8_t *d_words, *d_out, *d_ne, *d_fail;
+    int rc = cut_stage(ctx, [&](Arena &a) {
+      d_words = a.take<uint8_t>(chunk * n);
+      d_out = a.take<uint8_t>(chunk * n);
+      d_ne = a.take<uint8_t>(chunk);
+      d_fail = a.take<uint8_t>(chunk);
+    });
+    if (rc) return rc;
+    for (uint64_t f0 = 0; f0 < frames; f0 += chunk) {
+      const uint64_t nf = std::min(chunk, frames - f0);
+      awgn_hard_kernel<<<grid_for(ctx, nf * ((n + 3) / 4), kAwgnThreads), kAwgnThreads, 0, ctx->stream>>>(
+          d_words, static_cast<uint32_t>(n), sigma, seed, point, frame0 + f0, nf);
+      CU(cudaGetLastError());
+      rc = gf_rc(ctx, gf_launch(code->gf, d_words, nf, nullptr, nullptr, 0, d_out, d_ne, d_fail, ctx->sm_count, ctx->stream));
+      if (rc) return rc;
+      count_words_kernel<<<grid_for(ctx, nf, 8, 8), 256, 0, ctx->stream>>>(d_out, d_fail, static_cast<uint32_t>(n), nf,
+                                                                           counters);
+      CU(cudaGetLastError());
+      ctx->launches += 2;
+    }
+    return CCGPU_OK;
+  });
 }
 
 // ---- Chase-II (extension): K5 in chase.cu
 static int check_chase(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t p) {
-  if (code->ctx != ctx) return fail(ctx, CCGPU_ERR_INVALID, "code was not created on this context");
+  if (int rc = check_code(ctx, code)) return rc;
   if (p > kChaseMaxP) return fail(ctx, CCGPU_ERR_INVALID, "Chase-II takes 0 <= p <= 8 test positions");
   if (code->spec.family != 0) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "Chase-II decoding needs a binary BCH code");
   if (p > code->spec.n) return fail(ctx, CCGPU_ERR_INVALID, "p > n");
@@ -1564,33 +1551,14 @@ int ccgpu_decode_llr_chase(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t p, c
   CU(cudaSetDevice(ctx->device));
   const size_t n = code->spec.n;
   const bool dev = is_device_ptr(y);
-  if (is_device_ptr(bits) != dev || is_device_ptr(failed) != dev || (chosen && is_device_ptr(chosen) != dev))
+  if (!same_residency(dev, {bits, failed, chosen}))
     return fail(ctx, CCGPU_ERR_INVALID, "y and the outputs must all be device pointers or all host pointers");
   if (dev) return chase_rc(ctx, chase_launch(code->gf, p, y, frames, bits, failed, chosen, ctx->sm_count, ctx->stream));
-  // host buffers: chunks rotate over the staging slots so that copies and decoding overlap
-  const size_t per_frame = n * sizeof(float) + n + 2;
-  const uint64_t chunk = std::max<uint64_t>(1024, std::min<uint64_t>((frames + 15) / 16, (size_t(32) << 20) / per_frame));
-  rc = ensure_slots(ctx, chunk * per_frame + 256);
-  if (rc) return rc;
-  CU(cudaEventRecord(ctx->main_ready, ctx->stream));
-  for (int s = 0; s < kSlots; ++s) CU(cudaStreamWaitEvent(ctx->slot_stream[s], ctx->main_ready, 0));
-  int slot = 0;
-  for (uint64_t f0 = 0; f0 < frames; f0 += chunk, slot = (slot + 1) % kSlots) {
-    const uint64_t nf = std::min(chunk, frames - f0);
-    cudaStream_t st = ctx->slot_stream[slot];
-    float *d_y = static_cast<float *>(ctx->slot_buf[slot]);
-    uint8_t *d_bits = reinterpret_cast<uint8_t *>(d_y + chunk * n);
-    uint8_t *d_failed = d_bits + chunk * n;
-    uint8_t *d_chosen = d_failed + chunk;
-    CU(cudaMemcpyAsync(d_y, y + f0 * n, nf * n * sizeof(float), cudaMemcpyHostToDevice, st));
-    rc = chase_rc(ctx, chase_launch(code->gf, p, d_y, nf, d_bits, d_failed, chosen ? d_chosen : nullptr, ctx->sm_count, st));
-    if (rc) return rc;
-    CU(cudaMemcpyAsync(bits + f0 * n, d_bits, nf * n, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(failed + f0, d_failed, nf, cudaMemcpyDeviceToHost, st));
-    if (chosen) CU(cudaMemcpyAsync(chosen + f0, d_chosen, nf, cudaMemcpyDeviceToHost, st));
-  }
-  for (int s = 0; s < kSlots; ++s) CU(cudaStreamSynchronize(ctx->slot_stream[s]));
-  return CCGPU_OK;
+  const HostField fields[] = { { n * sizeof(float), y, false }, { n, bits, true }, { 1, failed, true }, { 1, chosen, true } };
+  return host_pipeline(ctx, frames, fields, [&](void *const *d, uint64_t nf, cudaStream_t st, int) {
+    return chase_rc(ctx, chase_launch(code->gf, p, static_cast<const float *>(d[0]), nf, static_cast<uint8_t *>(d[1]),
+                                      static_cast<uint8_t *>(d[2]), static_cast<uint8_t *>(d[3]), ctx->sm_count, st));
+  });
 }
 
 int ccgpu_awgn_point_chase(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t p, double ebno_db, uint64_t seed,
@@ -1600,18 +1568,10 @@ int ccgpu_awgn_point_chase(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t p, d
   if (rc) return rc;
   std::lock_guard<std::mutex> g(ctx->mu);
   CU(cudaSetDevice(ctx->device));
-  const bool dev = is_device_ptr(out);
-  unsigned long long *counters = dev ? reinterpret_cast<unsigned long long *>(out) : ctx->d_counters;
-  if (!dev) CU(cudaMemsetAsync(ctx->d_counters, 0, sizeof(ccgpu_counters), ctx->stream));
   const float sigma = static_cast<float>(ccgpu_sigma(code->spec.rate, ebno_db));
-  rc = chase_rc(ctx, chase_awgn_launch(code->gf, p, sigma, seed, point, frame0, frames, counters, ctx->sm_count, ctx->stream));
-  if (rc) return rc;
-  if (!dev) {
-    CU(cudaMemcpyAsync(ctx->h_counters, ctx->d_counters, sizeof(ccgpu_counters), cudaMemcpyDeviceToHost, ctx->stream));
-    CU(cudaStreamSynchronize(ctx->stream));
-    *out = *ctx->h_counters;
-  }
-  return CCGPU_OK;
+  return with_counters(ctx, out, [&](unsigned long long *counters) {
+    return chase_rc(ctx, chase_awgn_launch(code->gf, p, sigma, seed, point, frame0, frames, counters, ctx->sm_count, ctx->stream));
+  });
 }
 
 int ccgpu_code_set_recheck(ccgpu_code *code, int enable) {
