@@ -21,6 +21,7 @@
 #include "gf_decode.h"
 #include "ms_csr.h"
 #include "ms_params.h"
+#include "osd.h"
 
 using namespace ccgpu;
 
@@ -72,6 +73,7 @@ struct ccgpu_code {
   unsigned max_col_weight = 0;
   MsCsrDevice csr;     // general-H kernel tables (device)
   GfDevice gf;         // algebraic decoder tables (device)
+  OsdDevice osd;       // packed k-row H of the ordered-statistics decoder (device; binary BCH, n <= 127, k <= 64)
 };
 
 namespace {
@@ -580,6 +582,7 @@ int finish_code(ccgpu_ctx *ctx, ccgpu_code *c) {
   const int rc = refresh_H(c);
   if (rc || !ctx || c->spec.family == 2) return rc;
   if (gf_upload(c->spec, &c->gf) != 0) return fail(ctx, CCGPU_ERR_CUDA, "gf_upload failed");
+  if (osd_upload(c->spec, &c->osd) != 0) return fail(ctx, CCGPU_ERR_CUDA, "osd_upload failed");
   return CCGPU_OK;
 }
 
@@ -984,6 +987,7 @@ void ccgpu_code_destroy(ccgpu_code *code) {
   }
   ms_csr_free(&code->csr);
   gf_free(&code->gf);
+  osd_free(&code->osd);
   delete code;
 }
 
@@ -1571,6 +1575,54 @@ int ccgpu_awgn_point_chase(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t p, d
   const float sigma = static_cast<float>(ccgpu_sigma(code->spec.rate, ebno_db));
   return with_counters(ctx, out, [&](unsigned long long *counters) {
     return chase_rc(ctx, chase_awgn_launch(code->gf, p, sigma, seed, point, frame0, frames, counters, ctx->sm_count, ctx->stream));
+  });
+}
+
+// ---- ordered-statistics decoding (extension): K6 in osd.cu
+static int check_osd(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t order) {
+  if (int rc = check_code(ctx, code)) return rc;
+  if (order > kOsdMaxOrder) return fail(ctx, CCGPU_ERR_INVALID, "OSD takes 0 <= order <= 3");
+  if (code->spec.family != 0) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "OSD decoding needs a binary BCH code");
+  if (!code->osd.rows) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "code not supported by the OSD kernel (n <= 127, n - l <= 64)");
+  return CCGPU_OK;
+}
+static int osd_rc(ccgpu_ctx *ctx, int rc) {
+  if (rc == -3) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "code not supported by the OSD kernel (n <= 127, n - l <= 64)");
+  if (rc != 0) return cuda_fail(ctx, cudaGetLastError(), "osd_launch");
+  ctx->launches++;
+  return CCGPU_OK;
+}
+
+int ccgpu_decode_llr_osd(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t order, const float *y, uint64_t frames,
+                         uint8_t *bits, uint8_t *weight) {
+  if (!ctx || !code || !y || !bits) return fail(ctx, CCGPU_ERR_INVALID, "null argument");
+  int rc = check_osd(ctx, code, order);
+  if (rc) return rc;
+  std::lock_guard<std::mutex> g(ctx->mu);
+  if (frames == 0) return CCGPU_OK;
+  CU(cudaSetDevice(ctx->device));
+  const size_t n = code->spec.n;
+  const bool dev = is_device_ptr(y);
+  if (!same_residency(dev, {bits, weight}))
+    return fail(ctx, CCGPU_ERR_INVALID, "y and the outputs must all be device pointers or all host pointers");
+  if (dev) return osd_rc(ctx, osd_launch(code->osd, order, y, frames, bits, weight, ctx->sm_count, ctx->stream));
+  const HostField fields[] = { { n * sizeof(float), y, false }, { n, bits, true }, { 1, weight, true } };
+  return host_pipeline(ctx, frames, fields, [&](void *const *d, uint64_t nf, cudaStream_t st, int) {
+    return osd_rc(ctx, osd_launch(code->osd, order, static_cast<const float *>(d[0]), nf, static_cast<uint8_t *>(d[1]),
+                                  static_cast<uint8_t *>(d[2]), ctx->sm_count, st));
+  });
+}
+
+int ccgpu_awgn_point_osd(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t order, double ebno_db, uint64_t seed,
+                         uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out) {
+  if (!ctx || !code || !out) return fail(ctx, CCGPU_ERR_INVALID, "null argument");
+  int rc = check_osd(ctx, code, order);
+  if (rc) return rc;
+  std::lock_guard<std::mutex> g(ctx->mu);
+  CU(cudaSetDevice(ctx->device));
+  const float sigma = static_cast<float>(ccgpu_sigma(code->spec.rate, ebno_db));
+  return with_counters(ctx, out, [&](unsigned long long *counters) {
+    return osd_rc(ctx, osd_awgn_launch(code->osd, order, sigma, seed, point, frame0, frames, counters, ctx->sm_count, ctx->stream));
   });
 }
 

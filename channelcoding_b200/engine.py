@@ -365,6 +365,41 @@ class Code:
                                                           frames, C.addressof(c)))
         return c.as_dict()
 
+    def decode_osd(self, y, order, out=None):
+        """ordered-statistics decoding of order 0..3 (extension, ccgpu_decode_llr_osd; binary BCH codes with n <= 127,
+        n - l <= 64) -> bits (frames, n) uint8, weight (frames,) uint8 [number of information positions the returned
+        codeword flips]; numpy or torch CUDA tensors like decode()"""
+        if _is_torch(y):
+            import torch
+            y = y.contiguous().view(-1, self.n)
+            frames = y.shape[0]
+            if out is None:
+                out = (torch.empty((frames, self.n), dtype=torch.uint8, device=y.device),
+                       torch.empty(frames, dtype=torch.uint8, device=y.device))
+        else:
+            y = np.ascontiguousarray(y, np.float32).reshape(-1, self.n)
+            frames = y.shape[0]
+            if out is None:
+                out = (np.empty((frames, self.n), np.uint8), np.empty(frames, np.uint8))
+        bits, weight = out
+        self.ctx._follow_torch(y, bits)
+        self.ctx._check(_lib.lib().ccgpu_decode_llr_osd(self.ctx._h, self._h, int(order), _ptr(y), frames, _ptr(bits),
+                                                        _ptr(weight)))
+        return bits, weight
+
+    def awgn_point_osd(self, ebno_db, frames, order, seed=0, point=0, frame0=0, out=None):
+        """one Eb/N0 point decoded with OSD of the given order on the GPU (ccgpu_awgn_point_osd) -> counters.
+        out: optional torch uint64/int64 CUDA tensor of 8 slots that is accumulated into (no sync)."""
+        if out is not None:
+            self.ctx._follow_torch(out)
+            self.ctx._check(_lib.lib().ccgpu_awgn_point_osd(self.ctx._h, self._h, int(order), float(ebno_db), seed, point,
+                                                            frame0, frames, _ptr(out)))
+            return out
+        c = Counters()
+        self.ctx._check(_lib.lib().ccgpu_awgn_point_osd(self.ctx._h, self._h, int(order), float(ebno_db), seed, point, frame0,
+                                                        frames, C.addressof(c)))
+        return c.as_dict()
+
     def bitflip_point(self, weight, variant="MS", alpha=1.0, beta=0.0, max_iter=50,
                       stop_rule=STOP_REF_ZERO_OVERLAP, first=0, count=0, quant=None):
         """one error weight of bitflip_simulation (simulation.c++:156-213) -> counters"""
@@ -503,6 +538,12 @@ class GroupCode:
         c = Counters()
         self.group._check(_lib.lib().ccgpu_group_awgn_point_chase(self.group._h, self._arr, int(p), float(ebno_db), seed, point,
                                                                   frame0, frames, C.addressof(c)))
+        return c.as_dict()
+
+    def awgn_point_osd(self, ebno_db, frames, order, seed=0, point=0, frame0=0):
+        c = Counters()
+        self.group._check(_lib.lib().ccgpu_group_awgn_point_osd(self.group._h, self._arr, int(order), float(ebno_db), seed,
+                                                                point, frame0, frames, C.addressof(c)))
         return c.as_dict()
 
     def awgn_point_mbbp(self, ebno_db, frames, shifts, variant="MS", alpha=1.0, beta=0.0, max_iter=50,

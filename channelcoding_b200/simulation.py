@@ -101,3 +101,16 @@ def chase_point_fn(code, p, seed=0):
             code.ctx.sync()
         return out
     return fn
+
+
+def osd_point_fn(code, order, seed=0):
+    """point_fn for awgn_sweep backed by ccgpu_awgn_point_osd (OSD of the given order) on the code's device"""
+    import torch
+
+    def fn(ebno, point, frame0, frames):
+        out = torch.zeros(8, dtype=torch.int64, device="cuda:%d" % code.ctx.device)
+        if frames > 0:
+            code.awgn_point_osd(ebno, frames, order, seed=seed, point=point, frame0=frame0, out=out)
+            code.ctx.sync()
+        return out
+    return fn

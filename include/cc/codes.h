@@ -10,6 +10,7 @@
 //   cyclic::primitive_bch<q, Capability, Tag>          cc::primitive_bch<q, Capability, Tag>   codes/bch.h:16-161
 //   cyclic::rs<q, Capability, Tag>                     cc::rs<q, Capability, Tag>              codes/rs.h:6-94
 //   (extension) Chase-II                               cc::primitive_bch<q, Capability, chase_tag<P> >
+//   (extension) ordered-statistics decoding            cc::primitive_bch<q, Capability, osd_tag<Order> >
 //     .correct<R>(vector<float|uint>)  .to_string()  .rate  ::n  ::t  .H<T>()           codes/cyclic.h:282-359
 //
 // Differences a user sees: every object holds a ccgpu context/code handle (one GPU, or every GPU of the current
@@ -153,6 +154,17 @@ template <unsigned P> struct chase_tag : algorithm_tag {
 };
 template <typename Tag> struct is_chase_tag : std::false_type {};
 template <unsigned P> struct is_chase_tag<chase_tag<P> > : std::true_type {};
+
+// ---- extension: ordered-statistics decoding OSD-i (ccgpu_decode_llr_osd).  Re-encodes the most reliable basis of the
+// channel values with up to Order of its positions flipped; the candidate closest to the channel values wins.  Like
+// Chase-II it takes channel values and is neither a soft-decision (min-sum) nor a hard-decision tag.
+template <unsigned Order> struct osd_tag : algorithm_tag {
+  static_assert(Order <= 3, "OSD takes order 0 .. 3");
+  static constexpr unsigned order = Order;
+  static std::string to_string() { return "OSD" + std::to_string(Order); }
+};
+template <typename Tag> struct is_osd_tag : std::false_type {};
+template <unsigned Order> struct is_osd_tag<osd_tag<Order> > : std::true_type {};
 
 // ---- one GPU context shared by every code object of the process (per device) ------------------------
 class gpu_error : public std::runtime_error {
@@ -322,6 +334,7 @@ public:
   const double rate;  // public data member like cyclic.h:111
   static constexpr bool soft_tag = std::is_base_of<soft_decision_tag, Algorithm>::value;
   static constexpr bool chase = is_chase_tag<Algorithm>::value;
+  static constexpr bool osd = is_osd_tag<Algorithm>::value;
 
   std::string to_string() const {  // cyclic.h:282-287
     char buf[96];
@@ -541,6 +554,46 @@ public:
                                                         frame0, frames, &c));
     else
       this->h_->ctx->check(ccgpu_awgn_point_chase(this->h_->ctx->get(), this->h_->code, P, ebno_db, seed, point, frame0, frames, &c));
+    return c;
+  }
+};
+
+// extension: the same code decoded with ordered-statistics decoding of order Order (ccgpu_decode_llr_osd; n <= 127,
+// n - l <= 64)
+template <unsigned q, typename Capability, unsigned Order>
+class primitive_bch<q, Capability, osd_tag<Order> > : public cyclic_base<osd_tag<Order> > {
+  using base = cyclic_base<osd_tag<Order> >;
+
+public:
+  static constexpr unsigned n = (1u << q) - 1;
+  static constexpr unsigned t = correction_capability<Capability>::value;
+  explicit primitive_bch(int device = -1) : base(detail::make_bch<q, Capability>(device)) {}
+
+  // frames x n channel values -> frames x n bits, always a codeword; weight[f] (optional) is the number of information
+  // positions the returned codeword flips
+  void correct_batch(const float *y, uint64_t frames, uint8_t *bits, uint8_t *weight = nullptr) const {
+    this->h_->ctx->check(ccgpu_decode_llr_osd(this->h_->ctx->get(), this->h_->code, Order, y, frames, bits, weight));
+  }
+  // one frame of channel values; OSD never fails
+  template <typename Return_type = uint8_t, typename InputSequence>
+  std::vector<Return_type> correct(const InputSequence &b) const {
+    if (b.size() != n)
+      throw std::runtime_error("Channel code word has the wrong size (" + std::to_string(b.size()) + "). Expected " +
+                               std::to_string(n));
+    const std::vector<float> y(b.begin(), b.end());
+    std::vector<uint8_t> out(n);
+    correct_batch(y.data(), 1, out.data());
+    return std::vector<Return_type>(out.begin(), out.end());
+  }
+  // one Eb/N0 point (simulation.c++:112-149) decoded with OSD on the device, sharded over the code's group if any
+  ccgpu_counters awgn_point(double ebno_db, uint64_t frames, uint64_t seed = 0, uint32_t point = 0, uint64_t frame0 = 0) const {
+    ccgpu_counters c{};
+    if (this->h_->grp)
+      this->h_->grp->check(ccgpu_group_awgn_point_osd(this->h_->grp->get(), this->h_->codes.data(), Order, ebno_db, seed,
+                                                      point, frame0, frames, &c));
+    else
+      this->h_->ctx->check(ccgpu_awgn_point_osd(this->h_->ctx->get(), this->h_->code, Order, ebno_db, seed, point, frame0,
+                                                frames, &c));
     return c;
   }
 };

@@ -111,12 +111,14 @@ class decoder {
     unsigned n() const override { return T::n; }
     bool soft() const override { return T::soft_tag; }
     ccgpu_counters awgn_point(double e, uint64_t f, uint64_t s, uint32_t p, uint64_t f0) const override {
-      // soft tags and Chase-II take the channel values: their own fused point
-      return point_impl(e, f, s, p, f0, std::integral_constant<bool, T::soft_tag || T::chase>());
+      // soft tags, Chase-II and OSD take the channel values: their own fused point
+      return point_impl(e, f, s, p, f0, std::integral_constant<bool, T::soft_tag || T::chase || T::osd>());
     }
     ccgpu_counters bitflip_point(unsigned weight) const override {
       if constexpr (T::chase)
         throw std::runtime_error(implementation.to_string() + ": bit-flip simulation has no channel reliabilities for Chase-II");
+      else if constexpr (T::osd)
+        throw std::runtime_error(implementation.to_string() + ": bit-flip simulation has no channel reliabilities for OSD");
       else
         return flips_impl(weight, std::integral_constant<bool, T::soft_tag>());
     }

@@ -286,6 +286,35 @@ int ccgpu_decode_llr_chase(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t p, c
 int ccgpu_awgn_point_chase(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t p, double ebno_db, uint64_t seed,
                            uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
 
+/* EXTENSION (no reference implementation): ordered-statistics decoding (Fossorier-Lin OSD-i) of binary primitive BCH
+ * codes, a near-maximum-likelihood decoder for short codes.  l information bits, k = n - l rows of the k-row H of
+ * ccgpu_code_H at creation (codes/cyclic.h:346-359).  Per frame:
+ *   1. h_c = (y_c < 0) as codes/codes.h:43-52 (0 for -0.0 and NaN);
+ *   2. the columns are visited in ascending (bits of fabsf(y_c) as uint32, c): ties go to the lower column, NaN sorts
+ *      above +inf (the order of ccgpu_decode_llr_chase);
+ *   3. P = the columns picked greedily in that order, a column being picked when its H-column is not in the GF(2)
+ *      span of the H-columns picked before it (|P| = rank H = k); I = the other l columns.  P depends on the code
+ *      only, not on which rows H has, so ccgpu_code_set_rows does not change it; I is the "most reliable basis", the
+ *      l columns picked greedily from a generator matrix in the reverse order;
+ *   4. with i_0 < .. < i_{l-1} the columns of I, candidate e is the codeword x_e with x_e[I] = h[I] ^ 1_{E_e}; E_0 is
+ *      empty, then come the sets {i_a} (a ascending), {i_a, i_b} (a < b, lexicographic) and {i_a, i_b, i_c}
+ *      (lexicographic), none heavier than min(order, l): sum over w <= min(order, l) of C(l, w) candidates
+ *      (1 / 37 / 667 / 7807 for BCH(63,36));
+ *   5. D_e = sum of fabsf(y_c) over the columns where x_e != h, float32, c ascending, starting from +0.0; the winner
+ *      is the smallest (K(D_e), e), K = the bits of D_e as uint32 with every NaN counted as 0x7fc00000;
+ *   6. bits = x_winner, weight = |E_winner| <= order.  There is no failure: the result is always a codeword.
+ * If h is a codeword it is returned with weight 0 (candidate 0 is h with D = +0.0).
+ * Binary BCH codes with n <= 127 and k <= 64; 0 <= order <= 3 (order > 3: CCGPU_ERR_INVALID; RS, dense-H codes,
+ * n = 255 or k > 64: CCGPU_ERR_UNSUPPORTED).  bits frames x n, weight frames (nullable).  Host or device pointers like
+ * ccgpu_decode_llr, all of one kind. */
+int ccgpu_decode_llr_osd(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t order, const float *y, uint64_t frames,
+                         uint8_t *bits, uint8_t *weight);
+/* one Eb/N0 point, frames [frame0, frame0 + frames) of the ccgpu_awgn_point noise stream, decoded with OSD on chip;
+ * only counters leave: iterations = failures = 0, undetected = frame_errors.  `out` host or device pointer as in
+ * ccgpu_awgn_point. */
+int ccgpu_awgn_point_osd(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t order, double ebno_db, uint64_t seed,
+                         uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
+
 /* one weight class of bitflip_simulation::operator() (simulation.c++:156-213): all C(n, weight)
  * inputs x = -2*bit + 1, decoded and counted; patterns [first, first + count) in the
  * lexicographic order of std::next_permutation (count 0 = all). */
@@ -345,7 +374,7 @@ int ccgpu_group_size(const ccgpu_group *group);
 ccgpu_ctx *ccgpu_group_ctx(const ccgpu_group *group, int member);
 const char *ccgpu_group_last_error(const ccgpu_group *group);
 int ccgpu_group_set_min_frames(ccgpu_group *group, uint64_t frames_per_member);
-/* the Monte-Carlo points of ccgpu_awgn_point / _hard / _chase / _mbbp / _uncoded / ccgpu_bitflip_point, sharded; `out` is a
+/* the Monte-Carlo points of ccgpu_awgn_point / _hard / _chase / _osd / _mbbp / _uncoded / ccgpu_bitflip_point, sharded; `out` is a
  * host pointer and holds the merged counters on return */
 int ccgpu_group_awgn_point(ccgpu_group *group, ccgpu_code *const *codes, const ccgpu_ms_params *params, double ebno_db,
                            uint64_t seed, uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
@@ -353,6 +382,8 @@ int ccgpu_group_awgn_point_hard(ccgpu_group *group, ccgpu_code *const *codes, do
                                 uint64_t frame0, uint64_t frames, ccgpu_counters *out);
 int ccgpu_group_awgn_point_chase(ccgpu_group *group, ccgpu_code *const *codes, uint32_t p, double ebno_db,
                                  uint64_t seed, uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
+int ccgpu_group_awgn_point_osd(ccgpu_group *group, ccgpu_code *const *codes, uint32_t order, double ebno_db,
+                               uint64_t seed, uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
 int ccgpu_group_awgn_point_mbbp(ccgpu_group *group, ccgpu_code *const *codes, const ccgpu_ms_params *params,
                                 const uint32_t *shifts, uint32_t n_bases, double ebno_db, uint64_t seed, uint32_t point,
                                 uint64_t frame0, uint64_t frames, ccgpu_counters *out);

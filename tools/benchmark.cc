@@ -11,7 +11,8 @@
 // weight, bitflips.c++ uses 6), --out DIR, --device D (first CUDA device), --gpus N (shard every point over N devices
 // D .. D+N-1 through a ccgpu_group; the counters, hence the logs, are identical to the one-GPU run),
 // --algorithm chase1 .. chase8 (Chase-II over 1 .. 8 test positions, "(n, l, dmin)-CHASE<P>.log"; built only when
-// named, never part of "all" or of the default selection).
+// named, never part of "all" or of the default selection), --algorithm osd0 .. osd3 (ordered-statistics decoding of
+// order 0 .. 3, "(n, l, dmin)-OSD<i>.log"; likewise only when named).
 #include <getopt.h>
 
 #include <cmath>
@@ -48,6 +49,18 @@ template <unsigned P> static void add_chase(std::vector<decoder> &v) {
   add_chase_power<6, P>(v);
   add_chase_power<7, P>(v);
 }
+// OSD decoders (extension): only built when --algorithm osd<i> asks for them, never part of "all"
+template <unsigned Q, unsigned O> static void add_osd_power(std::vector<decoder> &v) {
+  v.emplace_back(primitive_bch<Q, dmin<3>, osd_tag<O> >());
+  v.emplace_back(primitive_bch<Q, dmin<5>, osd_tag<O> >());
+  v.emplace_back(primitive_bch<Q, dmin<7>, osd_tag<O> >());
+  v.emplace_back(primitive_bch<Q, dmin<9>, osd_tag<O> >());
+}
+template <unsigned O> static void add_osd(std::vector<decoder> &v) {
+  add_osd_power<5, O>(v);
+  add_osd_power<6, O>(v);
+  add_osd_power<7, O>(v);
+}
 template <unsigned Q> static void add_power(std::vector<decoder> &v) {
   add_code<Q, dmin<3> >(v);
   add_code<Q, dmin<5> >(v);
@@ -57,8 +70,8 @@ template <unsigned Q> static void add_power(std::vector<decoder> &v) {
 
 [[noreturn]] static void usage() {
   std::cout << "--simulation [awgn|bitflip]  choose the simulation (default awgn)\n"
-               "--algorithm <ms|nms|oms|scms1|scms2|2dnms|bm|pgz|euklid|all|chase1..chase8>   (repeatable;\n"
-               "             Chase-II only when named, awgn only)\n"
+               "--algorithm <ms|nms|oms|scms1|scms2|2dnms|bm|pgz|euklid|all|chase1..chase8|osd0..osd3>\n"
+               "             (repeatable; Chase-II and OSD only when named, awgn only)\n"
                "--k <5|6|7|all>   code length n = 2^k - 1   (repeatable)\n"
                "--dmin <3|5|7|9|all>                          (repeatable)\n"
                "--seed <num>  --seed-time  --threads <num>\n"
@@ -127,6 +140,9 @@ int main(int argc, char *const argv[]) {
                                                            add_chase<5>, add_chase<6>, add_chase<7>, add_chase<8> };
   for (unsigned p = 1; p <= 8; ++p)
     if (algorithms.count("chase" + std::to_string(p))) chase[p - 1](decoders);
+  static void (*const osd[])(std::vector<decoder> &) = { add_osd<0>, add_osd<1>, add_osd<2>, add_osd<3> };
+  for (unsigned o = 0; o <= 3; ++o)
+    if (algorithms.count("osd" + std::to_string(o))) osd[o](decoders);
 
   // selection by parsing to_string(), exactly like benchmark.c++:214-240
   std::vector<const decoder *> chosen;

@@ -3,6 +3,7 @@
 
     python tools/sweep.py --q 8 --t 18 --variant NMS --alpha 0.8 --ebno-from 0 --ebno-to 8 --ebno-step 0.5
     python tools/sweep.py --q 6 --t 5 --chase 4 ...      # Chase-II over the 4 least reliable positions
+    python tools/sweep.py --q 6 --t 5 --osd 2 ...        # ordered-statistics decoding of order 2
     torchrun --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 tools/sweep.py ...
 
 Every Eb/N0 point is simulated in rounds of --batch frames (split evenly over the ranks by global frame
@@ -35,8 +36,11 @@ def main():
     ap.add_argument("--min-errors", type=int, default=100)
     ap.add_argument("--max-frames", type=float, default=1e9)
     ap.add_argument("--seed", type=int, default=0)
-    ap.add_argument("--chase", type=int, default=None, metavar="P",
-                    help="decode with Chase-II over the P least reliable positions (0..8) instead of the min-sum variant")
+    algo = ap.add_mutually_exclusive_group()
+    algo.add_argument("--chase", type=int, default=None, metavar="P",
+                      help="decode with Chase-II over the P least reliable positions (0..8) instead of the min-sum variant")
+    algo.add_argument("--osd", type=int, default=None, metavar="ORDER",
+                      help="decode with ordered-statistics decoding of order 0..3 instead of the min-sum variant")
     a = ap.parse_args()
 
     import torch
@@ -56,6 +60,7 @@ def main():
     ctx.use_torch_stream()
     code = ctx.bch(a.q, errors=a.t)
     dev = torch.device("cuda", local)
+    tag = "CHASE%d" % a.chase if a.chase is not None else "OSD%d" % a.osd if a.osd is not None else a.variant
     point, eb = 0, a.ebno_from
     while eb < a.ebno_to + a.ebno_step / 2:
         total = torch.zeros(8, dtype=torch.int64, device=dev)
@@ -64,11 +69,13 @@ def main():
         while True:
             first, count = shard_range(a.batch, world, rank)
             part = torch.zeros(8, dtype=torch.int64, device=dev)
-            if a.chase is None:
+            if a.chase is not None:
+                code.awgn_point_chase(eb, count, a.chase, seed=a.seed, point=point, frame0=done + first, out=part)
+            elif a.osd is not None:
+                code.awgn_point_osd(eb, count, a.osd, seed=a.seed, point=point, frame0=done + first, out=part)
+            else:
                 code.awgn_point(eb, count, a.variant, a.alpha, a.beta, a.max_iter, a.stop_rule, seed=a.seed, point=point,
                                 frame0=done + first, out=part)
-            else:
-                code.awgn_point_chase(eb, count, a.chase, seed=a.seed, point=point, frame0=done + first, out=part)
             if world > 1:
                 dist.all_reduce(part, op=dist.ReduceOp.SUM)  # the one collective of the path
             total += part
@@ -78,7 +85,7 @@ def main():
                 break
         el = time.perf_counter() - t0
         if rank == 0:
-            print(json.dumps({"code": code.to_string(a.variant if a.chase is None else "CHASE%d" % a.chase), "ebno_db": eb, "frames": c[0], "frame_errors": c[1],
+            print(json.dumps({"code": code.to_string(tag), "ebno_db": eb, "frames": c[0], "frame_errors": c[1],
                               "bit_errors": c[2], "wer": c[1] / c[0], "ber": c[2] / c[0] / code.n,
                               "avg_iterations": c[3] / c[0], "failures": c[4], "undetected": c[5], "n_gpus": world,
                               "seconds": el, "frames_per_s": c[0] / el}), flush=True)
