@@ -19,6 +19,7 @@
 #include "chase.h"
 #include "codes.hpp"
 #include "gf_decode.h"
+#include "gmd.h"
 #include "ms_csr.h"
 #include "ms_params.h"
 #include "osd.h"
@@ -1623,6 +1624,58 @@ int ccgpu_awgn_point_osd(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t order,
   const float sigma = static_cast<float>(ccgpu_sigma(code->spec.rate, ebno_db));
   return with_counters(ctx, out, [&](unsigned long long *counters) {
     return osd_rc(ctx, osd_awgn_launch(code->osd, order, sigma, seed, point, frame0, frames, counters, ctx->sm_count, ctx->stream));
+  });
+}
+
+// ---- GMD decoding of Reed-Solomon codes (extension): K7 in gmd.cu
+static int check_gmd(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t max_erasures) {
+  if (int rc = check_code(ctx, code)) return rc;
+  if (code->spec.family != 1)
+    return fail(ctx, CCGPU_ERR_UNSUPPORTED, "GMD decoding needs a Reed-Solomon code (binary BCH codes have Chase-II)");
+  if (code->spec.roots.size() > kGmdMaxRoots || code->spec.step != 1)
+    return fail(ctx, CCGPU_ERR_UNSUPPORTED, "code not supported by the GMD kernel (2t <= 32, step = 1)");
+  if ((max_erasures & 1u) || max_erasures > 2 * code->spec.t)
+    return fail(ctx, CCGPU_ERR_INVALID, "GMD takes an even max_erasures <= 2t");
+  return CCGPU_OK;
+}
+static int gmd_rc(ccgpu_ctx *ctx, int rc) {
+  if (rc == -3) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "code not supported by the GMD kernel (2t <= 32, step = 1)");
+  if (rc != 0) return cuda_fail(ctx, cudaGetLastError(), "gmd_launch");
+  ctx->launches++;
+  return CCGPU_OK;
+}
+
+int ccgpu_decode_llr_gmd(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t max_erasures, const float *y, uint64_t frames,
+                         uint8_t *words, uint8_t *failed, uint8_t *chosen) {
+  if (!ctx || !code || !y || !words || !failed) return fail(ctx, CCGPU_ERR_INVALID, "null argument");
+  int rc = check_gmd(ctx, code, max_erasures);
+  if (rc) return rc;
+  std::lock_guard<std::mutex> g(ctx->mu);
+  if (frames == 0) return CCGPU_OK;
+  CU(cudaSetDevice(ctx->device));
+  const size_t n = code->spec.n, nq = n * code->spec.q;
+  const bool dev = is_device_ptr(y);
+  if (!same_residency(dev, {words, failed, chosen}))
+    return fail(ctx, CCGPU_ERR_INVALID, "y and the outputs must all be device pointers or all host pointers");
+  if (dev) return gmd_rc(ctx, gmd_launch(code->gf, max_erasures, y, frames, words, failed, chosen, ctx->sm_count, ctx->stream));
+  const HostField fields[] = { { nq * sizeof(float), y, false }, { n, words, true }, { 1, failed, true }, { 1, chosen, true } };
+  return host_pipeline(ctx, frames, fields, [&](void *const *d, uint64_t nf, cudaStream_t st, int) {
+    return gmd_rc(ctx, gmd_launch(code->gf, max_erasures, static_cast<const float *>(d[0]), nf, static_cast<uint8_t *>(d[1]),
+                                  static_cast<uint8_t *>(d[2]), static_cast<uint8_t *>(d[3]), ctx->sm_count, st));
+  });
+}
+
+int ccgpu_awgn_point_gmd(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t max_erasures, double ebno_db, uint64_t seed,
+                         uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out) {
+  if (!ctx || !code || !out) return fail(ctx, CCGPU_ERR_INVALID, "null argument");
+  int rc = check_gmd(ctx, code, max_erasures);
+  if (rc) return rc;
+  std::lock_guard<std::mutex> g(ctx->mu);
+  CU(cudaSetDevice(ctx->device));
+  const float sigma = static_cast<float>(ccgpu_sigma(code->spec.rate, ebno_db));
+  return with_counters(ctx, out, [&](unsigned long long *counters) {
+    return gmd_rc(ctx, gmd_awgn_launch(code->gf, max_erasures, sigma, seed, point, frame0, frames, counters, ctx->sm_count,
+                                       ctx->stream));
   });
 }
 

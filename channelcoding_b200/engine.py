@@ -400,6 +400,45 @@ class Code:
                                                         frames, C.addressof(c)))
         return c.as_dict()
 
+    def decode_gmd(self, y, max_erasures, out=None):
+        """GMD decoding of a Reed-Solomon code from the channel values of its binary image (extension,
+        ccgpu_decode_llr_gmd; 2t <= 32): y (frames, n*q), bit j of symbol c at position c*q + j; trials erase the 0, 2,
+        .., max_erasures least reliable symbols -> words (frames, n) uint8, failed (frames,) uint8, chosen (frames,)
+        uint8 [index i of the winning trial]; numpy or torch CUDA tensors like decode()"""
+        nq = self.n * self.q
+        if _is_torch(y):
+            import torch
+            y = y.contiguous().view(-1, nq)
+            frames = y.shape[0]
+            if out is None:
+                out = (torch.empty((frames, self.n), dtype=torch.uint8, device=y.device),
+                       torch.empty(frames, dtype=torch.uint8, device=y.device),
+                       torch.empty(frames, dtype=torch.uint8, device=y.device))
+        else:
+            y = np.ascontiguousarray(y, np.float32).reshape(-1, nq)
+            frames = y.shape[0]
+            if out is None:
+                out = (np.empty((frames, self.n), np.uint8), np.empty(frames, np.uint8), np.empty(frames, np.uint8))
+        words, failed, chosen = out
+        self.ctx._follow_torch(y, words)
+        self.ctx._check(_lib.lib().ccgpu_decode_llr_gmd(self.ctx._h, self._h, int(max_erasures), _ptr(y), frames,
+                                                        _ptr(words), _ptr(failed), _ptr(chosen)))
+        return words, failed, chosen
+
+    def awgn_point_gmd(self, ebno_db, frames, max_erasures, seed=0, point=0, frame0=0, out=None):
+        """one Eb/N0 point of a Reed-Solomon code decoded with GMD on the GPU (ccgpu_awgn_point_gmd; max_erasures = 0:
+        hard-decision decoding) -> counters.  out: optional torch uint64/int64 CUDA tensor of 8 slots that is
+        accumulated into (no sync)."""
+        if out is not None:
+            self.ctx._follow_torch(out)
+            self.ctx._check(_lib.lib().ccgpu_awgn_point_gmd(self.ctx._h, self._h, int(max_erasures), float(ebno_db), seed,
+                                                            point, frame0, frames, _ptr(out)))
+            return out
+        c = Counters()
+        self.ctx._check(_lib.lib().ccgpu_awgn_point_gmd(self.ctx._h, self._h, int(max_erasures), float(ebno_db), seed, point,
+                                                        frame0, frames, C.addressof(c)))
+        return c.as_dict()
+
     def bitflip_point(self, weight, variant="MS", alpha=1.0, beta=0.0, max_iter=50,
                       stop_rule=STOP_REF_ZERO_OVERLAP, first=0, count=0, quant=None):
         """one error weight of bitflip_simulation (simulation.c++:156-213) -> counters"""
@@ -544,6 +583,12 @@ class GroupCode:
         c = Counters()
         self.group._check(_lib.lib().ccgpu_group_awgn_point_osd(self.group._h, self._arr, int(order), float(ebno_db), seed,
                                                                 point, frame0, frames, C.addressof(c)))
+        return c.as_dict()
+
+    def awgn_point_gmd(self, ebno_db, frames, max_erasures, seed=0, point=0, frame0=0):
+        c = Counters()
+        self.group._check(_lib.lib().ccgpu_group_awgn_point_gmd(self.group._h, self._arr, int(max_erasures), float(ebno_db),
+                                                                seed, point, frame0, frames, C.addressof(c)))
         return c.as_dict()
 
     def awgn_point_mbbp(self, ebno_db, frames, shifts, variant="MS", alpha=1.0, beta=0.0, max_iter=50,

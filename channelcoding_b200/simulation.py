@@ -114,3 +114,17 @@ def osd_point_fn(code, order, seed=0):
             code.ctx.sync()
         return out
     return fn
+
+
+def gmd_point_fn(code, max_erasures, seed=0):
+    """point_fn for awgn_sweep backed by ccgpu_awgn_point_gmd (GMD of a Reed-Solomon code with up to max_erasures
+    erasures; 0 = hard decision) on the code's device"""
+    import torch
+
+    def fn(ebno, point, frame0, frames):
+        out = torch.zeros(8, dtype=torch.int64, device="cuda:%d" % code.ctx.device)
+        if frames > 0:
+            code.awgn_point_gmd(ebno, frames, max_erasures, seed=seed, point=point, frame0=frame0, out=out)
+            code.ctx.sync()
+        return out
+    return fn

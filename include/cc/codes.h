@@ -11,6 +11,7 @@
 //   cyclic::rs<q, Capability, Tag>                     cc::rs<q, Capability, Tag>              codes/rs.h:6-94
 //   (extension) Chase-II                               cc::primitive_bch<q, Capability, chase_tag<P> >
 //   (extension) ordered-statistics decoding            cc::primitive_bch<q, Capability, osd_tag<Order> >
+//   (extension) GMD decoding of RS codes               cc::rs<q, Capability, gmd_tag<F> >
 //     .correct<R>(vector<float|uint>)  .to_string()  .rate  ::n  ::t  .H<T>()           codes/cyclic.h:282-359
 //
 // Differences a user sees: every object holds a ccgpu context/code handle (one GPU, or every GPU of the current
@@ -165,6 +166,18 @@ template <unsigned Order> struct osd_tag : algorithm_tag {
 };
 template <typename Tag> struct is_osd_tag : std::false_type {};
 template <unsigned Order> struct is_osd_tag<osd_tag<Order> > : std::true_type {};
+
+// ---- extension: generalized minimum distance decoding of Reed-Solomon codes (ccgpu_decode_llr_gmd).  Takes the
+// channel values of the binary image (n q per word), erases the 0, 2, .., F least reliable symbols in turn, decodes each
+// trial with errors and erasures, and returns the candidate closest to the channel values.  F = 0 is hard-decision
+// decoding.  Like Chase-II it is neither a soft-decision (min-sum) nor a hard-decision tag.
+template <unsigned F> struct gmd_tag : algorithm_tag {
+  static_assert(F % 2 == 0, "GMD erases symbols in pairs: F must be even");
+  static constexpr unsigned max_erasures = F;
+  static std::string to_string() { return "GMD" + std::to_string(F); }
+};
+template <typename Tag> struct is_gmd_tag : std::false_type {};
+template <unsigned F> struct is_gmd_tag<gmd_tag<F> > : std::true_type {};
 
 // ---- one GPU context shared by every code object of the process (per device) ------------------------
 class gpu_error : public std::runtime_error {
@@ -335,6 +348,7 @@ public:
   static constexpr bool soft_tag = std::is_base_of<soft_decision_tag, Algorithm>::value;
   static constexpr bool chase = is_chase_tag<Algorithm>::value;
   static constexpr bool osd = is_osd_tag<Algorithm>::value;
+  static constexpr bool gmd = is_gmd_tag<Algorithm>::value;
 
   std::string to_string() const {  // cyclic.h:282-287
     char buf[96];
@@ -613,6 +627,55 @@ public:
   static constexpr unsigned n = (1u << q) - 1;
   static constexpr unsigned t = correction_capability<Capability>::value;
   explicit rs(int device = -1) : cyclic_base<Sigma>(make(device)) {}
+};
+
+// extension: the same RS code decoded with GMD over up to F erased symbols from the channel values of its binary image
+// (ccgpu_decode_llr_gmd; 2t <= 32).  A frame is n q channel values, bit j of symbol c at position c q + j.
+template <unsigned q, typename Capability, unsigned F, unsigned mu, unsigned step>
+class rs<q, Capability, gmd_tag<F>, mu, step> : public cyclic_base<gmd_tag<F> > {
+  using base = cyclic_base<gmd_tag<F> >;
+  static std::shared_ptr<detail::code_handle> make(int device) {
+    return detail::code_handle::make(device, [](ccgpu_ctx *ctx, ccgpu_code **out) {
+      return ccgpu_rs_create(ctx, q, correction_capability<Capability>::value, mu, step, out);
+    });
+  }
+
+public:
+  static constexpr unsigned n = (1u << q) - 1;
+  static constexpr unsigned t = correction_capability<Capability>::value;
+  static constexpr unsigned channel_length = n * q;  // channel values per word
+  static_assert(F <= 2 * t, "GMD erases at most 2t symbols");
+  explicit rs(int device = -1) : base(make(device)) {}
+
+  // frames x (n q) channel values -> frames x n symbols; failed[f] = 1: no trial decoded, words = the hard decision;
+  // chosen[f] (optional) = the winning trial i (2i symbols erased)
+  void correct_batch(const float *y, uint64_t frames, uint8_t *words, uint8_t *failed, uint8_t *chosen = nullptr) const {
+    this->h_->ctx->check(ccgpu_decode_llr_gmd(this->h_->ctx->get(), this->h_->code, F, y, frames, words, failed, chosen));
+  }
+  // one frame of n q channel values -> n symbols; throws decoding_failure when no trial decodes
+  template <typename Return_type = uint8_t, typename InputSequence>
+  std::vector<Return_type> correct(const InputSequence &b) const {
+    if (b.size() != channel_length)
+      throw std::runtime_error("Channel word has the wrong size (" + std::to_string(b.size()) + "). Expected " +
+                               std::to_string(channel_length));
+    const std::vector<float> y(b.begin(), b.end());
+    std::vector<uint8_t> out(n);
+    uint8_t failed = 0;
+    correct_batch(y.data(), 1, out.data(), &failed);
+    if (failed) throw decoding_failure("Decoding failure");
+    return std::vector<Return_type>(out.begin(), out.end());
+  }
+  // one Eb/N0 point (simulation.c++:112-149) decoded with GMD on the device, sharded over the code's group if any
+  ccgpu_counters awgn_point(double ebno_db, uint64_t frames, uint64_t seed = 0, uint32_t point = 0, uint64_t frame0 = 0) const {
+    ccgpu_counters c{};
+    if (this->h_->grp)
+      this->h_->grp->check(ccgpu_group_awgn_point_gmd(this->h_->grp->get(), this->h_->codes.data(), F, ebno_db, seed, point,
+                                                      frame0, frames, &c));
+    else
+      this->h_->ctx->check(ccgpu_awgn_point_gmd(this->h_->ctx->get(), this->h_->code, F, ebno_db, seed, point, frame0,
+                                                frames, &c));
+    return c;
+  }
 };
 
 // codes/uncoded.h:10-47 -- the pseudo-decoder of simulation/uncoded.c++: n symbols, hard decision, nominal rate 0.5.

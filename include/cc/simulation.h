@@ -108,17 +108,24 @@ class decoder {
     std::vector<uint8_t> correct(const std::vector<float> &b) const override { return implementation.template correct<uint8_t>(b); }
     std::string to_string() const override { return implementation.to_string(); }
     double rate() const override { return implementation.rate; }
-    unsigned n() const override { return T::n; }
+    unsigned n() const override {  // channel values per frame: n q for GMD, which takes the binary image of RS words
+      if constexpr (T::gmd)
+        return T::channel_length;
+      else
+        return T::n;
+    }
     bool soft() const override { return T::soft_tag; }
     ccgpu_counters awgn_point(double e, uint64_t f, uint64_t s, uint32_t p, uint64_t f0) const override {
-      // soft tags, Chase-II and OSD take the channel values: their own fused point
-      return point_impl(e, f, s, p, f0, std::integral_constant<bool, T::soft_tag || T::chase || T::osd>());
+      // soft tags, Chase-II, OSD and GMD take the channel values: their own fused point
+      return point_impl(e, f, s, p, f0, std::integral_constant<bool, T::soft_tag || T::chase || T::osd || T::gmd>());
     }
     ccgpu_counters bitflip_point(unsigned weight) const override {
       if constexpr (T::chase)
         throw std::runtime_error(implementation.to_string() + ": bit-flip simulation has no channel reliabilities for Chase-II");
       else if constexpr (T::osd)
         throw std::runtime_error(implementation.to_string() + ": bit-flip simulation has no channel reliabilities for OSD");
+      else if constexpr (T::gmd)
+        throw std::runtime_error(implementation.to_string() + ": bit-flip simulation has no channel reliabilities for GMD");
       else
         return flips_impl(weight, std::integral_constant<bool, T::soft_tag>());
     }

@@ -315,6 +315,36 @@ int ccgpu_decode_llr_osd(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t order,
 int ccgpu_awgn_point_osd(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t order, double ebno_db, uint64_t seed,
                          uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
 
+/* EXTENSION (no reference implementation): generalized minimum distance (GMD, Forney) soft-decision decoding of
+ * Reed-Solomon codes over the AWGN channel, from the channel values of their binary image.  Symbol c (0 <= c < n) is
+ * q bits; bit j of it is image position b = c q + j and equals (s_c >> j) & 1, with the symbol values of ccgpu_encode
+ * and ccgpu_gf_decode.  A frame is n q channel values in the raw-y convention of ccgpu_decode_llr.  Per frame:
+ *   1. h_b = (y_b < 0) as codes/codes.h:43-52 (0 for -0.0 and NaN); r_c = sum_j h_{cq+j} << j;
+ *   2. kappa_c = min_j K(fabsf(y_{cq+j})), K = the bits as uint32 with every NaN counted as 0x7fc00000; the symbols
+ *      are ranked in ascending (kappa_c, c);
+ *   3. trial i = 0 .. F/2 (F = max_erasures) erases E_i, the first 2i symbols of that ranking, and decodes r with
+ *      erasures E_i exactly as ccgpu_gf_decode_erasures would (bounded distance, 2e + 2i <= 2t, same failure rules;
+ *      for even erasure counts this is the reference's Euklid decoder, DESIGN.md section 7); a success x_i is a
+ *      candidate.  The 30-erasure limit of ccgpu_gf_decode_erasures does not apply: F = 2t = 32 is a pure erasure
+ *      decode with 32 erasures;
+ *   4. D_i = sum of fabsf(y_b) over the image positions b where the bit of x_i differs from h_b, float32, b ascending,
+ *      starting from +0.0;
+ *   5. the winner is the smallest (K(D_i), i).  If r is a codeword, trial 0 returns it with D = +0.0 and it wins;
+ *   6. words = x_winner; without a candidate failed = 1 and words = r; chosen (nullable) = the winner's i, 0 when the
+ *      frame failed.  F = 0 is ccgpu_gf_decode of r.
+ * RS codes with 2t <= 32 and step 1 (binary BCH, dense-H codes, 2t > 32: CCGPU_ERR_UNSUPPORTED; F odd or F > 2t:
+ * CCGPU_ERR_INVALID).  y frames x (n q), words frames x n, failed and chosen frames.  Host or device pointers like
+ * ccgpu_decode_llr, all of one kind. */
+int ccgpu_decode_llr_gmd(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t max_erasures, const float *y, uint64_t frames,
+                         uint8_t *words, uint8_t *failed, uint8_t *chosen);
+/* one Eb/N0 point, decoded with GMD on chip: frame f is what ccgpu_awgn_llr(n q, ccgpu_sigma(l / n, ebno_db), seed,
+ * point, frame0, frames) writes for it (the all-zero word sent).  Only counters leave: frame_errors = failed or any
+ * decided symbol non-zero, bit_errors = set bits of the decided binary image (r for a failed frame), failures = frames
+ * without a candidate, undetected = decoded to a non-zero word, iterations = 0.  `out` host or device pointer as in
+ * ccgpu_awgn_point.  With max_erasures = 0 this is the hard-decision RS curve. */
+int ccgpu_awgn_point_gmd(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t max_erasures, double ebno_db, uint64_t seed,
+                         uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
+
 /* one weight class of bitflip_simulation::operator() (simulation.c++:156-213): all C(n, weight)
  * inputs x = -2*bit + 1, decoded and counted; patterns [first, first + count) in the
  * lexicographic order of std::next_permutation (count 0 = all). */
@@ -374,7 +404,7 @@ int ccgpu_group_size(const ccgpu_group *group);
 ccgpu_ctx *ccgpu_group_ctx(const ccgpu_group *group, int member);
 const char *ccgpu_group_last_error(const ccgpu_group *group);
 int ccgpu_group_set_min_frames(ccgpu_group *group, uint64_t frames_per_member);
-/* the Monte-Carlo points of ccgpu_awgn_point / _hard / _chase / _osd / _mbbp / _uncoded / ccgpu_bitflip_point, sharded; `out` is a
+/* the Monte-Carlo points of ccgpu_awgn_point / _hard / _chase / _osd / _gmd / _mbbp / _uncoded / ccgpu_bitflip_point, sharded; `out` is a
  * host pointer and holds the merged counters on return */
 int ccgpu_group_awgn_point(ccgpu_group *group, ccgpu_code *const *codes, const ccgpu_ms_params *params, double ebno_db,
                            uint64_t seed, uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
@@ -383,6 +413,8 @@ int ccgpu_group_awgn_point_hard(ccgpu_group *group, ccgpu_code *const *codes, do
 int ccgpu_group_awgn_point_chase(ccgpu_group *group, ccgpu_code *const *codes, uint32_t p, double ebno_db,
                                  uint64_t seed, uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
 int ccgpu_group_awgn_point_osd(ccgpu_group *group, ccgpu_code *const *codes, uint32_t order, double ebno_db,
+                               uint64_t seed, uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
+int ccgpu_group_awgn_point_gmd(ccgpu_group *group, ccgpu_code *const *codes, uint32_t max_erasures, double ebno_db,
                                uint64_t seed, uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
 int ccgpu_group_awgn_point_mbbp(ccgpu_group *group, ccgpu_code *const *codes, const ccgpu_ms_params *params,
                                 const uint32_t *shifts, uint32_t n_bases, double ebno_db, uint64_t seed, uint32_t point,

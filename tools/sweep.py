@@ -4,6 +4,7 @@
     python tools/sweep.py --q 8 --t 18 --variant NMS --alpha 0.8 --ebno-from 0 --ebno-to 8 --ebno-step 0.5
     python tools/sweep.py --q 6 --t 5 --chase 4 ...      # Chase-II over the 4 least reliable positions
     python tools/sweep.py --q 6 --t 5 --osd 2 ...        # ordered-statistics decoding of order 2
+    python tools/sweep.py --q 8 --t 16 --gmd 32 ...      # RS(255,223), GMD with up to 32 erasures (--gmd 0: hard)
     torchrun --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 tools/sweep.py ...
 
 Every Eb/N0 point is simulated in rounds of --batch frames (split evenly over the ranks by global frame
@@ -41,6 +42,9 @@ def main():
                       help="decode with Chase-II over the P least reliable positions (0..8) instead of the min-sum variant")
     algo.add_argument("--osd", type=int, default=None, metavar="ORDER",
                       help="decode with ordered-statistics decoding of order 0..3 instead of the min-sum variant")
+    algo.add_argument("--gmd", type=int, default=None, metavar="F",
+                      help="simulate the Reed-Solomon code RS(2^q - 1, 2^q - 1 - 2t) decoded with GMD over up to F "
+                           "(even, <= 2t) erased symbols; 0 is hard-decision decoding")
     a = ap.parse_args()
 
     import torch
@@ -58,9 +62,11 @@ def main():
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     ctx = cc.Context(local)
     ctx.use_torch_stream()
-    code = ctx.bch(a.q, errors=a.t)
+    code = ctx.rs(a.q, a.t) if a.gmd is not None else ctx.bch(a.q, errors=a.t)
+    bits_per_frame = code.n * a.q if a.gmd is not None else code.n  # GMD counts the bits of the binary image
     dev = torch.device("cuda", local)
-    tag = "CHASE%d" % a.chase if a.chase is not None else "OSD%d" % a.osd if a.osd is not None else a.variant
+    tag = ("CHASE%d" % a.chase if a.chase is not None else "OSD%d" % a.osd if a.osd is not None else
+           "GMD%d" % a.gmd if a.gmd is not None else a.variant)
     point, eb = 0, a.ebno_from
     while eb < a.ebno_to + a.ebno_step / 2:
         total = torch.zeros(8, dtype=torch.int64, device=dev)
@@ -73,6 +79,8 @@ def main():
                 code.awgn_point_chase(eb, count, a.chase, seed=a.seed, point=point, frame0=done + first, out=part)
             elif a.osd is not None:
                 code.awgn_point_osd(eb, count, a.osd, seed=a.seed, point=point, frame0=done + first, out=part)
+            elif a.gmd is not None:
+                code.awgn_point_gmd(eb, count, a.gmd, seed=a.seed, point=point, frame0=done + first, out=part)
             else:
                 code.awgn_point(eb, count, a.variant, a.alpha, a.beta, a.max_iter, a.stop_rule, seed=a.seed, point=point,
                                 frame0=done + first, out=part)
@@ -86,7 +94,7 @@ def main():
         el = time.perf_counter() - t0
         if rank == 0:
             print(json.dumps({"code": code.to_string(tag), "ebno_db": eb, "frames": c[0], "frame_errors": c[1],
-                              "bit_errors": c[2], "wer": c[1] / c[0], "ber": c[2] / c[0] / code.n,
+                              "bit_errors": c[2], "wer": c[1] / c[0], "ber": c[2] / c[0] / bits_per_frame,
                               "avg_iterations": c[3] / c[0], "failures": c[4], "undetected": c[5], "n_gpus": world,
                               "seconds": el, "frames_per_s": c[0] / el}), flush=True)
         point += 1
