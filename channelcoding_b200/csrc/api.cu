@@ -19,6 +19,7 @@
 #include "chase.h"
 #include "codes.hpp"
 #include "gf_decode.h"
+#include "abp.h"
 #include "gmd.h"
 #include "ms_csr.h"
 #include "ms_params.h"
@@ -1676,6 +1677,59 @@ int ccgpu_awgn_point_gmd(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t max_er
   return with_counters(ctx, out, [&](unsigned long long *counters) {
     return gmd_rc(ctx, gmd_awgn_launch(code->gf, max_erasures, sigma, seed, point, frame0, frames, counters, ctx->sm_count,
                                        ctx->stream));
+  });
+}
+
+// ---- adaptive belief propagation (extension): K8 in abp.cu, on the OSD kernel's packed k-row H
+static int check_abp(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t max_iter, double gamma) {
+  if (int rc = check_code(ctx, code)) return rc;
+  if (max_iter > kAbpMaxIter) return fail(ctx, CCGPU_ERR_INVALID, "ABP takes 0 <= max_iter <= 255");
+  if (!(gamma > 0.0 && gamma <= 1.0)) return fail(ctx, CCGPU_ERR_INVALID, "ABP takes a finite gamma with 0 < gamma <= 1");
+  if (code->spec.family != 0) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "ABP decoding needs a binary BCH code");
+  if (!code->osd.rows) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "code not supported by the ABP kernel (n <= 127, n - l <= 64)");
+  return CCGPU_OK;
+}
+static int abp_rc(ccgpu_ctx *ctx, int rc) {
+  if (rc == -3) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "code not supported by the ABP kernel (n <= 127, n - l <= 64)");
+  if (rc != 0) return cuda_fail(ctx, cudaGetLastError(), "abp_launch");
+  ctx->launches++;
+  return CCGPU_OK;
+}
+
+int ccgpu_decode_llr_abp(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t max_iter, double gamma, const float *y,
+                         uint64_t frames, uint8_t *bits, float *L, uint8_t *iter, uint8_t *failed) {
+  if (!ctx || !code || !y || !bits || !iter || !failed) return fail(ctx, CCGPU_ERR_INVALID, "null argument");
+  int rc = check_abp(ctx, code, max_iter, gamma);
+  if (rc) return rc;
+  std::lock_guard<std::mutex> g(ctx->mu);
+  if (frames == 0) return CCGPU_OK;
+  CU(cudaSetDevice(ctx->device));
+  const size_t n = code->spec.n;
+  const float gf = static_cast<float>(gamma);
+  const bool dev = is_device_ptr(y);
+  if (!same_residency(dev, {bits, L, iter, failed}))
+    return fail(ctx, CCGPU_ERR_INVALID, "y and the outputs must all be device pointers or all host pointers");
+  if (dev) return abp_rc(ctx, abp_launch(code->osd, max_iter, gf, y, frames, bits, L, iter, failed, ctx->sm_count, ctx->stream));
+  const HostField fields[] = { { n * sizeof(float), y, false }, { n, bits, true }, { n * sizeof(float), L, true },
+                               { 1, iter, true }, { 1, failed, true } };
+  return host_pipeline(ctx, frames, fields, [&](void *const *d, uint64_t nf, cudaStream_t st, int) {
+    return abp_rc(ctx, abp_launch(code->osd, max_iter, gf, static_cast<const float *>(d[0]), nf, static_cast<uint8_t *>(d[1]),
+                                  static_cast<float *>(d[2]), static_cast<uint8_t *>(d[3]), static_cast<uint8_t *>(d[4]),
+                                  ctx->sm_count, st));
+  });
+}
+
+int ccgpu_awgn_point_abp(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t max_iter, double gamma, double ebno_db,
+                         uint64_t seed, uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out) {
+  if (!ctx || !code || !out) return fail(ctx, CCGPU_ERR_INVALID, "null argument");
+  int rc = check_abp(ctx, code, max_iter, gamma);
+  if (rc) return rc;
+  std::lock_guard<std::mutex> g(ctx->mu);
+  CU(cudaSetDevice(ctx->device));
+  const float sigma = static_cast<float>(ccgpu_sigma(code->spec.rate, ebno_db));
+  return with_counters(ctx, out, [&](unsigned long long *counters) {
+    return abp_rc(ctx, abp_awgn_launch(code->osd, max_iter, static_cast<float>(gamma), sigma, seed, point, frame0, frames,
+                                       counters, ctx->sm_count, ctx->stream));
   });
 }
 

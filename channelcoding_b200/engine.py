@@ -439,6 +439,44 @@ class Code:
                                                         frame0, frames, C.addressof(c)))
         return c.as_dict()
 
+    def decode_abp(self, y, max_iter=50, gamma=0.15, out=None):
+        """adaptive belief propagation with the min-sum check pass (extension, ccgpu_decode_llr_abp; binary BCH codes
+        with n <= 127, n - l <= 64; 0 <= max_iter <= 255, 0 < gamma <= 1) -> bits, L, iter, failed like decode();
+        out = (bits, L or None, iter, failed); numpy or torch CUDA tensors like decode()"""
+        if _is_torch(y):
+            import torch
+            y = y.contiguous().view(-1, self.n)
+            frames = y.shape[0]
+            if out is None:
+                out = (torch.empty((frames, self.n), dtype=torch.uint8, device=y.device),
+                       torch.empty((frames, self.n), dtype=torch.float32, device=y.device),
+                       torch.empty(frames, dtype=torch.uint8, device=y.device),
+                       torch.empty(frames, dtype=torch.uint8, device=y.device))
+        else:
+            y = np.ascontiguousarray(y, np.float32).reshape(-1, self.n)
+            frames = y.shape[0]
+            if out is None:
+                out = (np.empty((frames, self.n), np.uint8), np.empty((frames, self.n), np.float32),
+                       np.empty(frames, np.uint8), np.empty(frames, np.uint8))
+        bits, L, it, failed = out
+        self.ctx._follow_torch(y, bits)
+        self.ctx._check(_lib.lib().ccgpu_decode_llr_abp(self.ctx._h, self._h, int(max_iter), float(gamma), _ptr(y), frames,
+                                                        _ptr(bits), _ptr(L), _ptr(it), _ptr(failed)))
+        return bits, L, it, failed
+
+    def awgn_point_abp(self, ebno_db, frames, max_iter=50, gamma=0.15, seed=0, point=0, frame0=0, out=None):
+        """one Eb/N0 point decoded with ABP on the GPU (ccgpu_awgn_point_abp) -> counters.
+        out: optional torch uint64/int64 CUDA tensor of 8 slots that is accumulated into (no sync)."""
+        if out is not None:
+            self.ctx._follow_torch(out)
+            self.ctx._check(_lib.lib().ccgpu_awgn_point_abp(self.ctx._h, self._h, int(max_iter), float(gamma), float(ebno_db),
+                                                            seed, point, frame0, frames, _ptr(out)))
+            return out
+        c = Counters()
+        self.ctx._check(_lib.lib().ccgpu_awgn_point_abp(self.ctx._h, self._h, int(max_iter), float(gamma), float(ebno_db), seed,
+                                                        point, frame0, frames, C.addressof(c)))
+        return c.as_dict()
+
     def bitflip_point(self, weight, variant="MS", alpha=1.0, beta=0.0, max_iter=50,
                       stop_rule=STOP_REF_ZERO_OVERLAP, first=0, count=0, quant=None):
         """one error weight of bitflip_simulation (simulation.c++:156-213) -> counters"""
@@ -589,6 +627,12 @@ class GroupCode:
         c = Counters()
         self.group._check(_lib.lib().ccgpu_group_awgn_point_gmd(self.group._h, self._arr, int(max_erasures), float(ebno_db),
                                                                 seed, point, frame0, frames, C.addressof(c)))
+        return c.as_dict()
+
+    def awgn_point_abp(self, ebno_db, frames, max_iter=50, gamma=0.15, seed=0, point=0, frame0=0):
+        c = Counters()
+        self.group._check(_lib.lib().ccgpu_group_awgn_point_abp(self.group._h, self._arr, int(max_iter), float(gamma),
+                                                                float(ebno_db), seed, point, frame0, frames, C.addressof(c)))
         return c.as_dict()
 
     def awgn_point_mbbp(self, ebno_db, frames, shifts, variant="MS", alpha=1.0, beta=0.0, max_iter=50,

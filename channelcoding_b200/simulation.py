@@ -128,3 +128,16 @@ def gmd_point_fn(code, max_erasures, seed=0):
             code.ctx.sync()
         return out
     return fn
+
+
+def abp_point_fn(code, max_iter=50, gamma=0.15, seed=0):
+    """point_fn for awgn_sweep backed by ccgpu_awgn_point_abp (adaptive belief propagation) on the code's device"""
+    import torch
+
+    def fn(ebno, point, frame0, frames):
+        out = torch.zeros(8, dtype=torch.int64, device="cuda:%d" % code.ctx.device)
+        if frames > 0:
+            code.awgn_point_abp(ebno, frames, max_iter, gamma, seed=seed, point=point, frame0=frame0, out=out)
+            code.ctx.sync()
+        return out
+    return fn

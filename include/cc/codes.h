@@ -12,6 +12,7 @@
 //   (extension) Chase-II                               cc::primitive_bch<q, Capability, chase_tag<P> >
 //   (extension) ordered-statistics decoding            cc::primitive_bch<q, Capability, osd_tag<Order> >
 //   (extension) GMD decoding of RS codes               cc::rs<q, Capability, gmd_tag<F> >
+//   (extension) adaptive belief propagation            cc::primitive_bch<q, Capability, abp_tag<Iterations, Gamma> >
 //     .correct<R>(vector<float|uint>)  .to_string()  .rate  ::n  ::t  .H<T>()           codes/cyclic.h:282-359
 //
 // Differences a user sees: every object holds a ccgpu context/code handle (one GPU, or every GPU of the current
@@ -178,6 +179,20 @@ template <unsigned F> struct gmd_tag : algorithm_tag {
 };
 template <typename Tag> struct is_gmd_tag : std::false_type {};
 template <unsigned F> struct is_gmd_tag<gmd_tag<F> > : std::true_type {};
+
+// ---- extension: adaptive belief propagation (ccgpu_decode_llr_abp).  Before each of at most Iterations min-sum check
+// passes, H is reduced so that its least reliable independent columns have weight one; the soft values are updated
+// with the damping factor Gamma (a std::ratio, 0 < Gamma <= 1).  It takes channel values but is not one of the min-sum
+// variants of soft_decision_tag: it has its own entry points.
+template <unsigned Iterations, typename Gamma = std::ratio<15, 100> > struct abp_tag : algorithm_tag {
+  static_assert(Iterations <= 255, "ABP takes at most 255 iterations");
+  static_assert(Gamma::num > 0 && Gamma::num <= Gamma::den, "ABP takes a damping factor 0 < Gamma <= 1");
+  static constexpr unsigned iterations = Iterations;
+  static constexpr double gamma = static_cast<double>(Gamma::num) / Gamma::den;
+  static std::string to_string() { return "ABP" + std::to_string(Iterations); }
+};
+template <typename Tag> struct is_abp_tag : std::false_type {};
+template <unsigned I, typename G> struct is_abp_tag<abp_tag<I, G> > : std::true_type {};
 
 // ---- one GPU context shared by every code object of the process (per device) ------------------------
 class gpu_error : public std::runtime_error {
@@ -349,6 +364,7 @@ public:
   static constexpr bool chase = is_chase_tag<Algorithm>::value;
   static constexpr bool osd = is_osd_tag<Algorithm>::value;
   static constexpr bool gmd = is_gmd_tag<Algorithm>::value;
+  static constexpr bool abp = is_abp_tag<Algorithm>::value;
 
   std::string to_string() const {  // cyclic.h:282-287
     char buf[96];
@@ -568,6 +584,49 @@ public:
                                                         frame0, frames, &c));
     else
       this->h_->ctx->check(ccgpu_awgn_point_chase(this->h_->ctx->get(), this->h_->code, P, ebno_db, seed, point, frame0, frames, &c));
+    return c;
+  }
+};
+
+// extension: the same code decoded with adaptive belief propagation (ccgpu_decode_llr_abp; n <= 127, n - l <= 64)
+template <unsigned q, typename Capability, unsigned Iterations, typename Gamma>
+class primitive_bch<q, Capability, abp_tag<Iterations, Gamma> > : public cyclic_base<abp_tag<Iterations, Gamma> > {
+  using base = cyclic_base<abp_tag<Iterations, Gamma> >;
+  using tag = abp_tag<Iterations, Gamma>;
+
+public:
+  static constexpr unsigned n = (1u << q) - 1;
+  static constexpr unsigned t = correction_capability<Capability>::value;
+  explicit primitive_bch(int device = -1) : base(detail::make_bch<q, Capability>(device)) {}
+
+  // frames x n channel values -> frames x n bits, iter and failed per frame; L (optional) the final soft values
+  void correct_batch(const float *y, uint64_t frames, uint8_t *bits, uint8_t *iter, uint8_t *failed,
+                     float *L = nullptr) const {
+    this->h_->ctx->check(ccgpu_decode_llr_abp(this->h_->ctx->get(), this->h_->code, Iterations, tag::gamma, y, frames,
+                                              bits, L, iter, failed));
+  }
+  // one frame of channel values; throws decoding_failure when the stop test never passed
+  template <typename Return_type = uint8_t, typename InputSequence>
+  std::vector<Return_type> correct(const InputSequence &b) const {
+    if (b.size() != n)
+      throw std::runtime_error("Channel code word has the wrong size (" + std::to_string(b.size()) + "). Expected " +
+                               std::to_string(n));
+    const std::vector<float> y(b.begin(), b.end());
+    std::vector<uint8_t> out(n);
+    uint8_t iter = 0, failed = 0;
+    correct_batch(y.data(), 1, out.data(), &iter, &failed);
+    if (failed) throw decoding_failure("Decoding failure");
+    return std::vector<Return_type>(out.begin(), out.end());
+  }
+  // one Eb/N0 point (simulation.c++:112-149) decoded with ABP on the device, sharded over the code's group if any
+  ccgpu_counters awgn_point(double ebno_db, uint64_t frames, uint64_t seed = 0, uint32_t point = 0, uint64_t frame0 = 0) const {
+    ccgpu_counters c{};
+    if (this->h_->grp)
+      this->h_->grp->check(ccgpu_group_awgn_point_abp(this->h_->grp->get(), this->h_->codes.data(), Iterations, tag::gamma,
+                                                      ebno_db, seed, point, frame0, frames, &c));
+    else
+      this->h_->ctx->check(ccgpu_awgn_point_abp(this->h_->ctx->get(), this->h_->code, Iterations, tag::gamma, ebno_db, seed,
+                                                point, frame0, frames, &c));
     return c;
   }
 };

@@ -345,6 +345,35 @@ int ccgpu_decode_llr_gmd(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t max_er
 int ccgpu_awgn_point_gmd(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t max_erasures, double ebno_db, uint64_t seed,
                          uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
 
+/* EXTENSION (no reference implementation): adaptive belief propagation (ABP, Jiang-Narayanan) of binary primitive BCH
+ * codes with the min-sum check pass.  Before every check pass H is reduced so that the k least reliable independent
+ * columns have weight one, which keeps errors on unreliable bits out of the short cycles of the dense H.  The k-row H of
+ * ccgpu_code_H at creation is always used, whatever ccgpu_code_set_rows selected: the adapted matrix depends only on
+ * the row space of H.  Per frame, with B = 2^20 and gamma_f = (float)gamma:
+ *   1. L_c = y_c clamped to [-B, B]: NaN becomes +0.0, +-inf becomes +-B (every value is finite from here on);
+ *   2. for j = 0, 1, ..: x_c = (L_c < 0); if H x = 0 over GF(2): bits = x, iter = j, failed = 0, stop.  If j = max_iter:
+ *      bits = x, iter = max_iter, failed = 1, stop.  Otherwise apply 3-6 once;
+ *   3. the columns are visited in ascending (bits of fabsf(L_c) as uint32, c) (the order of ccgpu_decode_llr_osd); P =
+ *      p_0, .., p_{k-1} are the first k columns in that order whose H-columns are independent (OSD's step 3);
+ *   4. A is the unique k x n matrix with the row space of H and A[:, P] = identity, row i the row with its one among
+ *      the P columns at p_i;
+ *   5. for each row i and each column c of row i: mu_{i,c} = min over the other columns c' of row i of fabsf(L_c')
+ *      (+0.0 for a row of weight 1), s_{i,c} = parity of #{c' != c in row i : L_c' < 0}, m_{i,c} = s ? -mu : mu;
+ *      S_c = +0.0 + m_{0,c} + m_{1,c} + .. over the rows holding c in ascending i, float32, no FMA;
+ *   6. L_c <- fminf(fmaxf(L_c + gamma_f * S_c, -B), B), the product and the sum each rounded to nearest even.
+ * Binary BCH codes with n <= 127 and k <= 64; 0 <= max_iter <= 255 (0: the syndrome check of the hard decision) and a
+ * finite 0 < gamma <= 1, else CCGPU_ERR_INVALID; RS, dense-H codes, n = 255 or k > 64: CCGPU_ERR_UNSUPPORTED.  bits
+ * frames x n, L (nullable) frames x n final soft values (they can be fed to ccgpu_decode_llr_osd), iter and failed
+ * frames.  Host or device pointers like ccgpu_decode_llr, all of one kind. */
+int ccgpu_decode_llr_abp(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t max_iter, double gamma, const float *y,
+                         uint64_t frames, uint8_t *bits, float *L, uint8_t *iter, uint8_t *failed);
+/* one Eb/N0 point, frames [frame0, frame0 + frames) of the ccgpu_awgn_point noise stream (raw y, no LLR scaling),
+ * decoded with ABP on chip.  Only counters leave: iterations = sum of the updates applied (iter), failures = frames with
+ * failed = 1, frame_errors = failed or any decided bit set, bit_errors = decided bits set, undetected = frames that
+ * passed the stop test on a non-zero word.  `out` host or device pointer as in ccgpu_awgn_point. */
+int ccgpu_awgn_point_abp(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t max_iter, double gamma, double ebno_db,
+                         uint64_t seed, uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
+
 /* one weight class of bitflip_simulation::operator() (simulation.c++:156-213): all C(n, weight)
  * inputs x = -2*bit + 1, decoded and counted; patterns [first, first + count) in the
  * lexicographic order of std::next_permutation (count 0 = all). */
@@ -404,7 +433,7 @@ int ccgpu_group_size(const ccgpu_group *group);
 ccgpu_ctx *ccgpu_group_ctx(const ccgpu_group *group, int member);
 const char *ccgpu_group_last_error(const ccgpu_group *group);
 int ccgpu_group_set_min_frames(ccgpu_group *group, uint64_t frames_per_member);
-/* the Monte-Carlo points of ccgpu_awgn_point / _hard / _chase / _osd / _gmd / _mbbp / _uncoded / ccgpu_bitflip_point, sharded; `out` is a
+/* the Monte-Carlo points of ccgpu_awgn_point / _hard / _chase / _osd / _gmd / _abp / _mbbp / _uncoded / ccgpu_bitflip_point, sharded; `out` is a
  * host pointer and holds the merged counters on return */
 int ccgpu_group_awgn_point(ccgpu_group *group, ccgpu_code *const *codes, const ccgpu_ms_params *params, double ebno_db,
                            uint64_t seed, uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
@@ -416,6 +445,9 @@ int ccgpu_group_awgn_point_osd(ccgpu_group *group, ccgpu_code *const *codes, uin
                                uint64_t seed, uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
 int ccgpu_group_awgn_point_gmd(ccgpu_group *group, ccgpu_code *const *codes, uint32_t max_erasures, double ebno_db,
                                uint64_t seed, uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
+int ccgpu_group_awgn_point_abp(ccgpu_group *group, ccgpu_code *const *codes, uint32_t max_iter, double gamma,
+                               double ebno_db, uint64_t seed, uint32_t point, uint64_t frame0, uint64_t frames,
+                               ccgpu_counters *out);
 int ccgpu_group_awgn_point_mbbp(ccgpu_group *group, ccgpu_code *const *codes, const ccgpu_ms_params *params,
                                 const uint32_t *shifts, uint32_t n_bases, double ebno_db, uint64_t seed, uint32_t point,
                                 uint64_t frame0, uint64_t frames, ccgpu_counters *out);

@@ -12,7 +12,8 @@
 // D .. D+N-1 through a ccgpu_group; the counters, hence the logs, are identical to the one-GPU run),
 // --algorithm chase1 .. chase8 (Chase-II over 1 .. 8 test positions, "(n, l, dmin)-CHASE<P>.log"; built only when
 // named, never part of "all" or of the default selection), --algorithm osd0 .. osd3 (ordered-statistics decoding of
-// order 0 .. 3, "(n, l, dmin)-OSD<i>.log"; likewise only when named).
+// order 0 .. 3, "(n, l, dmin)-OSD<i>.log"; likewise only when named), --algorithm abp (adaptive belief propagation,
+// 50 iterations, damping 0.15, "(n, l, dmin)-ABP50.log"; likewise only when named).
 #include <getopt.h>
 
 #include <cmath>
@@ -61,6 +62,14 @@ template <unsigned O> static void add_osd(std::vector<decoder> &v) {
   add_osd_power<6, O>(v);
   add_osd_power<7, O>(v);
 }
+// ABP decoders (extension): only built when --algorithm abp asks for them, never part of "all"
+using abp_default = abp_tag<50>;
+template <unsigned Q> static void add_abp_power(std::vector<decoder> &v) {
+  v.emplace_back(primitive_bch<Q, dmin<3>, abp_default>());
+  v.emplace_back(primitive_bch<Q, dmin<5>, abp_default>());
+  v.emplace_back(primitive_bch<Q, dmin<7>, abp_default>());
+  v.emplace_back(primitive_bch<Q, dmin<9>, abp_default>());
+}
 template <unsigned Q> static void add_power(std::vector<decoder> &v) {
   add_code<Q, dmin<3> >(v);
   add_code<Q, dmin<5> >(v);
@@ -70,8 +79,8 @@ template <unsigned Q> static void add_power(std::vector<decoder> &v) {
 
 [[noreturn]] static void usage() {
   std::cout << "--simulation [awgn|bitflip]  choose the simulation (default awgn)\n"
-               "--algorithm <ms|nms|oms|scms1|scms2|2dnms|bm|pgz|euklid|all|chase1..chase8|osd0..osd3>\n"
-               "             (repeatable; Chase-II and OSD only when named, awgn only)\n"
+               "--algorithm <ms|nms|oms|scms1|scms2|2dnms|bm|pgz|euklid|all|chase1..chase8|osd0..osd3|abp>\n"
+               "             (repeatable; Chase-II, OSD and ABP only when named, awgn only)\n"
                "--k <5|6|7|all>   code length n = 2^k - 1   (repeatable)\n"
                "--dmin <3|5|7|9|all>                          (repeatable)\n"
                "--seed <num>  --seed-time  --threads <num>\n"
@@ -143,6 +152,12 @@ int main(int argc, char *const argv[]) {
   static void (*const osd[])(std::vector<decoder> &) = { add_osd<0>, add_osd<1>, add_osd<2>, add_osd<3> };
   for (unsigned o = 0; o <= 3; ++o)
     if (algorithms.count("osd" + std::to_string(o))) osd[o](decoders);
+  if (algorithms.count("abp")) {  // selected below by the name in the log: ABP50
+    add_abp_power<5>(decoders);
+    add_abp_power<6>(decoders);
+    add_abp_power<7>(decoders);
+    algorithms.insert(lower(abp_default::to_string()));
+  }
 
   // selection by parsing to_string(), exactly like benchmark.c++:214-240
   std::vector<const decoder *> chosen;

@@ -5,6 +5,7 @@
     python tools/sweep.py --q 6 --t 5 --chase 4 ...      # Chase-II over the 4 least reliable positions
     python tools/sweep.py --q 6 --t 5 --osd 2 ...        # ordered-statistics decoding of order 2
     python tools/sweep.py --q 8 --t 16 --gmd 32 ...      # RS(255,223), GMD with up to 32 erasures (--gmd 0: hard)
+    python tools/sweep.py --q 6 --t 5 --abp 50 --gamma 0.15 ...  # adaptive belief propagation, 50 updates at most
     torchrun --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 tools/sweep.py ...
 
 Every Eb/N0 point is simulated in rounds of --batch frames (split evenly over the ranks by global frame
@@ -45,6 +46,10 @@ def main():
     algo.add_argument("--gmd", type=int, default=None, metavar="F",
                       help="simulate the Reed-Solomon code RS(2^q - 1, 2^q - 1 - 2t) decoded with GMD over up to F "
                            "(even, <= 2t) erased symbols; 0 is hard-decision decoding")
+    algo.add_argument("--abp", type=int, default=None, metavar="ITERS",
+                      help="decode with adaptive belief propagation, at most ITERS (0..255) updates, instead of the "
+                           "min-sum variant")
+    ap.add_argument("--gamma", type=float, default=0.15, help="damping factor of --abp (0 < gamma <= 1)")
     a = ap.parse_args()
 
     import torch
@@ -66,7 +71,7 @@ def main():
     bits_per_frame = code.n * a.q if a.gmd is not None else code.n  # GMD counts the bits of the binary image
     dev = torch.device("cuda", local)
     tag = ("CHASE%d" % a.chase if a.chase is not None else "OSD%d" % a.osd if a.osd is not None else
-           "GMD%d" % a.gmd if a.gmd is not None else a.variant)
+           "GMD%d" % a.gmd if a.gmd is not None else "ABP%d" % a.abp if a.abp is not None else a.variant)
     point, eb = 0, a.ebno_from
     while eb < a.ebno_to + a.ebno_step / 2:
         total = torch.zeros(8, dtype=torch.int64, device=dev)
@@ -81,6 +86,8 @@ def main():
                 code.awgn_point_osd(eb, count, a.osd, seed=a.seed, point=point, frame0=done + first, out=part)
             elif a.gmd is not None:
                 code.awgn_point_gmd(eb, count, a.gmd, seed=a.seed, point=point, frame0=done + first, out=part)
+            elif a.abp is not None:
+                code.awgn_point_abp(eb, count, a.abp, a.gamma, seed=a.seed, point=point, frame0=done + first, out=part)
             else:
                 code.awgn_point(eb, count, a.variant, a.alpha, a.beta, a.max_iter, a.stop_rule, seed=a.seed, point=point,
                                 frame0=done + first, out=part)
