@@ -103,6 +103,8 @@ def lib():
     L.ccgpu_awgn_point_gmd.argtypes = [vp, vp, u32, dbl, u64, u32, u64, u64, vp]
     L.ccgpu_decode_llr_abp.argtypes = [vp, vp, u32, dbl, vp, u64, vp, vp, vp, vp]
     L.ccgpu_awgn_point_abp.argtypes = [vp, vp, u32, dbl, dbl, u64, u32, u64, u64, vp]
+    L.ccgpu_decode_llr_ml.argtypes = [vp, vp, vp, u64, vp]
+    L.ccgpu_awgn_point_ml.argtypes = [vp, vp, dbl, u64, u32, u64, u64, vp]
     L.ccgpu_gf_decode.argtypes = [vp, vp, vp, u64, vp, vp, vp]
     L.ccgpu_gf_decode_erasures.argtypes = [vp, vp, vp, u64, vp, vp, u32, vp, vp, vp]
     L.ccgpu_gf_decode_erasures_pgz.argtypes = [vp, vp, vp, u64, vp, vp, u32, vp, vp, vp]
@@ -123,6 +125,7 @@ def lib():
     L.ccgpu_group_awgn_point_osd.argtypes = [vp, cpp, u32, dbl, u64, u32, u64, u64, vp]
     L.ccgpu_group_awgn_point_gmd.argtypes = [vp, cpp, u32, dbl, u64, u32, u64, u64, vp]
     L.ccgpu_group_awgn_point_abp.argtypes = [vp, cpp, u32, dbl, dbl, u64, u32, u64, u64, vp]
+    L.ccgpu_group_awgn_point_ml.argtypes = [vp, cpp, dbl, u64, u32, u64, u64, vp]
     L.ccgpu_group_awgn_point_mbbp.argtypes = [vp, cpp, C.POINTER(MsParams), vp, u32, dbl, u64, u32, u64, u64, vp]
     L.ccgpu_group_awgn_point_uncoded.argtypes = [vp, u32, dbl, dbl, u64, u32, u64, u64, vp]
     L.ccgpu_group_bitflip_point.argtypes = [vp, cpp, C.POINTER(MsParams), u32, u64, u64, vp]
@@ -147,4 +150,5 @@ EXPORTS = ["ccgpu_abi_version", "ccgpu_create", "ccgpu_destroy", "ccgpu_last_err
            "ccgpu_group_decode_llr", "ccgpu_group_gf_decode", "ccgpu_decode_llr_chase", "ccgpu_awgn_point_chase",
            "ccgpu_group_awgn_point_chase", "ccgpu_decode_llr_osd", "ccgpu_awgn_point_osd", "ccgpu_group_awgn_point_osd",
            "ccgpu_decode_llr_gmd", "ccgpu_awgn_point_gmd", "ccgpu_group_awgn_point_gmd",
-           "ccgpu_decode_llr_abp", "ccgpu_awgn_point_abp", "ccgpu_group_awgn_point_abp"]
+           "ccgpu_decode_llr_abp", "ccgpu_awgn_point_abp", "ccgpu_group_awgn_point_abp",
+           "ccgpu_decode_llr_ml", "ccgpu_awgn_point_ml", "ccgpu_group_awgn_point_ml"]

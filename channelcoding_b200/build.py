@@ -32,7 +32,7 @@ def _groups():
 def _units():
     units = [("api.o", "api.cu", []), ("ms_registry.o", "ms_registry.cu", []), ("ms_csr.o", "ms_csr.cu", []),
              ("gf_decode.o", "gf_decode.cu", []), ("chase.o", "chase.cu", []),
-             ("osd.o", "osd.cu", []), ("gmd.o", "gmd.cu", []), ("abp.o", "abp.cu", []),
+             ("osd.o", "osd.cu", []), ("gmd.o", "gmd.cu", []), ("abp.o", "abp.cu", []), ("ml.o", "ml.cu", []),
              ("group.o", "group.cc", [])]
     units.append(("ms_cyclic_cta.o", "ms_cyclic_cta_inst.cu", []))
     units.append(("ms_cyclic_lane.o", "ms_cyclic_lane_inst.cu", []))
@@ -96,7 +96,8 @@ def build_tools(force=False):
             (os.path.join(TOOLS_BIN, "chase_test"), os.path.join(root, "tests", "cpp", "chase_test.cc")),
             (os.path.join(TOOLS_BIN, "osd_test"), os.path.join(root, "tests", "cpp", "osd_test.cc")),
             (os.path.join(TOOLS_BIN, "gmd_test"), os.path.join(root, "tests", "cpp", "gmd_test.cc")),
-            (os.path.join(TOOLS_BIN, "abp_test"), os.path.join(root, "tests", "cpp", "abp_test.cc"))]
+            (os.path.join(TOOLS_BIN, "abp_test"), os.path.join(root, "tests", "cpp", "abp_test.cc")),
+            (os.path.join(TOOLS_BIN, "ml_test"), os.path.join(root, "tests", "cpp", "ml_test.cc"))]
 
     def one(job):
         out, src = job

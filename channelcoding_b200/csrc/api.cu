@@ -21,6 +21,7 @@
 #include "gf_decode.h"
 #include "abp.h"
 #include "gmd.h"
+#include "ml.h"
 #include "ms_csr.h"
 #include "ms_params.h"
 #include "osd.h"
@@ -76,6 +77,7 @@ struct ccgpu_code {
   MsCsrDevice csr;     // general-H kernel tables (device)
   GfDevice gf;         // algebraic decoder tables (device)
   OsdDevice osd;       // packed k-row H of the ordered-statistics decoder (device; binary BCH, n <= 127, k <= 64)
+  MlCode ml;           // column syndromes of the k-row H for the Viterbi decoder (host; binary BCH, n <= 127, k <= 12)
 };
 
 namespace {
@@ -585,6 +587,7 @@ int finish_code(ccgpu_ctx *ctx, ccgpu_code *c) {
   if (rc || !ctx || c->spec.family == 2) return rc;
   if (gf_upload(c->spec, &c->gf) != 0) return fail(ctx, CCGPU_ERR_CUDA, "gf_upload failed");
   if (osd_upload(c->spec, &c->osd) != 0) return fail(ctx, CCGPU_ERR_CUDA, "osd_upload failed");
+  ml_prepare(c->spec, &c->ml);
   return CCGPU_OK;
 }
 
@@ -1730,6 +1733,52 @@ int ccgpu_awgn_point_abp(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t max_it
   return with_counters(ctx, out, [&](unsigned long long *counters) {
     return abp_rc(ctx, abp_awgn_launch(code->osd, max_iter, static_cast<float>(gamma), sigma, seed, point, frame0, frames,
                                        counters, ctx->sm_count, ctx->stream));
+  });
+}
+
+// ---- maximum-likelihood decoding (extension): K9 in ml.cu, on the column syndromes of the k-row H
+static int check_ml(ccgpu_ctx *ctx, const ccgpu_code *code) {
+  if (int rc = check_code(ctx, code)) return rc;
+  if (code->spec.family != 0) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "ML decoding needs a binary BCH code");
+  if (!code->ml.k) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "code not supported by the ML kernel (n <= 127, n - l <= 12)");
+  return CCGPU_OK;
+}
+static int ml_rc(ccgpu_ctx *ctx, int rc) {
+  if (rc == -3) return fail(ctx, CCGPU_ERR_UNSUPPORTED, "code not supported by the ML kernel (n <= 127, n - l <= 12)");
+  if (rc != 0) return cuda_fail(ctx, cudaGetLastError(), "ml_launch");
+  ctx->launches++;
+  return CCGPU_OK;
+}
+
+int ccgpu_decode_llr_ml(ccgpu_ctx *ctx, const ccgpu_code *code, const float *y, uint64_t frames, uint8_t *bits) {
+  if (!ctx || !code || !y || !bits) return fail(ctx, CCGPU_ERR_INVALID, "null argument");
+  int rc = check_ml(ctx, code);
+  if (rc) return rc;
+  std::lock_guard<std::mutex> g(ctx->mu);
+  if (frames == 0) return CCGPU_OK;
+  CU(cudaSetDevice(ctx->device));
+  const size_t n = code->spec.n;
+  const bool dev = is_device_ptr(y);
+  if (!same_residency(dev, {bits}))
+    return fail(ctx, CCGPU_ERR_INVALID, "y and the outputs must all be device pointers or all host pointers");
+  if (dev) return ml_rc(ctx, ml_launch(code->ml, y, frames, bits, ctx->sm_count, ctx->stream));
+  const HostField fields[] = { { n * sizeof(float), y, false }, { n, bits, true } };
+  return host_pipeline(ctx, frames, fields, [&](void *const *d, uint64_t nf, cudaStream_t st, int) {
+    return ml_rc(ctx, ml_launch(code->ml, static_cast<const float *>(d[0]), nf, static_cast<uint8_t *>(d[1]),
+                                ctx->sm_count, st));
+  });
+}
+
+int ccgpu_awgn_point_ml(ccgpu_ctx *ctx, const ccgpu_code *code, double ebno_db, uint64_t seed, uint32_t point,
+                        uint64_t frame0, uint64_t frames, ccgpu_counters *out) {
+  if (!ctx || !code || !out) return fail(ctx, CCGPU_ERR_INVALID, "null argument");
+  int rc = check_ml(ctx, code);
+  if (rc) return rc;
+  std::lock_guard<std::mutex> g(ctx->mu);
+  CU(cudaSetDevice(ctx->device));
+  const float sigma = static_cast<float>(ccgpu_sigma(code->spec.rate, ebno_db));
+  return with_counters(ctx, out, [&](unsigned long long *counters) {
+    return ml_rc(ctx, ml_awgn_launch(code->ml, sigma, seed, point, frame0, frames, counters, ctx->sm_count, ctx->stream));
   });
 }
 

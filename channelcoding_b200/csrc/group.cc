@@ -250,6 +250,14 @@ int ccgpu_group_awgn_point_abp(ccgpu_group *g, ccgpu_code *const *codes, uint32_
   });
 }
 
+int ccgpu_group_awgn_point_ml(ccgpu_group *g, ccgpu_code *const *codes, double ebno_db, uint64_t seed, uint32_t point,
+                              uint64_t frame0, uint64_t frames, ccgpu_counters *out) {
+  if (!codes) return fail(g, CCGPU_ERR_INVALID, "null argument");
+  return sharded_point(g, frames, out, [&](int m, uint64_t off, uint64_t cnt, ccgpu_counters *c) {
+    return ccgpu_awgn_point_ml(g->ctx[m], codes[m], ebno_db, seed, point, frame0 + off, cnt, c);
+  });
+}
+
 int ccgpu_group_awgn_point_mbbp(ccgpu_group *g, ccgpu_code *const *codes, const ccgpu_ms_params *params,
                                 const uint32_t *shifts, uint32_t n_bases, double ebno_db, uint64_t seed, uint32_t point,
                                 uint64_t frame0, uint64_t frames, ccgpu_counters *out) {

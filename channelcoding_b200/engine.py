@@ -477,6 +477,38 @@ class Code:
                                                         point, frame0, frames, C.addressof(c)))
         return c.as_dict()
 
+    def decode_ml(self, y, out=None):
+        """maximum-likelihood decoding by a Viterbi search over the syndrome trellis of the k-row H (extension,
+        ccgpu_decode_llr_ml; binary BCH codes with n <= 127, n - l <= 12) -> bits (frames, n) uint8, a codeword closest
+        to y; out: the bits array to write; numpy or torch CUDA tensors like decode()"""
+        if _is_torch(y):
+            import torch
+            y = y.contiguous().view(-1, self.n)
+            frames = y.shape[0]
+            if out is None:
+                out = torch.empty((frames, self.n), dtype=torch.uint8, device=y.device)
+        else:
+            y = np.ascontiguousarray(y, np.float32).reshape(-1, self.n)
+            frames = y.shape[0]
+            if out is None:
+                out = np.empty((frames, self.n), np.uint8)
+        self.ctx._follow_torch(y, out)
+        self.ctx._check(_lib.lib().ccgpu_decode_llr_ml(self.ctx._h, self._h, _ptr(y), frames, _ptr(out)))
+        return out
+
+    def awgn_point_ml(self, ebno_db, frames, seed=0, point=0, frame0=0, out=None):
+        """one Eb/N0 point decoded with ML on the GPU (ccgpu_awgn_point_ml) -> counters.
+        out: optional torch uint64/int64 CUDA tensor of 8 slots that is accumulated into (no sync)."""
+        if out is not None:
+            self.ctx._follow_torch(out)
+            self.ctx._check(_lib.lib().ccgpu_awgn_point_ml(self.ctx._h, self._h, float(ebno_db), seed, point, frame0, frames,
+                                                           _ptr(out)))
+            return out
+        c = Counters()
+        self.ctx._check(_lib.lib().ccgpu_awgn_point_ml(self.ctx._h, self._h, float(ebno_db), seed, point, frame0, frames,
+                                                       C.addressof(c)))
+        return c.as_dict()
+
     def bitflip_point(self, weight, variant="MS", alpha=1.0, beta=0.0, max_iter=50,
                       stop_rule=STOP_REF_ZERO_OVERLAP, first=0, count=0, quant=None):
         """one error weight of bitflip_simulation (simulation.c++:156-213) -> counters"""
@@ -633,6 +665,12 @@ class GroupCode:
         c = Counters()
         self.group._check(_lib.lib().ccgpu_group_awgn_point_abp(self.group._h, self._arr, int(max_iter), float(gamma),
                                                                 float(ebno_db), seed, point, frame0, frames, C.addressof(c)))
+        return c.as_dict()
+
+    def awgn_point_ml(self, ebno_db, frames, seed=0, point=0, frame0=0):
+        c = Counters()
+        self.group._check(_lib.lib().ccgpu_group_awgn_point_ml(self.group._h, self._arr, float(ebno_db), seed, point,
+                                                               frame0, frames, C.addressof(c)))
         return c.as_dict()
 
     def awgn_point_mbbp(self, ebno_db, frames, shifts, variant="MS", alpha=1.0, beta=0.0, max_iter=50,

@@ -141,3 +141,16 @@ def abp_point_fn(code, max_iter=50, gamma=0.15, seed=0):
             code.ctx.sync()
         return out
     return fn
+
+
+def ml_point_fn(code, seed=0):
+    """point_fn for awgn_sweep backed by ccgpu_awgn_point_ml (maximum-likelihood decoding) on the code's device"""
+    import torch
+
+    def fn(ebno, point, frame0, frames):
+        out = torch.zeros(8, dtype=torch.int64, device="cuda:%d" % code.ctx.device)
+        if frames > 0:
+            code.awgn_point_ml(ebno, frames, seed=seed, point=point, frame0=frame0, out=out)
+            code.ctx.sync()
+        return out
+    return fn

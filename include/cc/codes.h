@@ -13,6 +13,7 @@
 //   (extension) ordered-statistics decoding            cc::primitive_bch<q, Capability, osd_tag<Order> >
 //   (extension) GMD decoding of RS codes               cc::rs<q, Capability, gmd_tag<F> >
 //   (extension) adaptive belief propagation            cc::primitive_bch<q, Capability, abp_tag<Iterations, Gamma> >
+//   (extension) maximum-likelihood (Viterbi) decoding  cc::primitive_bch<q, Capability, ml_tag>
 //     .correct<R>(vector<float|uint>)  .to_string()  .rate  ::n  ::t  .H<T>()           codes/cyclic.h:282-359
 //
 // Differences a user sees: every object holds a ccgpu context/code handle (one GPU, or every GPU of the current
@@ -194,6 +195,15 @@ template <unsigned Iterations, typename Gamma = std::ratio<15, 100> > struct abp
 template <typename Tag> struct is_abp_tag : std::false_type {};
 template <unsigned I, typename G> struct is_abp_tag<abp_tag<I, G> > : std::true_type {};
 
+// ---- extension: maximum-likelihood decoding (ccgpu_decode_llr_ml).  A Viterbi search over the syndrome trellis of the
+// k-row H returns a codeword closest to the channel values; high-rate codes only (n - l <= 12).  Like Chase-II it takes
+// channel values and is neither a soft-decision (min-sum) nor a hard-decision tag.
+struct ml_tag : algorithm_tag {
+  static std::string to_string() { return "ML"; }
+};
+template <typename Tag> struct is_ml_tag : std::false_type {};
+template <> struct is_ml_tag<ml_tag> : std::true_type {};
+
 // ---- one GPU context shared by every code object of the process (per device) ------------------------
 class gpu_error : public std::runtime_error {
 public:
@@ -365,6 +375,7 @@ public:
   static constexpr bool osd = is_osd_tag<Algorithm>::value;
   static constexpr bool gmd = is_gmd_tag<Algorithm>::value;
   static constexpr bool abp = is_abp_tag<Algorithm>::value;
+  static constexpr bool ml = is_ml_tag<Algorithm>::value;
 
   std::string to_string() const {  // cyclic.h:282-287
     char buf[96];
@@ -627,6 +638,43 @@ public:
     else
       this->h_->ctx->check(ccgpu_awgn_point_abp(this->h_->ctx->get(), this->h_->code, Iterations, tag::gamma, ebno_db, seed,
                                                 point, frame0, frames, &c));
+    return c;
+  }
+};
+
+// extension: the same code decoded with maximum-likelihood decoding (ccgpu_decode_llr_ml; n <= 127, n - l <= 12)
+template <unsigned q, typename Capability>
+class primitive_bch<q, Capability, ml_tag> : public cyclic_base<ml_tag> {
+  using base = cyclic_base<ml_tag>;
+
+public:
+  static constexpr unsigned n = (1u << q) - 1;
+  static constexpr unsigned t = correction_capability<Capability>::value;
+  explicit primitive_bch(int device = -1) : base(detail::make_bch<q, Capability>(device)) {}
+
+  // frames x n channel values -> frames x n bits, always a codeword closest to the channel values
+  void correct_batch(const float *y, uint64_t frames, uint8_t *bits) const {
+    this->h_->ctx->check(ccgpu_decode_llr_ml(this->h_->ctx->get(), this->h_->code, y, frames, bits));
+  }
+  // one frame of channel values; ML never fails
+  template <typename Return_type = uint8_t, typename InputSequence>
+  std::vector<Return_type> correct(const InputSequence &b) const {
+    if (b.size() != n)
+      throw std::runtime_error("Channel code word has the wrong size (" + std::to_string(b.size()) + "). Expected " +
+                               std::to_string(n));
+    const std::vector<float> y(b.begin(), b.end());
+    std::vector<uint8_t> out(n);
+    correct_batch(y.data(), 1, out.data());
+    return std::vector<Return_type>(out.begin(), out.end());
+  }
+  // one Eb/N0 point (simulation.c++:112-149) decoded with ML on the device, sharded over the code's group if any
+  ccgpu_counters awgn_point(double ebno_db, uint64_t frames, uint64_t seed = 0, uint32_t point = 0, uint64_t frame0 = 0) const {
+    ccgpu_counters c{};
+    if (this->h_->grp)
+      this->h_->grp->check(ccgpu_group_awgn_point_ml(this->h_->grp->get(), this->h_->codes.data(), ebno_db, seed, point,
+                                                     frame0, frames, &c));
+    else
+      this->h_->ctx->check(ccgpu_awgn_point_ml(this->h_->ctx->get(), this->h_->code, ebno_db, seed, point, frame0, frames, &c));
     return c;
   }
 };

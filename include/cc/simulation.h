@@ -116,8 +116,9 @@ class decoder {
     }
     bool soft() const override { return T::soft_tag; }
     ccgpu_counters awgn_point(double e, uint64_t f, uint64_t s, uint32_t p, uint64_t f0) const override {
-      // soft tags, Chase-II, OSD, GMD and ABP take the channel values: their own fused point
-      return point_impl(e, f, s, p, f0, std::integral_constant<bool, T::soft_tag || T::chase || T::osd || T::gmd || T::abp>());
+      // soft tags, Chase-II, OSD, GMD, ABP and ML take the channel values: their own fused point
+      return point_impl(e, f, s, p, f0,
+                        std::integral_constant<bool, T::soft_tag || T::chase || T::osd || T::gmd || T::abp || T::ml>());
     }
     ccgpu_counters bitflip_point(unsigned weight) const override {
       if constexpr (T::chase)
@@ -128,6 +129,8 @@ class decoder {
         throw std::runtime_error(implementation.to_string() + ": bit-flip simulation has no channel reliabilities for GMD");
       else if constexpr (T::abp)
         throw std::runtime_error(implementation.to_string() + ": bit-flip simulation has no channel reliabilities for ABP");
+      else if constexpr (T::ml)
+        throw std::runtime_error(implementation.to_string() + ": bit-flip simulation has no channel reliabilities for ML");
       else
         return flips_impl(weight, std::integral_constant<bool, T::soft_tag>());
     }

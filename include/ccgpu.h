@@ -374,6 +374,33 @@ int ccgpu_decode_llr_abp(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t max_it
 int ccgpu_awgn_point_abp(ccgpu_ctx *ctx, const ccgpu_code *code, uint32_t max_iter, double gamma, double ebno_db,
                          uint64_t seed, uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
 
+/* EXTENSION (no reference implementation): maximum-likelihood decoding of high-rate binary primitive BCH codes by a
+ * Viterbi search over the syndrome trellis of the k-row H (2^k states, n sections).  It returns a codeword closest to
+ * the channel values in the metric of ccgpu_decode_llr_chase / _osd, with no approximation: the exact yardstick of the
+ * other soft-decision decoders.  The k-row H of ccgpu_code_H at creation is always used, whatever
+ * ccgpu_code_set_rows selected.  Per frame, with sigma_c = sum_r H[r][c] 2^r the k-bit syndrome of column c (never 0
+ * for a BCH code):
+ *   1. h_c = (y_c < 0) (codes/codes.h:43-52: 0 for -0.0 and NaN);
+ *   2. w_c = fminf(fabsf(y_c), 2^20), NaN giving +0.0 (a NaN is an erasure; every w_c is finite);
+ *   3. M_0(0) = +0.0, M_0(s) = +inf for s != 0;
+ *   4. for c = 0 .. n-1 and every state s in [0, 2^k): the branch x_c = 0 comes from state s with cost [h_c != 0] w_c,
+ *      the branch x_c = 1 from state s ^ sigma_c with cost [h_c != 1] w_c; M_{c+1}(s) is the smaller of the two sums
+ *      M_c(pred) + cost, each one float32 add rounded to nearest even (no FMA); on equal sums the branch with
+ *      x_c = h_c wins; d_c(s) is the x_c of the winning branch;
+ *   5. traceback from s = 0: for c = n-1 down to 0: x_c = d_c(s), s ^= x_c sigma_c.  bits = x.
+ * x is a codeword, its D (the float32 sum of w_c over the positions where x_c != h_c, c ascending, from +0.0) is M_n(0)
+ * and at most the D of every codeword, and a codeword h is returned as it is.  There is no failure.  Binary BCH codes
+ * with n <= 127 and 4 <= k <= 12 (BCH(15,11), (15,7), (15,5), (31,26), (31,21), (63,57), (63,51), (127,120)); RS,
+ * dense-H codes, n = 255 or k > 12: CCGPU_ERR_UNSUPPORTED.  bits frames x n.  Host or device pointers like
+ * ccgpu_decode_llr, all of one kind. */
+int ccgpu_decode_llr_ml(ccgpu_ctx *ctx, const ccgpu_code *code, const float *y, uint64_t frames, uint8_t *bits);
+/* one Eb/N0 point, frames [frame0, frame0 + frames) of the ccgpu_awgn_point noise stream (raw y, no LLR scaling),
+ * decoded with ML on chip.  Only counters leave: frame_errors = frames with any decided bit set, bit_errors = decided
+ * bits set, undetected = frame_errors, iterations = failures = 0.  `out` host or device pointer as in
+ * ccgpu_awgn_point. */
+int ccgpu_awgn_point_ml(ccgpu_ctx *ctx, const ccgpu_code *code, double ebno_db, uint64_t seed, uint32_t point,
+                        uint64_t frame0, uint64_t frames, ccgpu_counters *out);
+
 /* one weight class of bitflip_simulation::operator() (simulation.c++:156-213): all C(n, weight)
  * inputs x = -2*bit + 1, decoded and counted; patterns [first, first + count) in the
  * lexicographic order of std::next_permutation (count 0 = all). */
@@ -433,7 +460,7 @@ int ccgpu_group_size(const ccgpu_group *group);
 ccgpu_ctx *ccgpu_group_ctx(const ccgpu_group *group, int member);
 const char *ccgpu_group_last_error(const ccgpu_group *group);
 int ccgpu_group_set_min_frames(ccgpu_group *group, uint64_t frames_per_member);
-/* the Monte-Carlo points of ccgpu_awgn_point / _hard / _chase / _osd / _gmd / _abp / _mbbp / _uncoded / ccgpu_bitflip_point, sharded; `out` is a
+/* the Monte-Carlo points of ccgpu_awgn_point / _hard / _chase / _osd / _gmd / _abp / _ml / _mbbp / _uncoded / ccgpu_bitflip_point, sharded; `out` is a
  * host pointer and holds the merged counters on return */
 int ccgpu_group_awgn_point(ccgpu_group *group, ccgpu_code *const *codes, const ccgpu_ms_params *params, double ebno_db,
                            uint64_t seed, uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
@@ -448,6 +475,8 @@ int ccgpu_group_awgn_point_gmd(ccgpu_group *group, ccgpu_code *const *codes, uin
 int ccgpu_group_awgn_point_abp(ccgpu_group *group, ccgpu_code *const *codes, uint32_t max_iter, double gamma,
                                double ebno_db, uint64_t seed, uint32_t point, uint64_t frame0, uint64_t frames,
                                ccgpu_counters *out);
+int ccgpu_group_awgn_point_ml(ccgpu_group *group, ccgpu_code *const *codes, double ebno_db, uint64_t seed,
+                              uint32_t point, uint64_t frame0, uint64_t frames, ccgpu_counters *out);
 int ccgpu_group_awgn_point_mbbp(ccgpu_group *group, ccgpu_code *const *codes, const ccgpu_ms_params *params,
                                 const uint32_t *shifts, uint32_t n_bases, double ebno_db, uint64_t seed, uint32_t point,
                                 uint64_t frame0, uint64_t frames, ccgpu_counters *out);

@@ -13,7 +13,9 @@
 // --algorithm chase1 .. chase8 (Chase-II over 1 .. 8 test positions, "(n, l, dmin)-CHASE<P>.log"; built only when
 // named, never part of "all" or of the default selection), --algorithm osd0 .. osd3 (ordered-statistics decoding of
 // order 0 .. 3, "(n, l, dmin)-OSD<i>.log"; likewise only when named), --algorithm abp (adaptive belief propagation,
-// 50 iterations, damping 0.15, "(n, l, dmin)-ABP50.log"; likewise only when named).
+// 50 iterations, damping 0.15, "(n, l, dmin)-ABP50.log"; likewise only when named), --algorithm ml (maximum-likelihood
+// decoding of the catalogue codes with n - l <= 12: (31,26,3), (31,21,5), (63,57,3), (63,51,5), (127,120,3);
+// "(n, l, dmin)-ML.log"; likewise only when named).
 #include <getopt.h>
 
 #include <cmath>
@@ -70,6 +72,15 @@ template <unsigned Q> static void add_abp_power(std::vector<decoder> &v) {
   v.emplace_back(primitive_bch<Q, dmin<7>, abp_default>());
   v.emplace_back(primitive_bch<Q, dmin<9>, abp_default>());
 }
+// ML decoders (extension): only built when --algorithm ml asks for them, never part of "all"; the catalogue codes with
+// at most 12 parity checks, the bound of the Viterbi kernel
+static void add_ml(std::vector<decoder> &v) {
+  v.emplace_back(primitive_bch<5, dmin<3>, ml_tag>());
+  v.emplace_back(primitive_bch<5, dmin<5>, ml_tag>());
+  v.emplace_back(primitive_bch<6, dmin<3>, ml_tag>());
+  v.emplace_back(primitive_bch<6, dmin<5>, ml_tag>());
+  v.emplace_back(primitive_bch<7, dmin<3>, ml_tag>());
+}
 template <unsigned Q> static void add_power(std::vector<decoder> &v) {
   add_code<Q, dmin<3> >(v);
   add_code<Q, dmin<5> >(v);
@@ -79,8 +90,8 @@ template <unsigned Q> static void add_power(std::vector<decoder> &v) {
 
 [[noreturn]] static void usage() {
   std::cout << "--simulation [awgn|bitflip]  choose the simulation (default awgn)\n"
-               "--algorithm <ms|nms|oms|scms1|scms2|2dnms|bm|pgz|euklid|all|chase1..chase8|osd0..osd3|abp>\n"
-               "             (repeatable; Chase-II, OSD and ABP only when named, awgn only)\n"
+               "--algorithm <ms|nms|oms|scms1|scms2|2dnms|bm|pgz|euklid|all|chase1..chase8|osd0..osd3|abp|ml>\n"
+               "             (repeatable; Chase-II, OSD, ABP and ML only when named, awgn only)\n"
                "--k <5|6|7|all>   code length n = 2^k - 1   (repeatable)\n"
                "--dmin <3|5|7|9|all>                          (repeatable)\n"
                "--seed <num>  --seed-time  --threads <num>\n"
@@ -158,6 +169,8 @@ int main(int argc, char *const argv[]) {
     add_abp_power<7>(decoders);
     algorithms.insert(lower(abp_default::to_string()));
   }
+
+  if (algorithms.count("ml")) add_ml(decoders);
 
   // selection by parsing to_string(), exactly like benchmark.c++:214-240
   std::vector<const decoder *> chosen;

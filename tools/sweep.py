@@ -6,6 +6,7 @@
     python tools/sweep.py --q 6 --t 5 --osd 2 ...        # ordered-statistics decoding of order 2
     python tools/sweep.py --q 8 --t 16 --gmd 32 ...      # RS(255,223), GMD with up to 32 erasures (--gmd 0: hard)
     python tools/sweep.py --q 6 --t 5 --abp 50 --gamma 0.15 ...  # adaptive belief propagation, 50 updates at most
+    python tools/sweep.py --q 6 --t 2 --ml ...           # maximum-likelihood (Viterbi) decoding, n - l <= 12
     torchrun --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 tools/sweep.py ...
 
 Every Eb/N0 point is simulated in rounds of --batch frames (split evenly over the ranks by global frame
@@ -49,6 +50,9 @@ def main():
     algo.add_argument("--abp", type=int, default=None, metavar="ITERS",
                       help="decode with adaptive belief propagation, at most ITERS (0..255) updates, instead of the "
                            "min-sum variant")
+    algo.add_argument("--ml", action="store_true",
+                      help="decode with maximum-likelihood (Viterbi) decoding on the syndrome trellis (n - l <= 12) "
+                           "instead of the min-sum variant")
     ap.add_argument("--gamma", type=float, default=0.15, help="damping factor of --abp (0 < gamma <= 1)")
     a = ap.parse_args()
 
@@ -71,7 +75,8 @@ def main():
     bits_per_frame = code.n * a.q if a.gmd is not None else code.n  # GMD counts the bits of the binary image
     dev = torch.device("cuda", local)
     tag = ("CHASE%d" % a.chase if a.chase is not None else "OSD%d" % a.osd if a.osd is not None else
-           "GMD%d" % a.gmd if a.gmd is not None else "ABP%d" % a.abp if a.abp is not None else a.variant)
+           "GMD%d" % a.gmd if a.gmd is not None else "ABP%d" % a.abp if a.abp is not None else
+           "ML" if a.ml else a.variant)
     point, eb = 0, a.ebno_from
     while eb < a.ebno_to + a.ebno_step / 2:
         total = torch.zeros(8, dtype=torch.int64, device=dev)
@@ -88,6 +93,8 @@ def main():
                 code.awgn_point_gmd(eb, count, a.gmd, seed=a.seed, point=point, frame0=done + first, out=part)
             elif a.abp is not None:
                 code.awgn_point_abp(eb, count, a.abp, a.gamma, seed=a.seed, point=point, frame0=done + first, out=part)
+            elif a.ml:
+                code.awgn_point_ml(eb, count, seed=a.seed, point=point, frame0=done + first, out=part)
             else:
                 code.awgn_point(eb, count, a.variant, a.alpha, a.beta, a.max_iter, a.stop_rule, seed=a.seed, point=point,
                                 frame0=done + first, out=part)
